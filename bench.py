@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Headline benchmark: rays/s of a 3-view 128x128 pixelNeRF render (BASELINE.json config 2).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 One step = ONE full target image (16 384 rays, 64 coarse + 96 fine samples per ray, 3 source views, resnet34-sized
 512-channel feature maps, random-init weights) through NeRFRenderer.forward.
@@ -379,6 +379,17 @@ def train_step_block(device):
             "flops": "3 x forward algorithmic FLOPs (forward + dgrad + wgrad)"}
 
 
+def dump_outputs(out_dir, image):
+    """--dump-outputs: the image of the last timed step as the render API returns it, rgb.npy (1, 16384, 3) and depth.npy
+    (1, 16384), float32.  Scene, weights and sampling noise all come from fixed seeds (the noise from torch.manual_seed(0) in
+    build_ours and the same sequence of draws), so two builds run with the same arguments can be compared array for array."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    image = image.float().cpu()
+    np.save(os.path.join(out_dir, "rgb.npy"), image[:, :3].unsqueeze(0).contiguous().numpy())
+    np.save(os.path.join(out_dir, "depth.npy"), image[:, 3].unsqueeze(0).contiguous().numpy())
+
+
 # ---------------------------------------------------------------------------------------------------------------------
 def run_ours(args):
     import torch.distributed as dist
@@ -447,16 +458,17 @@ def run_ours(args):
         return packed
 
     def timed_loop(fn, steps):
-        total = 0.0
+        """-> (total ms of `steps` calls of fn, what the last call returned)"""
+        total, out = 0.0, None
         for _ in range(steps):
             flush.fill_(1)                                                                # evict L2 between steps
             e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             e0.record()
-            fn()
+            out = fn()
             e1.record()
             e1.synchronize()
             total += e0.elapsed_time(e1)
-        return total
+        return total, out
 
     def sync_all():
         torch.cuda.synchronize()
@@ -475,11 +487,11 @@ def run_ours(args):
         sync_all()
         if rank == 0:
             sampler.start()
-        ms_dev = timed_loop(lambda: step_device(live_events), args.steps)
+        ms_dev, last_image = timed_loop(lambda: step_device(live_events), args.steps)
         sync_all()
         renderer.field_events = None
         launches = renderer.last_launches
-        ms_e2e = timed_loop(step_e2e, args.steps)
+        ms_e2e, _ = timed_loop(step_e2e, args.steps)
         sync_all()
         clocks = sampler.stop() if rank == 0 else None
         roofline_pass = "live, inside the timed region"
@@ -493,6 +505,8 @@ def run_ours(args):
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     ms_dev, ms_e2e = t.tolist()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last_image)
     field_total_ms = sum(a.elapsed_time(b) for a, b in field_pairs)
     n_field = len(field_pairs)
 
@@ -590,7 +604,13 @@ def main():
                     help="rays in the bounded CPU sample (default 4096 for cpu_baseline = 10-15 s of CPU work, 512 per step for --impl reference)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip config 4, the train step and the GPU eager baseline")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the rgb and depth of the last timed step to DIR/rgb.npy and DIR/depth.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the output of --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.cpu_rays is None:
         args.cpu_rays = 4096 if args.impl == "ours" else 512

@@ -28,19 +28,6 @@ def test_hocon_subset_parser(tmp_path):
     assert "model.mlp_fine" not in c and c.get_int("model.missing", 7) == 7
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/conf"), reason="reference confs only exist in the build container")
-def test_parses_every_reference_conf():
-    from pixel_nerf_yolo_b200 import conf
-    for name in ("default.conf", "default_mv.conf", "exp/dtu.conf", "exp/multi_obj.conf", "exp/sn64.conf",
-                 "exp/sn64_unseen.conf", "exp/srn.conf", "exp/yolo.conf"):
-        c = conf.parse_file(os.path.join("/root/reference/conf", name))
-        assert c.get_string("model.mlp_coarse.type") == "resnet", name
-        assert c.get_int("renderer.n_coarse") in (64, 128), name
-    c = conf.parse_file("/root/reference/conf/exp/yolo.conf")
-    assert c["yolo.anchors"][2][2] == [0.9, 0.78] and c.get_bool("model.mlp_coarse.yolo") is True
-    assert c.get_int("model.mlp_coarse.n_blocks") == 5 and c.get_string("model.encoder.backbone") == "custom"
-
-
 def test_dotmap_contract():
     from pixel_nerf_yolo_b200.conf import DotMap
     d = DotMap(coarse=DotMap(rgb=1))
