@@ -189,6 +189,11 @@ int pnr_positional_encoding(const float* x, float* out, long long n, int d, int 
 int pnr_index_features(const pnr_scene* scene, const float* uv, int uv_views, int P, float* out, void* stream);
 
 /* ---- ResnetFC weights (src/model/resnetfc.py:103-132) ------------------------------------------- */
+/* View pooling of ResnetFC (combine_type, resnetfc.py:172-174, util.combine_interleaved util.py:489-499): the NS source views of
+ * a point are reduced before block combine_layer by their mean or by their elementwise max. */
+#define PNR_COMBINE_AVERAGE 0
+#define PNR_COMBINE_MAX 1
+
 /* fp32 parameters of one ResnetFC in state_dict order; all device pointers. */
 typedef struct pnr_mlp_params {
   const float* lin_in_w;  const float* lin_in_b;     /* (H, d_in), (H)                 */
@@ -196,7 +201,10 @@ typedef struct pnr_mlp_params {
   const float* fc0_w[8];  const float* fc0_b[8];     /* blocks.i.fc_0  (H,H),(H)       */
   const float* fc1_w[8];  const float* fc1_b[8];     /* blocks.i.fc_1  (H,H),(H)       */
   const float* linz_w[8]; const float* linz_b[8];    /* lin_z.i  (H, d_latent),(H)     */
+  /* combine_layer = min(combine_layer, n_blocks): the views are pooled before block combine_layer; combine_layer == n_blocks
+   * never pools (the single-view network of conf/default.conf), which is only defined for NS == 1 */
   int32_t d_in, d_latent, d_hidden, d_out, n_blocks, combine_layer;
+  int32_t combine_type;                              /* PNR_COMBINE_*; the packed weight stream does not depend on it */
 } pnr_mlp_params;
 
 /* Bytes of the packed bf16 weight stream + fp32 bias tables for the tcgen05 path. */
@@ -235,7 +243,9 @@ typedef struct pnr_mlp_grads {
 } pnr_mlp_grads;
 
 /* PixelNeRFNet.forward in training mode: fp32 arithmetic, fp32 channels-last feature maps (feat_fp32=1), every
- * activation the backward pass needs is kept on the caller-owned `tape` (pnr_field_tape_bytes()). */
+ * activation the backward pass needs is kept on the caller-owned `tape` (pnr_field_tape_bytes()).  With PNR_COMBINE_MAX
+ * the tape also holds the winning view of every (point, feature) (one byte each): the backward pass sends the pooled
+ * gradient to the first maximal view, as torch.max(dim) does. */
 size_t pnr_field_tape_bytes(const pnr_scene* scene, const pnr_points* pts, const pnr_mlp_params* params);
 int pnr_field_forward_train(const pnr_scene* scene, const pnr_points* pts, const pnr_mlp_params* params, float* out,
                             void* tape, size_t tape_bytes, int num_freqs, float freq_factor, void* stream);

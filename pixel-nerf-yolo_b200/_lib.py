@@ -22,6 +22,7 @@ SCENE_RAW_OUTPUT = 2
 SCENE_PROJECTED = 4
 SCENE_TRAIN_TF32 = 8
 SCENE_TRAIN_BF16 = 16
+COMBINE_TYPES = {"average": 0, "max": 1}     # pnr_mlp_params.combine_type
 
 # every symbol include/pixelnerf_b200.h declares
 EXPORTS = [
@@ -78,7 +79,7 @@ class MlpParams(C.Structure):
                 ("fc1_w", C.c_void_p * 8), ("fc1_b", C.c_void_p * 8), ("linz_w", C.c_void_p * 8),
                 ("linz_b", C.c_void_p * 8), ("d_in", C.c_int32), ("d_latent", C.c_int32),
                 ("d_hidden", C.c_int32), ("d_out", C.c_int32), ("n_blocks", C.c_int32),
-                ("combine_layer", C.c_int32)]
+                ("combine_layer", C.c_int32), ("combine_type", C.c_int32)]
 
 
 class MlpGrads(C.Structure):

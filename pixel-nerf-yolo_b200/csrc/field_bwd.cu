@@ -375,51 +375,83 @@ static int colsum(const float* dY, float* db, long long M, int N, cudaStream_t s
   return PNR_OK;
 }
 
-// mean over the NS source views (util.py:489-499) and its transpose
-__global__ void view_mean_kernel(const float* __restrict__ x, float* __restrict__ y, int SB, int NS, int P, int H) {
+// view pooling over the NS source views (util.py:489-499) and its transpose.  arg == nullptr: mean (combine_type average);
+// otherwise elementwise max (combine_type max), and arg (SB, P, H) records the first maximal view, the one torch.max(dim)
+// routes the gradient to.
+__global__ void view_mean_kernel(const float* __restrict__ x, float* __restrict__ y, uint8_t* __restrict__ arg, int SB, int NS, int P,
+                                 int H) {
   const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= (long long)SB * P * H) return;
   const int h = (int)(i % H);
   const long long sp = i / H;
   const int p = (int)(sp % P), s = (int)(sp / P);
+  if (arg) {
+    float m = x[((long long)s * NS * P + p) * H + h];
+    int win = 0;
+    for (int v = 1; v < NS; ++v) {
+      const float a = x[(((long long)s * NS + v) * P + p) * H + h];
+      if (a > m) { m = a; win = v; }
+    }
+    y[i] = m;
+    arg[i] = (uint8_t)win;
+    return;
+  }
   float acc = 0.f;
   for (int v = 0; v < NS; ++v) acc += x[(((long long)s * NS + v) * P + p) * H + h];
   y[i] = acc / (float)NS;
 }
-__global__ void view_mean_bwd_kernel(const float* __restrict__ dy, float* __restrict__ dx, int SB, int NS, int P, int H) {
+__global__ void view_mean_bwd_kernel(const float* __restrict__ dy, float* __restrict__ dx, const uint8_t* __restrict__ arg, int SB, int NS,
+                                     int P, int H) {
   const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= (long long)SB * NS * P * H) return;
   const int h = (int)(i % H);
   const long long svp = i / H;
   const int p = (int)(svp % P);
   const int s = (int)(svp / P / NS);
-  dx[i] = dy[((long long)s * P + p) * H + h] / (float)NS;
+  const long long o = ((long long)s * P + p) * H + h;
+  if (arg) { dx[i] = arg[o] == (int)(svp / P - (long long)s * NS) ? dy[o] : 0.f; return; }
+  dx[i] = dy[o] / (float)NS;
 }
 
 // bf16 path helpers -----------------------------------------------------------------------------------------------------
-// view mean that also emits the relu'd bf16 operand of the next fc_0; 4 consecutive features per thread (H % 4 == 0)
-__global__ void view_mean_bf16_kernel(const float* __restrict__ x, float* __restrict__ y, __nv_bfloat16* __restrict__ y16, int SB, int NS,
-                                      int P, int H) {
+// view pooling (as view_mean_kernel, arg != nullptr: max) that also emits the relu'd bf16 operand of the next fc_0; 4 consecutive
+// features per thread (H % 4 == 0)
+__global__ void view_mean_bf16_kernel(const float* __restrict__ x, float* __restrict__ y, __nv_bfloat16* __restrict__ y16,
+                                      uint8_t* __restrict__ arg, int SB, int NS, int P, int H) {
   const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   const int H4 = H >> 2;
   if (i >= (long long)SB * P * H4) return;
   const int h4 = (int)(i % H4);
   const long long sp = i / H4;
   const int p = (int)(sp % P), s = (int)(sp / P);
-  float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
-  for (int v = 0; v < NS; ++v) {
-    const float4 a = __ldg(reinterpret_cast<const float4*>(x + (((long long)s * NS + v) * P + p) * H) + h4);
-    acc.x += a.x; acc.y += a.y; acc.z += a.z; acc.w += a.w;
+  float4 m;
+  if (arg) {
+    m = __ldg(reinterpret_cast<const float4*>(x + ((long long)s * NS * P + p) * H) + h4);
+    uchar4 win = make_uchar4(0, 0, 0, 0);
+    for (int v = 1; v < NS; ++v) {
+      const float4 a = __ldg(reinterpret_cast<const float4*>(x + (((long long)s * NS + v) * P + p) * H) + h4);
+      if (a.x > m.x) { m.x = a.x; win.x = (unsigned char)v; }
+      if (a.y > m.y) { m.y = a.y; win.y = (unsigned char)v; }
+      if (a.z > m.z) { m.z = a.z; win.z = (unsigned char)v; }
+      if (a.w > m.w) { m.w = a.w; win.w = (unsigned char)v; }
+    }
+    reinterpret_cast<uchar4*>(arg)[i] = win;
+  } else {
+    float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
+    for (int v = 0; v < NS; ++v) {
+      const float4 a = __ldg(reinterpret_cast<const float4*>(x + (((long long)s * NS + v) * P + p) * H) + h4);
+      acc.x += a.x; acc.y += a.y; acc.z += a.z; acc.w += a.w;
+    }
+    const float n = (float)NS;
+    m = make_float4(acc.x / n, acc.y / n, acc.z / n, acc.w / n);
   }
-  const float n = (float)NS;
-  const float4 m = make_float4(acc.x / n, acc.y / n, acc.z / n, acc.w / n);
   reinterpret_cast<float4*>(y)[i] = m;
   __nv_bfloat162* o = reinterpret_cast<__nv_bfloat162*>(y16) + i * 2;
   o[0] = __floats2bfloat162_rn(fmaxf(m.x, 0.f), fmaxf(m.y, 0.f));
   o[1] = __floats2bfloat162_rn(fmaxf(m.z, 0.f), fmaxf(m.w, 0.f));
 }
-__global__ void view_mean_bwd_bf16_kernel(const float* __restrict__ dy, float* __restrict__ dx, __nv_bfloat16* __restrict__ dx16, int SB,
-                                          int NS, int P, int H) {
+__global__ void view_mean_bwd_bf16_kernel(const float* __restrict__ dy, float* __restrict__ dx, __nv_bfloat16* __restrict__ dx16,
+                                          const uint8_t* __restrict__ arg, int SB, int NS, int P, int H) {
   const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   const int H4 = H >> 2;
   if (i >= (long long)SB * NS * P * H4) return;
@@ -428,8 +460,15 @@ __global__ void view_mean_bwd_bf16_kernel(const float* __restrict__ dy, float* _
   const int p = (int)(svp % P);
   const int s = (int)(svp / P / NS);
   const float4 a = __ldg(reinterpret_cast<const float4*>(dy + ((long long)s * P + p) * H) + h4);
-  const float n = (float)NS;
-  const float4 g = make_float4(a.x / n, a.y / n, a.z / n, a.w / n);
+  float4 g;
+  if (arg) {
+    const int v = (int)(svp / P - (long long)s * NS);
+    const uchar4 w = reinterpret_cast<const uchar4*>(arg)[((long long)s * P + p) * H4 + h4];
+    g = make_float4(w.x == v ? a.x : 0.f, w.y == v ? a.y : 0.f, w.z == v ? a.z : 0.f, w.w == v ? a.w : 0.f);
+  } else {
+    const float n = (float)NS;
+    g = make_float4(a.x / n, a.y / n, a.z / n, a.w / n);
+  }
   reinterpret_cast<float4*>(dx)[i] = g;
   __nv_bfloat162* o = reinterpret_cast<__nv_bfloat162*>(dx16) + i * 2;
   o[0] = __floats2bfloat162_rn(g.x, g.y);
@@ -634,9 +673,14 @@ struct Tape {
   float* NET[8];    // rows x H: fc_0 output of pre-combine block b
   float* XM[9];     // pts x H : input of post-combine block b (b >= CL); XM[n_blocks] = input of lin_out
   float* NETM[8];   // pts x H
+  uint8_t* ARG;     // pts x H: winning view of the max pooling (combine_type max only)
   size_t floats;
 };
-static Tape carve_tape(float* base, long long rows, long long pts, int C, int d_in, int H, int nb, int CL) {
+// combine_type max with more than one view to pool: the tape records the winning view of every (point, feature)
+static bool pool_max(const pnr_scene* sc, const pnr_mlp_params* mp) {
+  return mp->combine_type == PNR_COMBINE_MAX && sc->NS > 1 && mp->combine_layer < mp->n_blocks;
+}
+static Tape carve_tape(float* base, long long rows, long long pts, int C, int d_in, int H, int nb, int CL, bool vmax) {
   Tape t = {};
   float* p = base;
   t.lat = p; p += rows * C;
@@ -645,6 +689,7 @@ static Tape carve_tape(float* base, long long rows, long long pts, int C, int d_
   for (int b = 0; b < CL; ++b) { t.NET[b] = p; p += rows * H; }
   for (int b = CL; b <= nb; ++b) { t.XM[b] = p; p += pts * H; }
   for (int b = CL; b < nb; ++b) { t.NETM[b] = p; p += pts * H; }
+  if (vmax) { t.ARG = reinterpret_cast<uint8_t*>(p); p += (pts * H + 3) / 4; }
   t.floats = (size_t)(p - base);
   return t;
 }
@@ -667,6 +712,8 @@ static int check_train(const pnr_scene* sc, const pnr_points* q, const pnr_mlp_p
   PNR_REQUIRE(mp->n_blocks >= 1 && mp->n_blocks <= 8, PNR_ERR_UNSUPPORTED, "%s: n_blocks=%d", who, mp->n_blocks);
   PNR_REQUIRE(mp->combine_layer >= 1 && mp->combine_layer <= mp->n_blocks, PNR_ERR_ARG, "%s: combine_layer=%d", who, mp->combine_layer);
   PNR_REQUIRE(mp->combine_layer < mp->n_blocks || sc->NS == 1, PNR_ERR_UNSUPPORTED, "%s: combine_layer >= n_blocks needs NS=1", who);
+  PNR_REQUIRE(mp->combine_type == PNR_COMBINE_AVERAGE || mp->combine_type == PNR_COMBINE_MAX, PNR_ERR_ARG, "%s: combine_type=%d", who,
+              mp->combine_type);
   PNR_REQUIRE(mp->d_out >= 1 && mp->d_out <= 32, PNR_ERR_UNSUPPORTED, "%s: d_out=%d", who, mp->d_out);
   PNR_REQUIRE((long long)sc->SB * sc->NS * q->P < (1LL << 31), PNR_ERR_ARG, "%s: too many rows per call", who);
   return PNR_OK;
@@ -684,6 +731,7 @@ struct TapeB {
   __nv_bfloat16* RXM[9];            // pts x H: same for the post-combine blocks; RXM[n_blocks] = operand of lin_out
   __nv_bfloat16* RNM[8];
   float *x, *xm;                    // rows x H, pts x H fp32 residual stream (scratch of the forward pass)
+  uint8_t* arg;                     // pts x H winning view of the max pooling (combine_type max only)
   uint8_t* wpack;                   // forward packed weights
   size_t bytes;
 };
@@ -699,7 +747,7 @@ static WPack wpack_layout(int C, int d_in_pad, int H, int nb, int CL, bool trans
   w.total = off;
   return w;
 }
-static TapeB carve_tape_b(uint8_t* base, long long rows, long long pts, int C, int H, int nb, int CL) {
+static TapeB carve_tape_b(uint8_t* base, long long rows, long long pts, int C, int H, int nb, int CL, bool vmax) {
   TapeB t = {};
   size_t off = 0;
   auto take = [&](size_t bytes) { uint8_t* p = base ? base + off : nullptr; off += (bytes + 1023) & ~(size_t)1023; return p; };
@@ -711,6 +759,7 @@ static TapeB carve_tape_b(uint8_t* base, long long rows, long long pts, int C, i
   for (int b = CL; b < nb; ++b) t.RNM[b] = (__nv_bfloat16*)take((size_t)pts * H * 2);
   t.x = (float*)take((size_t)rows * H * 4);
   t.xm = (float*)take((size_t)pts * H * 4);
+  if (vmax) t.arg = take((size_t)pts * H);
   t.wpack = take(wpack_layout(C, 64, H, nb, CL, false).total);
   t.bytes = off + 1024;
   return t;
@@ -745,7 +794,7 @@ static int forward_bf16(const pnr_scene* sc, const pnr_points* q, const pnr_mlp_
                         float freq_factor, cudaStream_t st) {
   const long long rows = (long long)sc->SB * sc->NS * q->P, pts = (long long)sc->SB * q->P;
   const int H = mp->d_hidden, C = sc->C, d_in = mp->d_in, nb = mp->n_blocks, CL = mp->combine_layer;
-  const TapeB t = carve_tape_b(align1k(tape), rows, pts, C, H, nb, CL);
+  const TapeB t = carve_tape_b(align1k(tape), rows, pts, C, H, nb, CL, pool_max(sc, mp));
   const WPack w = wpack_layout(C, 64, H, nb, CL, false);
   int launches = 0, rc;
   // gather: latent rows straight to bf16; z-features via an fp32 scratch (the x buffer, not yet in use) then padded to K = 64
@@ -772,7 +821,7 @@ static int forward_bf16(const pnr_scene* sc, const pnr_points* q, const pnr_mlp_
   }
   {
     const long long n = pts * H / 4;
-    view_mean_bf16_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(t.x, t.xm, t.RXM[CL], sc->SB, sc->NS, q->P, H);      // util.py:489-499
+    view_mean_bf16_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(t.x, t.xm, t.RXM[CL], t.arg, sc->SB, sc->NS, q->P, H);  // util.py:489-499
     PNR_CHECK_LAUNCH("bwd::view_mean_bf16_kernel");
     ++launches;
   }
@@ -812,7 +861,7 @@ static int backward_bf16(const pnr_scene* sc, const pnr_points* q, const pnr_mlp
                          int num_freqs, float freq_factor, cudaStream_t st) {
   const long long rows = (long long)sc->SB * sc->NS * q->P, pts = (long long)sc->SB * q->P;
   const int H = mp->d_hidden, C = sc->C, d_in = mp->d_in, nb = mp->n_blocks, CL = mp->combine_layer, NS = sc->NS;
-  const TapeB t = carve_tape_b(align1k(const_cast<void*>(tape)), rows, pts, C, H, nb, CL);
+  const TapeB t = carve_tape_b(align1k(const_cast<void*>(tape)), rows, pts, C, H, nb, CL, pool_max(sc, mp));
   const BwdWsB ws = carve_bwd_b(align1k(workspace), rows, pts, C, d_in, H, nb, CL);
   const WPack w = wpack_layout(C, 64, H, nb, CL, true);
   int launches = 0, rc;
@@ -832,7 +881,8 @@ static int backward_bf16(const pnr_scene* sc, const pnr_points* q, const pnr_mlp
   // Bias gradients are column sums of the gradient g_b that ENTERS block b from above (= leaves block b + 1 downwards):
   //   d fc_1.bias[b] = colsum(g_{b+1}),  d lin_z.bias[b] = d lin_in.bias (b = 0) = colsum(g_b).
   // Each is accumulated by the epilogue that produces the tensor (lin_out_bwd for g_nb, the dx GEMM of block b for g_b); the
-  // view-mean transpose preserves column sums (sum over views of g / NS), so g_CL's sum is taken in the post-combine space.
+  // view-pooling transpose preserves column sums (mean: sum over views of g / NS; max: all of g goes to one view), so g_CL's sum
+  // is taken in the post-combine space.
   // One residual block backwards (resnetfc.py:53-62); dx (fp32 master + bf16 operand copy) is updated in place.
   auto block_bwd = [&](const __nv_bfloat16* RXb, const __nv_bfloat16* RNb, int b, float* dx, long long M) -> int {
     STEP(tg::wgrad(ws.dx16, H, RNb, H, gr->fc1_w[b], H, M, H, H, st));                          // dW1 += dx^T relu(net)
@@ -851,7 +901,7 @@ static int backward_bf16(const pnr_scene* sc, const pnr_points* q, const pnr_mlp
     if ((rc = block_bwd(t.RXM[b], t.RNM[b], b, ws.dxm, pts))) return rc;
   {
     const long long n4 = rows * H / 4;
-    view_mean_bwd_bf16_kernel<<<(unsigned)((n4 + 255) / 256), 256, 0, st>>>(ws.dxm, ws.dx, ws.dx16, sc->SB, NS, q->P, H);
+    view_mean_bwd_bf16_kernel<<<(unsigned)((n4 + 255) / 256), 256, 0, st>>>(ws.dxm, ws.dx, ws.dx16, t.arg, sc->SB, NS, q->P, H);
     PNR_CHECK_LAUNCH("bwd::view_mean_bwd_bf16_kernel");
     ++launches;
   }
@@ -891,8 +941,9 @@ using namespace pnr::bwd;
 extern "C" size_t pnr_field_tape_bytes(const pnr_scene* sc, const pnr_points* q, const pnr_mlp_params* mp) {
   if (!sc || !q || !mp) return 0;
   const long long rows = (long long)sc->SB * sc->NS * q->P, pts = (long long)sc->SB * q->P;
-  if (sc->flags & PNR_SCENE_TRAIN_BF16) return carve_tape_b(nullptr, rows, pts, sc->C, mp->d_hidden, mp->n_blocks, mp->combine_layer).bytes;
-  return carve_tape(nullptr, rows, pts, sc->C, mp->d_in, mp->d_hidden, mp->n_blocks, mp->combine_layer).floats * sizeof(float) + 256;
+  const bool vmax = pool_max(sc, mp);
+  if (sc->flags & PNR_SCENE_TRAIN_BF16) return carve_tape_b(nullptr, rows, pts, sc->C, mp->d_hidden, mp->n_blocks, mp->combine_layer, vmax).bytes;
+  return carve_tape(nullptr, rows, pts, sc->C, mp->d_in, mp->d_hidden, mp->n_blocks, mp->combine_layer, vmax).floats * sizeof(float) + 256;
 }
 
 extern "C" int pnr_field_forward_train(const pnr_scene* sc, const pnr_points* q, const pnr_mlp_params* mp, float* out,
@@ -906,7 +957,7 @@ extern "C" int pnr_field_forward_train(const pnr_scene* sc, const pnr_points* q,
   if (sc->flags & PNR_SCENE_TRAIN_BF16) return forward_bf16(sc, q, mp, out, tape, num_freqs, freq_factor, (cudaStream_t)stream);
   const int H = mp->d_hidden, C = sc->C, d_in = mp->d_in, nb = mp->n_blocks, CL = mp->combine_layer;
   cudaStream_t st = (cudaStream_t)stream;
-  const Tape t = carve_tape((float*)tape, rows, pts, C, d_in, H, nb, CL);
+  const Tape t = carve_tape((float*)tape, rows, pts, C, d_in, H, nb, CL, pool_max(sc, mp));
   int launches = 0;
   rc = pnr_gather_encode(sc, q, t.lat, t.zf, 1, num_freqs, freq_factor, stream);
   if (rc) return rc;
@@ -920,7 +971,7 @@ extern "C" int pnr_field_forward_train(const pnr_scene* sc, const pnr_points* q,
   }
   {
     const long long n = pts * H;
-    view_mean_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(t.X[CL], t.XM[CL], sc->SB, sc->NS, q->P, H);  // util.py:489-499
+    view_mean_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(t.X[CL], t.XM[CL], t.ARG, sc->SB, sc->NS, q->P, H);  // util.py:489-499
     PNR_CHECK_LAUNCH("bwd::view_mean_kernel");
     ++launches;
   }
@@ -963,7 +1014,7 @@ extern "C" int pnr_field_backward(const pnr_scene* sc, const pnr_points* q, cons
     return backward_bf16(sc, q, mp, tape, out, d_out, gr, d_feat, d_xyz, d_z, workspace, num_freqs, freq_factor, (cudaStream_t)stream);
   const int H = mp->d_hidden, C = sc->C, d_in = mp->d_in, nb = mp->n_blocks, CL = mp->combine_layer, NS = sc->NS;
   cudaStream_t st = (cudaStream_t)stream;
-  const Tape t = carve_tape((float*)const_cast<void*>(tape), rows, pts, C, d_in, H, nb, CL);
+  const Tape t = carve_tape((float*)const_cast<void*>(tape), rows, pts, C, d_in, H, nb, CL, pool_max(sc, mp));
   float* dA = (float*)workspace;            // current dx
   float* dB = dA + rows * H;                // dnet / scratch
   float* dlat = dB + rows * H;
@@ -996,7 +1047,7 @@ extern "C" int pnr_field_backward(const pnr_scene* sc, const pnr_points* q, cons
     if ((rc = block_bwd(t.XM[b], t.NETM[b], b, dA, dB, pts))) return rc;
   {
     const long long n = rows * H;
-    view_mean_bwd_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(dA, dB, sc->SB, NS, q->P, H);
+    view_mean_bwd_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(dA, dB, t.ARG, sc->SB, NS, q->P, H);
     PNR_CHECK_LAUNCH("bwd::view_mean_bwd_kernel");
     ++launches;
     float* tmp = dA; dA = dB; dB = tmp;

@@ -15,7 +15,7 @@ constexpr size_t kPackHeader = 1024;
 
 struct Sched {
   int n_blocks;   // ResnetFC blocks
-  int CL;         // block index before which the view mean happens (combine_layer), < n_blocks
+  int CL;         // block index before which the views are pooled (combine_layer); == n_blocks: no pooling (NS == 1 only)
   int n_linz;     // min(combine_layer, n_blocks)
   int KBz;        // d_latent / 64
 };
@@ -65,8 +65,10 @@ static int make_sched(const pnr_mlp_params* p, Sched* s, const char* who) {
   PNR_REQUIRE(p->d_in > 0 && p->d_in <= 64, PNR_ERR_UNSUPPORTED, "%s: d_in=%d must be in (0,64]", who, p->d_in);
   PNR_REQUIRE(p->d_latent > 0 && p->d_latent % 64 == 0, PNR_ERR_UNSUPPORTED, "%s: d_latent=%d must be a positive multiple of 64", who, p->d_latent);
   PNR_REQUIRE(p->n_blocks >= 1 && p->n_blocks <= 8, PNR_ERR_UNSUPPORTED, "%s: n_blocks=%d", who, p->n_blocks);
-  PNR_REQUIRE(p->combine_layer >= 1 && p->combine_layer < p->n_blocks, PNR_ERR_UNSUPPORTED,
-              "%s: combine_layer=%d must be in [1, n_blocks) for the fused path", who, p->combine_layer);
+  PNR_REQUIRE(p->combine_layer >= 1 && p->combine_layer <= p->n_blocks, PNR_ERR_ARG,
+              "%s: combine_layer=%d (pass min(combine_layer, n_blocks))", who, p->combine_layer);
+  PNR_REQUIRE(p->combine_type == PNR_COMBINE_AVERAGE || p->combine_type == PNR_COMBINE_MAX, PNR_ERR_ARG,
+              "%s: combine_type=%d", who, p->combine_type);
   PNR_REQUIRE(p->d_out >= 1 && p->d_out <= 32, PNR_ERR_UNSUPPORTED, "%s: d_out=%d", who, p->d_out);
   s->n_blocks = p->n_blocks; s->CL = p->combine_layer; s->n_linz = p->combine_layer; s->KBz = p->d_latent / 64;
   return PNR_OK;
@@ -93,6 +95,8 @@ int field_forward_umma(const pnr_scene* sc, const pnr_points* q, const pnr_mlp_p
   }
   PNR_REQUIRE(mp->d_in == 6 * num_freqs + 6, PNR_ERR_ARG, "field_forward_umma: d_in/num_freqs mismatch");
   PNR_REQUIRE(sc->NS >= 1 && sc->NS <= 8 && sc->NS != 7, PNR_ERR_UNSUPPORTED, "field_forward_umma: NS=%d source views", sc->NS);
+  PNR_REQUIRE(mp->combine_layer < mp->n_blocks || sc->NS == 1, PNR_ERR_UNSUPPORTED,
+              "field_forward_umma: combine_layer >= n_blocks never pools the views; only valid with one source view");
   if ((long long)sc->SB * q->P == 0) return PNR_OK;
   const PackOffsets po = pack_offsets(sch, mp, proj);
   const uint8_t* blob = (const uint8_t*)packed;

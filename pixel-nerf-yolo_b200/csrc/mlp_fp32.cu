@@ -74,8 +74,8 @@ sgemm_nt_kernel(const float* __restrict__ X, const float* __restrict__ W, const 
   }
 }
 
-// mean over the NS source views: x (SB, NS, P, H) -> (SB, P, H)          util.py:489-499
-__global__ void view_mean_kernel(const float* __restrict__ x, float* __restrict__ y, int SB, int NS, int P, int H) {
+// mean (combine_type average) or elementwise max (max) over the NS source views: x (SB, NS, P, H) -> (SB, P, H)   util.py:489-499
+__global__ void view_mean_kernel(const float* __restrict__ x, float* __restrict__ y, int SB, int NS, int P, int H, int vmax) {
   long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   long long n = (long long)SB * P * H;
   if (i >= n) return;
@@ -83,8 +83,15 @@ __global__ void view_mean_kernel(const float* __restrict__ x, float* __restrict_
   long long sp = i / H;
   int p = (int)(sp % P);
   int s = (int)(sp / P);
+  const float* xv = x + ((long long)s * NS * P + p) * H + h;
+  if (vmax) {
+    float m = xv[0];
+    for (int v = 1; v < NS; ++v) m = fmaxf(m, xv[(long long)v * P * H]);
+    y[i] = m;
+    return;
+  }
   float acc = 0.f;
-  for (int v = 0; v < NS; ++v) acc += x[(((long long)s * NS + v) * P + p) * H + h];
+  for (int v = 0; v < NS; ++v) acc += xv[(long long)v * P * H];
   y[i] = acc / (float)NS;
 }
 
@@ -132,9 +139,9 @@ static int resnetfc_chain(const pnr_mlp_params* mp, const float* lat, int ld_lat
   float* cur = x;
   long long cur_rows = rows;
   for (int b = 0; b < mp->n_blocks; ++b) {
-    if (b == mp->combine_layer) {                                                             // view mean
+    if (b == mp->combine_layer) {                                                             // view pooling
       long long n = pts * H;
-      view_mean_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(x, xm, SB, NS, P, H);
+      view_mean_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(x, xm, SB, NS, P, H, mp->combine_type == PNR_COMBINE_MAX);
       PNR_CHECK_LAUNCH("view_mean_kernel");
       cur = xm; cur_rows = pts; ++*launches;
     }
@@ -163,7 +170,9 @@ static int check_mlp(const pnr_mlp_params* mp, int NS, const char* who) {
   PNR_REQUIRE(mp->combine_layer >= 1 && mp->combine_layer <= mp->n_blocks, PNR_ERR_ARG,
               "%s: combine_layer=%d (pass min(combine_layer, n_blocks))", who, mp->combine_layer);
   PNR_REQUIRE(mp->combine_layer < mp->n_blocks || NS == 1, PNR_ERR_UNSUPPORTED,
-              "%s: combine_layer >= n_blocks never averages the views; only valid with one source view", who);
+              "%s: combine_layer >= n_blocks never pools the views; only valid with one source view", who);
+  PNR_REQUIRE(mp->combine_type == PNR_COMBINE_AVERAGE || mp->combine_type == PNR_COMBINE_MAX, PNR_ERR_ARG,
+              "%s: combine_type=%d", who, mp->combine_type);
   PNR_REQUIRE(mp->d_out >= 1 && mp->d_out <= 64, PNR_ERR_UNSUPPORTED, "%s: d_out=%d", who, mp->d_out);
   return PNR_OK;
 }

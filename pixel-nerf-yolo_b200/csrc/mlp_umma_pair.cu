@@ -321,10 +321,13 @@ constexpr int kTraceLen = 16384;
 #define PPROF_ADD(slot) do { if (prof && lane == 0) prof[slot] += clock64() - t0__; } while (0)
 
 // Work unit of a CTA pair = a "super group": G = 64 / PP consecutive tile pairs.
-//   pre-combine  (G times): tile of PP points x NS views per CTA: gather, lin_in, lin_z, blocks [0, CL), view mean
-//                -> x-bar (fp32, bias folded in) into this pair's private scratch (L2-resident, 256 KiB per pair);
+//   pre-combine  (G times): tile of PP points x NS views per CTA: gather, lin_in, lin_z, blocks [0, CL), view pooling
+//                (mean, or elementwise max when VMAX) -> x-bar (fp32, bias folded in) into this pair's private scratch
+//                (L2-resident, 256 KiB per pair);
 //   post-combine (once)   : the G x PP (<= 64) points each CTA gathered form ONE 64-column tile: x-bar -> TMEM,
 //                blocks [CL, n_blocks), lin_out, sigmoid/relu.
+// Without pooling (CL == n_blocks, NS == 1 only: G = 1) the pre-combine part runs every block and the post-combine part is
+// lin_out alone on relu(x-bar).
 // So every MMA of the kernel runs at N = 128, and the post-combine layers need 1/G of the weight passes and
 // epilogue hand-offs per point that a per-tile post phase would.
 //
@@ -335,7 +338,8 @@ constexpr int kTraceLen = 16384;
 // landing in the non-leader are counted on its B_LAND barrier, and its otherwise idle warp 1 relays that to the leader.
 // PROF = true compiles the per-role cycle counters in (PNR_PROF=1 selects that instantiation); the production instantiation
 // carries none of their branches -- the single-thread MMA issue loop is sensitive to every extra instruction.
-template <int NS, bool ASYNC, int PROF>   // PROF: 0 production, 1 per-role cycle counters (PNR_PROF), 2 event log of pair 0 only (PNR_TRACE)
+// PROF: 0 production, 1 per-role cycle counters (PNR_PROF), 2 event log of pair 0 only (PNR_TRACE).  VMAX: combine_type "max".
+template <int NS, bool ASYNC, int PROF, bool VMAX = false>
 __global__ void __launch_bounds__(kThreads, 1)
 field_pair_kernel(const pnr_scene sc, const pnr_points q, const __grid_constant__ CUtensorMap wmap,
                   const float* __restrict__ bias_x, const float* __restrict__ bias_h,
@@ -347,6 +351,7 @@ field_pair_kernel(const pnr_scene sc, const pnr_points q, const __grid_constant_
   constexpr int PP = kNCol / NS;                       // points per pre-combine tile
   constexpr int G = kNCol / PP;                        // pre-combine tile pairs per super group
   constexpr int NLIVE = G * PP;                        // live columns of a post-combine tile (<= 64)
+  const bool pooled = NS > 1 || sch.CL < sch.n_blocks;   // false: no block after the combine step, lin_out follows it
   const int n_sg = ((n_tiles + 1) / 2 + G - 1) / G;
   float* const xbar = xbar_all + (size_t)pair_id * (2 * kNCol * kHidden);   // [tile slot 2][column 64][feature 512]
   extern __shared__ __align__(1024) uint8_t smem[];
@@ -682,7 +687,8 @@ field_pair_kernel(const pnr_scene sc, const pnr_points q, const __grid_constant_
         for (int mt = 0; mt < kMT; ++mt) bias_mean[mt] = __ldg(bias_x + sch.CL * kHidden + mt * 256 + (int)crank * 128 + fl);
         for (int mt = 0; mt < kMT; ++mt) wait(B_X_FULL + mt);
         if (order3 && crank == 0 && sch.CL > 0) wait(B_C0_FREE);      // keep the phase in step (the last fc_1 signalled it too)
-        // view mean (combine_interleaved) + cumulative bias -> x-bar, column g*PP + p of slot hs
+        // view pooling (combine_interleaved) + cumulative bias -> x-bar, column g*PP + p of slot hs.  max(x_v + b) = max(x_v) + b
+        // exactly: rounding is monotonic
 #pragma unroll
         for (int mt = 0; mt < kMT; ++mt) {
           const int f = mt * 256 + (int)crank * 128 + fl;
@@ -697,11 +703,19 @@ field_pair_kernel(const pnr_scene sc, const pnr_points q, const __grid_constant_
           float* dst = xbar + ((size_t)hs * kNCol + g * PP) * kHidden + f;
 #pragma unroll
           for (int p = 0; p < PP; ++p) {
-            float acc = 0.f;
+            float pooled_x;
+            if constexpr (VMAX) {
+              pooled_x = __uint_as_float(v[p]);
 #pragma unroll
-            for (int vw = 0; vw < NS; ++vw) acc += __uint_as_float(v[vw * PP + p]);
+              for (int vw = 1; vw < NS; ++vw) pooled_x = fmaxf(pooled_x, __uint_as_float(v[vw * PP + p]));
+            } else {
+              float acc = 0.f;
+#pragma unroll
+              for (int vw = 0; vw < NS; ++vw) acc += __uint_as_float(v[vw * PP + p]);
+              pooled_x = __fdiv_rn(acc, (float)NS);
+            }
             const bool ok = live && p0 + p < q.P;
-            __stcg(dst + (size_t)p * kHidden, ok ? __fdiv_rn(acc, (float)NS) + bias : 0.f);
+            __stcg(dst + (size_t)p * kHidden, ok ? pooled_x + bias : 0.f);
           }
         }
       }
@@ -732,7 +746,7 @@ field_pair_kernel(const pnr_scene sc, const pnr_points q, const __grid_constant_
         }
         publish(kc);
       }
-      h_epilogue(sch.CL);
+      if (pooled) h_epilogue(sch.CL);
       for (int e = sch.CL + 1; e <= sch.n_blocks; ++e) {
         x_epilogue(e, true);
         if (e < sch.n_blocks) h_epilogue(e);
@@ -1006,6 +1020,10 @@ int field_forward_pair(const pnr_scene* sc, const pnr_points* q, const pnr_mlp_p
   cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
   const int G = pair::kNCol / PP;                        // tile pairs per super group (see field_pair_kernel)
   const bool async_x = pair_async();
+  // max over one view is the view itself: NS == 1 runs the average instantiation whatever combine_type says
+  const bool vmax = mp->combine_type == PNR_COMBINE_MAX && sc->NS > 1;
+  PNR_REQUIRE(!vmax || (async_x && !getenv("PNR_TRACE") && !getenv("PNR_PROF")), PNR_ERR_UNSUPPORTED,
+              "field_forward_pair: the PNR_ASYNC=0 / PNR_PROF / PNR_TRACE instruments are built for combine_type average only");
   const int n_groups = ((n_tiles + 1) / 2 + G - 1) / G;  // super groups
   long long* prof_dev = nullptr;
   long long* trace_dev = nullptr;
@@ -1022,7 +1040,8 @@ int field_forward_pair(const pnr_scene* sc, const pnr_points* q, const pnr_mlp_p
   }
 #define PNR_LAUNCH_PAIR(NSV)                                                                                     \
   case NSV: {                                                                                                    \
-    auto kern = async_x ? (trace_dev ? pair::field_pair_kernel<NSV, true, 2> : prof_dev ? pair::field_pair_kernel<NSV, true, 1> : pair::field_pair_kernel<NSV, true, 0>) \
+    auto kern = vmax ? pair::field_pair_kernel<NSV, true, 0, (NSV > 1)>                                          \
+              : async_x ? (trace_dev ? pair::field_pair_kernel<NSV, true, 2> : prof_dev ? pair::field_pair_kernel<NSV, true, 1> : pair::field_pair_kernel<NSV, true, 0>) \
                         : pair::field_pair_kernel<NSV, false, 0>;                                           \
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pair::Smem::total); \
     PNR_REQUIRE(e == cudaSuccess, PNR_ERR_CUDA, "cudaFuncSetAttribute: %s", cudaGetErrorString(e));             \

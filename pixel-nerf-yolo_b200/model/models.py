@@ -87,7 +87,9 @@ class PixelNeRFNet(torch.nn.Module):
         self.use_code_viewdirs = conf.get_bool("use_code_viewdirs", True)
         self.use_viewdirs = conf.get_bool("use_viewdirs", False)
         self.use_global_encoder = conf.get_bool("use_global_encoder", False)
-        # The fused kernels implement the switch set of every shipped conf (conf/default*.conf, conf/exp/*.conf).
+        # The fused kernels implement the switch set of every shipped conf (conf/default*.conf, conf/exp/*.conf), and both
+        # view-pooling modes of ResnetFC: combine_type average / max before block combine_layer, or no pooling at all
+        # (combine_layer >= n_blocks, the single-view conf/default.conf network; one source view only).
         unsupported = []
         if not self.use_encoder: unsupported.append("use_encoder=False")
         if not self.use_xyz: unsupported.append("use_xyz=False")
@@ -152,8 +154,14 @@ class PixelNeRFNet(torch.nn.Module):
             poses = poses.reshape(-1, 4, 4)
         else:
             self.num_views_per_obj = 1
+        self._check_views()
         self.encoder(images, return_latent=False)
         self.set_cameras(poses, focal, (images.shape[-1], images.shape[-2]), c)
+
+    def _check_views(self):
+        for mlp in (self.mlp_coarse, self.mlp_fine):
+            if mlp is not None:
+                mlp.check_views(self.num_views_per_obj)
 
     def set_cameras(self, poses, focal, image_wh, c=None):
         """The camera half of ``encode`` (models.py:116-148) without running the encoder trunk."""
@@ -194,6 +202,7 @@ class PixelNeRFNet(torch.nn.Module):
         fp32 copy); ``cams`` re-uses the camera tensors captured at forward time."""
         n_views = self.poses.shape[0]
         NS = self.num_views_per_obj
+        self._check_views()
         SB = n_views // NS
         dev = self.poses.device
         if self._cam_cache is None:

@@ -34,8 +34,13 @@ class ResnetFC(nn.Module):
     def __init__(self, d_in, d_out, n_blocks=5, d_latent=0, d_hidden=128, beta=0.0, combine_layer=1000,
                  combine_type="average", use_spade=False):
         super().__init__()
-        if combine_type != "average":
-            raise NotImplementedError(f"ResnetFC: combine_type={combine_type!r} is not built (average only)")
+        if combine_type not in _lib.COMBINE_TYPES:
+            raise NotImplementedError(f"ResnetFC: combine_type={combine_type!r} is not built (average or max)")
+        if combine_type != "average" and combine_layer >= n_blocks:
+            # a network that never pools its views has no pooling step for the mode to select; only the reference's default
+            # ("average") is accepted there, so that a conf naming a mode it cannot apply is not silently ignored
+            raise NotImplementedError(f"ResnetFC: combine_type={combine_type!r} needs combine_layer < n_blocks "
+                                      f"(combine_layer={combine_layer}, n_blocks={n_blocks}: the views are never pooled)")
         if use_spade:
             raise NotImplementedError("ResnetFC: use_spade is not built")
         if beta > 0:
@@ -74,7 +79,18 @@ class ResnetFC(nn.Module):
             p.linz_w[i], p.linz_b[i] = f(lz.weight), f(lz.bias)
         p.d_in, p.d_latent, p.d_hidden, p.d_out = self.d_in, self.d_latent, self.d_hidden, self.d_out
         p.n_blocks, p.combine_layer = self.n_blocks, min(self.combine_layer, self.n_blocks)
+        p.combine_type = _lib.COMBINE_TYPES[self.combine_type]
         return p
+
+    def pools_views(self) -> bool:
+        """False for a network whose combine_layer is at or past its last block (conf/default.conf): it never pools the source
+        views, so it is only defined for one view per object."""
+        return self.combine_layer < self.n_blocks
+
+    def check_views(self, num_views: int) -> None:
+        if num_views > 1 and not self.pools_views():
+            raise NotImplementedError(f"ResnetFC: combine_layer={self.combine_layer} >= n_blocks={self.n_blocks} never pools the "
+                                      f"source views; it is only defined for one view per object (got {num_views})")
 
     def ordered_params(self):
         """Parameters in the fixed order the training-path autograd function passes them (and returns grads)."""
@@ -181,14 +197,15 @@ class ResnetFC(nn.Module):
         assert zx.size(-1) == self.d_latent + self.d_in
         if combine_index is not None:
             raise NotImplementedError("ResnetFC: combine_index (frustum culling) is not built")
-        _lib.require_cuda(zx, "ResnetFC input")
-        _lib.require_device(zx.device)
-        zx2 = zx.reshape(-1, zx.size(-1)).contiguous().float()
-        rows = zx2.shape[0]
+        rows = zx.numel() // zx.size(-1)
         if len(combine_inner_dims) == 1:
             ns, pts = 1, max(rows, 1)
         else:
             ns, pts = int(combine_inner_dims[0]), int(combine_inner_dims[1])
+        self.check_views(ns)
+        _lib.require_cuda(zx, "ResnetFC input")
+        _lib.require_device(zx.device)
+        zx2 = zx.reshape(-1, zx.size(-1)).contiguous().float()
         lib = _lib.load()
         cp = self.c_params()
         out = torch.empty(rows // ns, self.d_out, device=zx.device, dtype=torch.float32)
