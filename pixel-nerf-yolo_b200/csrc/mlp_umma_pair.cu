@@ -28,35 +28,16 @@
 #include "pnr_common.cuh"
 #include "umma.cuh"
 #include <cuda.h>
-#include <stdlib.h>
-#include <vector>
 
 namespace pnr {
 using namespace umma;
 
 namespace pair {
 
-// Timing diagnostics (WRONG RESULTS, scripts/build_diag_variants.sh): PNR_DIAG_MMAONLY = the MMA thread's instruction stream alone;
-// its parts can be switched off one by one: OFF_RING (no weight stream, no W_FULL wait), OFF_WAITS (the MMA thread waits for no
-// epilogue / gather barrier), OFF_EPI (no epilogue / relay warps), OFF_GATHER (no gather warps).
-#ifdef PNR_DIAG_MMAONLY
-#define PNR_DIAG_OFF_RING
-#define PNR_DIAG_OFF_WAITS
-#define PNR_DIAG_OFF_EPI
-#define PNR_DIAG_OFF_GATHER
-#endif
-#ifdef PNR_DIAG_NORING
-#define PNR_DIAG_OFF_RING
-#define PNR_DIAG_OFF_EMPTY_COMMIT
-#endif
-
 constexpr int kNCol = 64;                    // columns per CTA tile
 constexpr int kMT = 2;                       // 256-feature tiles per 512-wide layer
 constexpr int kKBlocksH = kHidden / kBlockK; // 8
-#ifndef PNR_STAGES
-#define PNR_STAGES 5
-#endif
-constexpr int kStages = PNR_STAGES;   // weight ring depth (16 KiB each); -DPNR_STAGES=n builds an experiment
+constexpr int kStages = 5;                   // weight ring depth (16 KiB each): the most that fits the shared-memory budget
 constexpr int kThreads = 512;
 constexpr int kProducers = 3;                // warps 0,12,13
 constexpr int kGatherWarps = 4;              // warps 2,3,14,15
@@ -67,7 +48,7 @@ constexpr int kTmemCols = 512;
 constexpr int kHCol = 256;
 constexpr int kMaxStages = 1024;
 
-struct Sched { int n_blocks, CL, n_linz, KBz, order, proj; };   // order: (chunk, tile) pair order inside a layer, see fc_pair;
+struct Sched { int n_blocks, CL, n_linz, KBz, proj; };
 // proj: the feature maps hold the lin_z pre-projections (512 channels per lin_z layer, PNR_SCENE_PROJECTED): every lin_z[b]
 // is an IDENTITY-weight accumulate of its own freshly gathered 512-channel slice (KBz = 8)
 enum { MAT_LIN_IN = 0, MAT_LINZ = 1, MAT_FC0 = 2, MAT_FC1 = 3, MAT_LIN_OUT = 4 };
@@ -82,40 +63,23 @@ __host__ __device__ inline int sched_total(const Sched& s) {
 __host__ __device__ inline int sched_pre(const Sched& s) { return kMT + s.n_linz * kMT * s.KBz + s.CL * 32; }
 // per-tile stage order = MMA issue order:
 //   lin_in (2) | lin_z[0] | per block: fc_0 (8 (chunk, tile) pairs x kk(2), see fc_pair) | lin_z[b+1] | fc_1 (same) | lin_out (8)
-// Order of the (K-chunk kc, feature tile mt) pairs inside a 512x512 layer.  Chunks 0,1 come from the previous
-// layer's tile 0 and arrive first, so both output tiles consume them first; then tile 0 is finished (its
-// completion is signalled on its own barrier, so its epilogue overlaps the last two pairs), then tile 1.
-// order 2 (default) additionally starts with the ODD chunk of each pair of chunks: odd chunks are produced by the non-leader
-// CTA and their remote rows land in the leader, on the very barrier the MMA warp waits on, while even chunks need the relay
-// hop from the non-leader (asynchronous exchange) -- that hop then overlaps the MMAs of the odd chunk.
+// Order of the (K-chunk kc, feature tile mt) pairs inside a 512x512 layer: (c1,t0)(c0,t0)(c1,t1)(c0,t1)(c3,t0)(c2,t0)(c3,t1)(c2,t1).
+// Chunks 0,1 come from the previous layer's tile 0 and arrive first, so both output tiles consume them first; then tile 0 is
+// finished (its completion is signalled on its own barrier, so its epilogue overlaps the last two pairs), then tile 1.
+// Each pair of chunks starts with its ODD chunk: odd chunks are produced by the non-leader CTA and their remote rows land in
+// the leader, on the very barrier the MMA warp waits on, while even chunks need the relay hop from the non-leader -- that hop
+// then overlaps the MMAs of the odd chunk.
 // first / last: this is the first / last (k-block of the) pair that touches output tile mt.
-__host__ __device__ inline void fc_pair(int order, int t, int& kc, int& mt, int& kk, bool& first, bool& last) {
+__host__ __device__ inline void fc_pair(int t, int& kc, int& mt, int& kk, bool& first, bool& last) {
   const int pr = t >> 1;                       // 0..7
   kk = t & 1;
-  if (order == 0) {                            // K-chunk outer: (c0,t0)(c0,t1)(c1,t0)...
-    kc = pr >> 1; mt = pr & 1;
-    first = pr < 2 && kk == 0; last = pr >= 6 && kk == 1;
-    return;
-  }
-  if (order == 3) {
-    // (c1,t0)(c0,t0)(c1,t1)(c3,t0)(c2,t0)(c0,t1)(c3,t1)(c2,t1): tile 0 is complete after FIVE pairs and tile 1 three pairs later.
-    // With hand-off latency H and P cycles per pair a layer's period is H + max(a, 10 - a) P when tile 0 completes after a
-    // pairs (chunks 2, 3 of the next layer become ready (8 - a) P after chunks 0, 1 and are first needed (a - 2) P after them):
-    // a = 5 is the minimum, one pair less than orders 1 / 2 (a = 6).
-    kc = (int)((0x23023101u >> (4 * pr)) & 0xFu);   // 1,0,1,3,2,0,3,2 (nibble pr)
-    mt = (int)((0xE4u >> pr) & 1u);                  // 0,0,1,0,0,1,1,1
-    first = (pr == 0 || pr == 2) && kk == 0;
-    last = (pr == 4 || pr == 7) && kk == 1;
-    return;
-  }
-  kc = (pr < 4) ? (pr & 1) : (2 + (pr & 1));   // (c0,t0)(c1,t0)(c0,t1)(c1,t1)(c2,t0)(c3,t0)(c2,t1)(c3,t1)
-  if (order == 2) kc ^= 1;                     // (c1,t0)(c0,t0)(c1,t1)(c0,t1)(c3,t0)(c2,t0)(c3,t1)(c2,t1)
+  kc = ((pr < 4) ? (pr & 1) : (2 + (pr & 1))) ^ 1;
   mt = (pr >> 1) & 1;
   first = (pr == 0 || pr == 2) && kk == 0;
   last = (pr == 5 || pr == 7) && kk == 1;
 }
-// chunk order of lin_out (one output tile): 0,1,2,3 or, for order 2, 1,0,3,2
-__host__ __device__ inline int out_chunk(int order, int t) { return order >= 2 ? ((t >> 1) ^ 1) : (t >> 1); }
+// chunk order of lin_out (one output tile): 1,0,3,2, odd chunk first as in fc_pair
+__host__ __device__ inline int out_chunk(int t) { return (t >> 1) ^ 1; }
 __host__ __device__ inline Seg walk_stage(const Sched& sc, int s) {
   Seg g;
   const int s1 = kMT * sc.KBz;
@@ -155,8 +119,8 @@ __host__ __device__ inline StageSrc decode_stage(const Sched& sc, int s) {
     case MAT_LIN_IN: r.row0 = g.t * 256; r.k0 = 0; break;
     case MAT_LINZ: { const ZPos z = z_position(sc.KBz, g.t); r.row0 = z.mt * 256; r.k0 = (z.pass * 8 + z.kbi) * 64; } break;
     case MAT_FC0:
-    case MAT_FC1: { int kc, mt, kk; bool f, l; fc_pair(sc.order, g.t, kc, mt, kk, f, l); r.row0 = mt * 256; r.k0 = kc * 128 + kk * 64; } break;
-    default: r.row0 = 0; r.k0 = out_chunk(sc.order, g.t) * 128 + (g.t & 1) * 64; break;
+    case MAT_FC1: { int kc, mt, kk; bool f, l; fc_pair(g.t, kc, mt, kk, f, l); r.row0 = mt * 256; r.k0 = kc * 128 + kk * 64; } break;
+    default: r.row0 = 0; r.k0 = out_chunk(g.t) * 128 + (g.t & 1) * 64; break;
   }
   return r;
 }
@@ -198,7 +162,6 @@ enum {
   B_RDY = B_H_FULL + kMT, B_X_FREE = B_RDY + 4,  // one per feature tile: the view-mean epilogue has read x tile mt out of TMEM
   B_LAND = B_X_FREE + kMT,                                       // non-leader CTA only: remote rows of chunk 2*i have landed (st.async bytes)
   B_OUT_FREE = B_LAND + kMT,                    // leader: the output epilogue has read lin_out's result out of the h region
-  B_C0_FREE,                                    // order 3 only: the layer's last MMAs reading chunk 0 ((c0, t1), issued AFTER tile 0 is complete) are done
   B_COUNT
 };
 static_assert(B_COUNT <= 30, "barrier parity bits live in one 32-bit word");
@@ -227,16 +190,15 @@ __device__ inline ProgEntry make_prog(const Sched& sc, int s, uint32_t sbase) {
     case MAT_FC1: {
       int kc, mt, kk;
       bool first_of_tile, last_of_tile;
-      fc_pair(sc.order, g.t, kc, mt, kk, first_of_tile, last_of_tile);
+      fc_pair(g.t, kc, mt, kk, first_of_tile, last_of_tile);
       const bool fc0 = g.kind == MAT_FC0;
       b_addr = sbase + Smem::ring + (kc * 2 + kk) * kOperandKB; dcol = (fc0 ? kHCol : 0) + mt * 128;
       if (fc0) acc = first_of_tile ? 0 : 1;                      // fc_1 always accumulates into x
       if (mt == 0 && kk == 0) wait_id = B_RDY + kc + 1;          // first use of chunk kc (tile 0 precedes tile 1 for every chunk)
       if (last_of_tile) c2 = (fc0 ? B_H_FULL : B_X_FULL) + mt + 1;   // tile mt complete
-      if (sc.order == 3 && g.t == 11) c1 = B_C0_FREE + 1;          // pair 5 = (c0, t1): chunk buffer 0 may be overwritten
     } break;
     default: {
-      const int kc = out_chunk(sc.order, g.t), kk = g.t % 2;
+      const int kc = out_chunk(g.t), kk = g.t % 2;
       b_addr = sbase + Smem::ring + (kc * 2 + kk) * kOperandKB; dcol = kHCol; acc = g.t > 0;
       if (kk == 0) wait_id = B_RDY + kc + 1;
       if (last) c2 = B_H_FULL + 1;
@@ -266,7 +228,7 @@ __device__ __forceinline__ uint32_t pack_relu_bf16x2(float lo, float hi) {
 
 template <int NC, bool REMOTE, bool ADD_BIAS>
 __device__ __forceinline__ void store_transposed(uint32_t base, const uint32_t* vals, float bias, int lane, int kq, int row0,
-                                                 uint32_t async_bar = 0) {   // != 0: remote rows go out as st.async counted on that barrier
+                                                 uint32_t async_bar = 0) {   // REMOTE: the rows go out as st.async counted on that barrier
   const int g = lane >> 3, i = lane & 7;
   const int k = kq + 8 * g;                                     // first of the 8 features this lane stores, within the chunk
   const uint32_t kb_off = (uint32_t)(k >> 6) * kOperandKB;
@@ -275,10 +237,6 @@ __device__ __forceinline__ void store_transposed(uint32_t base, const uint32_t* 
     // pair column j with column j+8: after the transpose lane i owns rows c0+i and c0+8+i, whose (row & 7) differ
     // across the 8 lanes of a group -> the swizzled 16-byte stores of a quarter warp hit 8 different bank groups
     uint32_t p[8];
-#ifdef PNR_DIAG_EPI_NOALU   // timing diagnostic only (wrong results): the epilogue's stores without its arithmetic / TMEM reads
-#pragma unroll
-    for (int j = 0; j < 8; ++j) p[j] = (uint32_t)(lane + j + c0);
-#else
 #pragma unroll
     for (int j = 0; j < 8; ++j) {
       float x = __uint_as_float(vals[c0 + j]), y = __uint_as_float(vals[c0 + 8 + j]);
@@ -286,39 +244,16 @@ __device__ __forceinline__ void store_transposed(uint32_t base, const uint32_t* 
       p[j] = pack_relu_bf16x2(x, y);
     }
     transpose8x8(p, lane);                                      // p[f] = (feature 8g+f at column c0+i, at column c0+8+i)
-#endif
     const uint32_t e0 = __byte_perm(p[0], p[1], 0x5410), e1 = __byte_perm(p[2], p[3], 0x5410);
     const uint32_t e2 = __byte_perm(p[4], p[5], 0x5410), e3 = __byte_perm(p[6], p[7], 0x5410);
     const uint32_t o0 = __byte_perm(p[0], p[1], 0x7632), o1 = __byte_perm(p[2], p[3], 0x7632);
     const uint32_t o2 = __byte_perm(p[4], p[5], 0x7632), o3 = __byte_perm(p[6], p[7], 0x7632);
     const uint32_t addr_e = base + kb_off + swz_offset(row0 + c0 + i, k & 63);
     const uint32_t addr_o = base + kb_off + swz_offset(row0 + c0 + 8 + i, k & 63);
-#ifdef PNR_DIAG_EPI_NOSTORE   // timing diagnostic only (wrong results): all of the epilogue's arithmetic, none of its stores
-    if ((e0 ^ e1 ^ e2 ^ e3 ^ o0 ^ o1 ^ o2 ^ o3) != 0x9E3779B9u) continue;
-#endif
-    if (REMOTE) {
-      if (async_bar) { st_async_v4(addr_e, e0, e1, e2, e3, async_bar); st_async_v4(addr_o, o0, o1, o2, o3, async_bar); }
-      else { st_cluster_v4(addr_e, e0, e1, e2, e3); st_cluster_v4(addr_o, o0, o1, o2, o3); }
-    } else { st_shared_v4(addr_e, e0, e1, e2, e3); st_shared_v4(addr_o, o0, o1, o2, o3); }
+    if (REMOTE) { st_async_v4(addr_e, e0, e1, e2, e3, async_bar); st_async_v4(addr_o, o0, o1, o2, o3, async_bar); }
+    else { st_shared_v4(addr_e, e0, e1, e2, e3); st_shared_v4(addr_o, o0, o1, o2, o3); }
   }
 }
-
-// optional per-role wait counters (PNR_PROF=1): [0] MMA total [1] wait weights [2] wait gather [4] wait relu(x) chunk
-// [5] wait relu(h) chunk [6] blocked in issue | [8] epilogue total [9] wait x_full [10] wait h_full [11] wait ax_free
-// [12] wait ah_free | [16] gather total [17] wait in_free    (leader CTA's MMA warp; warp 4 and warp 2 of every CTA)
-__device__ long long* g_prof_pair = nullptr;
-// optional event log of CTA pair 0 (PNR_TRACE=<file>, PROF instantiation only): role r writes (clock64 << 8 | tag) entries to
-// g_trace_pair[r * kTraceLen + n].  Roles: 0 MMA thread, 1 / 2 epilogue warp 4 of CTA 0 / 1, 3 relay, 4 gather warp 2 of CTA 0, 5..7 / 8..10 weight producers of CTA 0 / CTA 1
-// (0x84 = TMA issued).
-// Tags: 0x10+id wait for barrier id begins, 0x40+id wait satisfied, 0x01..0x04 commit of X_FULL[0], X_FULL[1], H_FULL[0], H_FULL[1]
-// issued, 0x80 TMEM read done, 0x81 remote half stored, 0x82 local half stored, 0x83 published, 0xFF cluster start (clock alignment)
-__device__ long long* g_trace_pair = nullptr;
-__device__ int g_trace_stages = 0;      // PNR_TRACE_STAGES=1: also log every stage of the MMA thread (0x72 weights ready, 0x71 issued)
-constexpr int kTraceLen = 16384;
-#define PTRACE_L0(role_, tag_) do { if (lane == 0) PTRACE(role_, tag_); } while (0)
-#define PTRACE(role_, tag_) do { if (PROF == 2 && trace && n_tr < kTraceLen) trace[(role_) * kTraceLen + n_tr++] = (clock64() << 8) | (long long)(tag_); } while (0)
-#define PPROF_T0() const long long t0__ = prof ? clock64() : 0
-#define PPROF_ADD(slot) do { if (prof && lane == 0) prof[slot] += clock64() - t0__; } while (0)
 
 // Work unit of a CTA pair = a "super group": G = 64 / PP consecutive tile pairs.
 //   pre-combine  (G times): tile of PP points x NS views per CTA: gather, lin_in, lin_z, blocks [0, CL), view pooling
@@ -331,15 +266,13 @@ constexpr int kTraceLen = 16384;
 // So every MMA of the kernel runs at N = 128, and the post-combine layers need 1/G of the weight passes and
 // epilogue hand-offs per point that a per-tile post phase would.
 //
-// Epilogue exchange, ASYNC = true: the half of every epilogue unit that belongs to the peer CTA goes out as st.async
-// (16 bytes per store, counted on an mbarrier of the DESTINATION CTA), so the epilogue warps no longer sit in
-// fence.proxy.async.shared::cluster waiting for their remote rows to be performed (14.5 % of all warp-stall samples of the
-// synchronous version).  Rows landing in the leader are counted directly on the chunk barrier the MMA warp waits on; rows
-// landing in the non-leader are counted on its B_LAND barrier, and its otherwise idle warp 1 relays that to the leader.
-// PROF = true compiles the per-role cycle counters in (PNR_PROF=1 selects that instantiation); the production instantiation
-// carries none of their branches -- the single-thread MMA issue loop is sensitive to every extra instruction.
-// PROF: 0 production, 1 per-role cycle counters (PNR_PROF), 2 event log of pair 0 only (PNR_TRACE).  VMAX: combine_type "max".
-template <int NS, bool ASYNC, int PROF, bool VMAX = false>
+// Epilogue exchange: the half of every epilogue unit that belongs to the peer CTA goes out as st.async (16 bytes per store,
+// counted on an mbarrier of the DESTINATION CTA), so the epilogue warps do not sit in fence.proxy.async.shared::cluster
+// waiting for their remote rows to be performed (14.5 % of all warp-stall samples of a synchronous exchange).  Rows landing
+// in the leader are counted directly on the chunk barrier the MMA warp waits on; rows landing in the non-leader are counted
+// on its B_LAND barrier, and its otherwise idle warp 1 relays that to the leader.
+// VMAX: combine_type "max".
+template <int NS, bool VMAX>
 __global__ void __launch_bounds__(kThreads, 1)
 field_pair_kernel(const pnr_scene sc, const pnr_points q, const __grid_constant__ CUtensorMap wmap,
                   const float* __restrict__ bias_x, const float* __restrict__ bias_h,
@@ -359,11 +292,6 @@ field_pair_kernel(const pnr_scene sc, const pnr_points q, const __grid_constant_
   volatile uint32_t* tmem_base_slot = reinterpret_cast<volatile uint32_t*>(smem + Smem::bars + 8 * B_COUNT);
   const int warp = __shfl_sync(0xffffffffu, (int)(threadIdx.x >> 5), 0);
   const int lane = threadIdx.x & 31;
-  long long* const prof = (PROF == 1 && g_prof_pair) ? reinterpret_cast<long long*>(smem + Smem::bars + 256) : nullptr;
-  if (prof && threadIdx.x < 32) prof[threadIdx.x] = 0;
-  long long* const trace = (PROF == 2 && g_trace_pair && (blockIdx.x >> 1) == 0) ? g_trace_pair : nullptr;
-  int n_tr = 0;
-  const bool trace_stages = PROF == 2 && trace && g_trace_stages;
   auto bar = [&](int i) -> uint32_t { return sbase + Smem::bars + 8u * i; };
   auto lbar = [&](int i) -> uint32_t { return mapa_u32(sbase + Smem::bars + 8u * i, 0); };   // the leader's copy
   if ((sbase & 1023u) != 0) { if (threadIdx.x == 0) printf("pnr: dynamic smem not 1024-aligned\n"); __trap(); }
@@ -373,11 +301,10 @@ field_pair_kernel(const pnr_scene sc, const pnr_points q, const __grid_constant_
     mbar_init(bar(B_IN_READY), 2 * kGatherWarps);
     mbar_init(bar(B_IN_FREE), 1);
     for (int i = 0; i < kMT; ++i) { mbar_init(bar(B_X_FULL + i), 1); mbar_init(bar(B_H_FULL + i), 1); }
-    // chunk kc is produced by CTA kc % 2; in ASYNC mode even chunks need one more arrival: the relay of the non-leader CTA
-    for (int i = 0; i < 4; ++i) mbar_init(bar(B_RDY + i), kEpiWarps + ((ASYNC && (i & 1) == 0) ? 1 : 0));
+    // chunk kc is produced by CTA kc % 2; even chunks need one more arrival: the relay of the non-leader CTA
+    for (int i = 0; i < 4; ++i) mbar_init(bar(B_RDY + i), kEpiWarps + ((i & 1) == 0 ? 1 : 0));
     for (int i = 0; i < kMT; ++i) mbar_init(bar(B_LAND + i), kEpiWarps);
     mbar_init(bar(B_OUT_FREE), 2);
-    mbar_init(bar(B_C0_FREE), 1);
     for (int i = 0; i < kMT; ++i) mbar_init(bar(B_X_FREE + i), 2 * kEpiWarps);
     fence_barrier_init();
   }
@@ -395,12 +322,7 @@ field_pair_kernel(const pnr_scene sc, const pnr_points q, const __grid_constant_
   cluster_sync_all();                    // both CTAs' barriers initialised and TMEM allocated before any remote signal
   tc_fence_after();
   const uint32_t tmem_base = __shfl_sync(0xffffffffu, *tmem_base_slot, 0);
-  if (warp == 4) PTRACE_L0(1 + (int)crank, 0xFF);
-#ifdef PNR_DIAG_N   // timing diagnostic only (wrong results): same instruction stream, less tensor work per MMA
-  const uint32_t idesc = instr_desc_bf16_2sm(PNR_DIAG_N);
-#else
   const uint32_t idesc = instr_desc_bf16_2sm(2 * kNCol);
-#endif
 
   if (warp == 0 || warp == 12 || warp == 13) {
     // ===================== weight producers: warp p streams global stages g = p (mod kProducers); each CTA loads its
@@ -413,23 +335,9 @@ field_pair_kernel(const pnr_scene sc, const pnr_points q, const __grid_constant_
         int fi = carry;
         int st = fi < G * s_pre ? fi % s_pre : fi - (G - 1) * s_pre;   // G passes over the pre stages, one over the post stages
         for (; fi < n_flat; fi += kProducers) {
-#ifdef PNR_DIAG_OFF_RING   // timing diagnostic only (wrong results): no weight ring at all
-          continue;
-#endif
-          PTRACE(5 + pid + 3 * (int)crank, 0x10 + B_W_EMPTY + slot);
-#if PNR_IDLE_WAIT
-          mbar_wait_idle(bar(B_W_EMPTY + slot), par);
-#else
           mbar_wait_cluster(bar(B_W_EMPTY + slot), par);
-#endif
-          PTRACE(5 + pid + 3 * (int)crank, 0x40 + B_W_EMPTY + slot);
-#ifdef PNR_DIAG_NOWEIGHTS   // timing diagnostic only (wrong results): the weight slot is declared full without loading anything
-          if (crank == 0) mbar_arrive(bar(B_W_FULL + slot));
-#else
           if (crank == 0) mbar_arrive_expect_tx(bar(B_W_FULL + slot), 2 * kStageBytes);
           tma_load_2d_2sm(sbase + Smem::w + slot * kStageBytes, &wmap, 0, (st * 2 + (int)crank) * kStageRows, bar(B_W_FULL + slot));
-#endif
-          PTRACE(5 + pid + 3 * (int)crank, 0x84);
           slot += kProducers;
           if (slot >= kStages) { slot -= kStages; par ^= 1; }
           // next stage id without a division: inside the pre passes the id wraps at s_pre, after them it just continues
@@ -448,7 +356,6 @@ field_pair_kernel(const pnr_scene sc, const pnr_points q, const __grid_constant_
       // issuing warp's own instruction stream is.  So the whole role is a single elected thread in a tight per-stage loop --
       // no ballot probe of the ring, no per-batch elect / __syncwarp: it polls the barriers itself (try_wait), issues the four
       // MMAs of the stage (~45 cycles) and its commits (~70 cycles), and prefetches the next program entry meanwhile.
-      const long long t_role0 = prof ? clock64() : 0;
       if (elect_one()) {
         uint32_t slot = 0, wpar = 0, ph = 0;
         uint32_t full_bar = bar(B_W_FULL), empty_bar = bar(B_W_EMPTY);      // running addresses of the current ring slot's barriers
@@ -457,30 +364,22 @@ field_pair_kernel(const pnr_scene sc, const pnr_points q, const __grid_constant_
         const uint64_t bdesc_hi = smem_desc(0);
         constexpr uint64_t kStageStep = kStageBytes >> 4;
         const uint2* prog = reinterpret_cast<const uint2*>(smem + Smem::prog);
-#define MPROF_T0() const long long t0__ = prof ? clock64() : 0
-#define MPROF_ADD(slot_) do { if (prof) prof[slot_] += clock64() - t0__; } while (0)
         for (int sg = pair_id; sg < n_sg; sg += n_pairs) {
           for (int seg = 0; seg <= G; ++seg) {              // G pre-combine passes, then the post-combine pass
             const bool after_mean = seg > 0 && seg < G;
             if (after_mean) {
               // the view-mean epilogue of the previous tile must have read x tile 0 out of TMEM before lin_in (stage 0) overwrites
               // it; tile 1 is first written by stage 1 (see below)
-              MPROF_T0();
-#ifndef PNR_DIAG_OFF_WAITS
               mbar_wait_cluster(bar(B_X_FREE), (ph >> B_X_FREE) & 1u);
-#endif
               ph ^= (1u << B_X_FREE);
               tc_fence_after();
-              MPROF_ADD(5);
             }
             const int st_beg = seg < G ? 0 : s_pre, st_end = seg < G ? s_pre : n_stages;
             if (seg == 0 && sg != pair_id) {
               // The previous super group's output epilogue (two warps of this CTA) reads lin_out's result from h tile 0; the first
               // fc_0 of this super group only waits for a chunk signalled by the OTHER CTA's warps (odd-chunk-first order).  In
               // practice that is thousands of cycles later; this wait (a few hundred cycles after lin_out at most) makes it explicit.
-#ifndef PNR_DIAG_OFF_WAITS
               mbar_wait(bar(B_OUT_FREE), (ph >> B_OUT_FREE) & 1u);
-#endif
               ph ^= (1u << B_OUT_FREE);
             }
             uint2 cur = prog[st_beg];
@@ -489,40 +388,23 @@ field_pair_kernel(const pnr_scene sc, const pnr_points q, const __grid_constant_
               const uint2 nxt = prog[st + 1];               // in flight while this stage is issued (the program is padded by one entry)
               const uint32_t wait_id = cur.x >> 25;
               if (wait_id) {
-                MPROF_T0();
                 const uint32_t id = wait_id - 1;
-                PTRACE(0, 0x10 + id);
-#ifndef PNR_DIAG_OFF_WAITS   // timing diagnostic only (wrong results): the MMA thread's instruction stream alone, nothing to wait for
                 mbar_wait_cluster(bar(id), (ph >> id) & 1u);
-#endif
                 ph ^= (1u << id);
-                PTRACE(0, 0x40 + id);
-                if (ASYNC) fence_proxy_async();             // rows that landed in this CTA by st.async
+                fence_proxy_async();                        // rows that landed in this CTA by st.async
                 tc_fence_after();                           // the other warps' tcgen05.ld / st of this TMEM precede the MMAs below
-                MPROF_ADD(id == B_IN_READY ? 2 : 4);
               }
-#ifndef PNR_DIAG_OFF_RING
-              {
-                MPROF_T0();
-                mbar_wait(full_bar, wpar);                  // completed by the TMA engine: no tcgen05 fence needed
-                MPROF_ADD(1);
-                if (trace_stages) PTRACE(0, 0x72);
-              }
-#endif
+              mbar_wait(full_bar, wpar);                    // completed by the TMA engine: no tcgen05 fence needed
               const uint64_t b_desc = bdesc_hi | (uint64_t)(cur.x & 0x3FFFu);
               const uint32_t d_col = (cur.x >> 14) & 0x1FFu;
               mma_kblock_desc_2sm(tmem_base + d_col, a_desc, b_desc, idesc, (cur.x >> 23) & 1u);
-#ifndef PNR_DIAG_OFF_EMPTY_COMMIT
-              mma_commit_2sm(empty_bar, 3);       // (kept under PNR_DIAG_MMAONLY: nobody waits on it)
-#endif
+              mma_commit_2sm(empty_bar, 3);
               if (cur.y & (1u << 19)) {
                 const uint32_t c1 = cur.y & 31u, c2 = (cur.y >> 5) & 31u, c3 = (cur.y >> 14) & 31u;
                 if (c1) mma_commit_2sm(bar(c1 - 1), 3);
                 if (c2) mma_commit_2sm(bar(c2 - 1), 3);
                 if (c3) mma_commit_2sm(bar(c3 - 1), 3);
-                if (PROF == 2 && c2 > B_X_FULL && c2 <= B_X_FULL + 4) PTRACE(0, c2 - B_X_FULL);
               }
-              if (trace_stages) PTRACE(0, 0x71);
               if (++slot == kStages) { slot = 0; wpar ^= 1; full_bar = bar(B_W_FULL); empty_bar = bar(B_W_EMPTY); a_desc = wdesc0; }
               else { full_bar += 8; empty_bar += 8; a_desc += kStageStep; }
               cur = nxt;
@@ -530,27 +412,16 @@ field_pair_kernel(const pnr_scene sc, const pnr_points q, const __grid_constant_
             int st = st_beg;
             if (after_mean) {                               // lin_in's second stage is the first write into x tile 1
               issue_stage(st++);
-              MPROF_T0();
-#ifndef PNR_DIAG_OFF_WAITS
               mbar_wait_cluster(bar(B_X_FREE + 1), (ph >> (B_X_FREE + 1)) & 1u);
-#endif
               ph ^= (1u << (B_X_FREE + 1));
               tc_fence_after();
-              MPROF_ADD(5);
             }
             for (; st < st_end; ++st) issue_stage(st);
           }
         }
-#undef MPROF_T0
-#undef MPROF_ADD
       }
       __syncwarp();
-      if (prof && lane == 0) prof[0] += clock64() - t_role0;
-#ifdef PNR_DIAG_OFF_EPI
-    } else if (false) {
-#else
-    } else if (ASYNC) {
-#endif
+    } else {
       // ===================== relay (non-leader CTA): remote rows of the even chunks have landed here -> tell the leader
       const int n_pub = G * 2 * sch.CL + 2 * (sch.n_blocks - sch.CL) + 1;     // publishes of each chunk per super group
       uint32_t par = 0;
@@ -559,109 +430,58 @@ field_pair_kernel(const pnr_scene sc, const pnr_points q, const __grid_constant_
 #pragma unroll
           for (int mt = 0; mt < kMT; ++mt) {
             mbar_wait_cluster(bar(B_LAND + mt), par);
-            PTRACE_L0(3, 0x40 + B_LAND + mt);
             fence_proxy_async();
             __syncwarp();
             if (lane == 0) mbar_arrive_cluster_relaxed(lbar(B_RDY + 2 * mt));
-            PTRACE_L0(3, 0x83);
           }
           par ^= 1;
         }
       }
     }
-#ifdef PNR_DIAG_OFF_EPI
-  } else if (false) {
-#else
   } else if (warp >= 4 && warp < 12) {
-#endif
     // ===================== epilogue warps ===================================================================
     // 8 warps = 4 TMEM lane quadrants (qd) x 2.  Unit = this CTA's 128 features of feature tile mt x all 128 columns of
     // the pair = K-chunk kc = 2*mt + crank, written to chunk buffer kc of BOTH CTAs (rows = that CTA's own columns).
     //  * regular epilogues: warp (qd, part) converts columns [part*NC/2, (part+1)*NC/2) of BOTH tiles, the peer's first
-    //    (remote st.shared::cluster stores are in flight while the local half is computed), one publish per unit;
+    //    (remote st.async stores are in flight while the local half is computed), one publish per unit;
     //  * view-mean epilogue: warp (qd, hs) needs all 64 columns of tile hs (the three views of a point) in one thread.
     const int qd = warp & 3;                       // TMEM lane quadrant (warp % 4)
     const int hs = (warp - 4) >> 2;                // second index: column part, or tile in the mean / output epilogues
     const int fl = qd * 32 + lane;                 // feature row inside this CTA's 128-row half
     const uint32_t tlane = tmem_base + ((uint32_t)(qd * 32) << 16);
     uint32_t ph = 0;
-    const bool prof_warp = warp == 4;
-    auto wait = [&](int id) {
-      PPROF_T0();
-      if (prof_warp) PTRACE_L0(1 + (int)crank, 0x10 + id);
-#if PNR_IDLE_WAIT
-      mbar_wait_idle(bar(id), (ph >> id) & 1u); ph ^= (1u << id); tc_fence_after();
-#else
-      mbar_wait_cluster(bar(id), (ph >> id) & 1u); ph ^= (1u << id); tc_fence_after();
-#endif
-      if (prof_warp) PTRACE_L0(1 + (int)crank, 0x40 + id);
-      if (prof_warp) PPROF_ADD(id < B_H_FULL ? 9 : 10);
-    };
-    const long long t_role0 = prof ? clock64() : 0;
+    auto wait = [&](int id) { mbar_wait_cluster(bar(id), (ph >> id) & 1u); ph ^= (1u << id); tc_fence_after(); };
     const uint32_t peer = crank ^ 1u;
     constexpr uint32_t kRemoteBytes = (kNCol / 2) * 32 * 2;        // remote half of one warp's unit: 32 columns x 32 features bf16
     // barrier (in the peer CTA) that counts this CTA's st.async rows of chunk kc = 2*mt + crank
     auto land_bar = [&](int kc) -> uint32_t { return crank == 0 ? mapa_u32(bar(B_LAND + (kc >> 1)), 1) : lbar(B_RDY + kc); };
     auto publish = [&](int kc) {                   // operand rows of chunk kc written -> tell the leader's MMA warp
-      const long long tp0 = (prof && prof_warp) ? clock64() : 0;
-      if (ASYNC) {
-        fence_proxy_async();                       // local rows only; the remote rows are counted where they land
-        tc_fence_before();
-        __syncwarp();
-        if (lane == 0) {
-#if defined(PNR_DIAG_NOEPI) || defined(PNR_DIAG_EPI_NOSTORE)   // timing diagnostic only (wrong results): no rows were stored, so no bytes are expected
-          if (crank == 0) mbar_arrive(bar(B_RDY + kc));
-          mbar_arrive_cluster_relaxed(land_bar(kc));
-#else
-          if (crank == 0) { mbar_arrive(bar(B_RDY + kc)); mbar_arrive_expect_tx_cluster(land_bar(kc), kRemoteBytes); }
-          else mbar_arrive_expect_tx_cluster(land_bar(kc), kRemoteBytes);      // = the leader's chunk barrier
-#endif
-        }
-      } else {
-        fence_proxy_async_cluster();               // waits until this warp's local AND remote rows are performed
-        tc_fence_before();
-        __syncwarp();
-        // the fence already made the rows visible where the tensor cores read them: no cluster-scope release needed
-        if (lane == 0) { if (crank == 0) mbar_arrive(bar(B_RDY + kc)); else mbar_arrive_cluster_relaxed(lbar(B_RDY + kc)); }
+      fence_proxy_async();                         // local rows only; the remote rows are counted where they land
+      tc_fence_before();
+      __syncwarp();
+      if (lane == 0) {
+        if (crank == 0) { mbar_arrive(bar(B_RDY + kc)); mbar_arrive_expect_tx_cluster(land_bar(kc), kRemoteBytes); }
+        else mbar_arrive_expect_tx_cluster(land_bar(kc), kRemoteBytes);        // = the leader's chunk barrier
       }
-      if (prof && prof_warp && lane == 0) prof[18] += clock64() - tp0;
-      if (prof_warp) PTRACE_L0(1 + (int)crank, 0x83);
     };
     // both halves of a unit: columns [hs*32, hs*32+32) of tile `peer` (remote rows) then of tile `crank` (local rows)
-    // c0_busy: (order 3) this unit rewrites chunk buffer 0 while the layer that produced it may still be reading the buffer
-    const bool order3 = sch.order == 3;
-    auto convert_unit = [&](uint32_t tcol, int kc, float bias, bool c0_busy) {
+    auto convert_unit = [&](uint32_t tcol, int kc, float bias) {
       const uint32_t loc = sbase + Smem::ring + kc * kChunkBytes;
       const uint32_t rem = mapa_u32(loc, peer);
-#ifdef PNR_DIAG_NOEPI   // timing diagnostic only (wrong results): the regular epilogues cost nothing but their barrier traffic
-      (void)loc; (void)rem; (void)tcol; (void)bias;
-      return;
-#endif
       uint32_t v[kNCol / 2], u[kNCol / 2];
-#ifdef PNR_DIAG_EPI_NOALU
-#pragma unroll
-      for (int c = 0; c < kNCol / 2; ++c) { v[c] = 0u; u[c] = 0u; }
-#else
       tmem_ld_nowait<kNCol / 2>(tlane + tcol + peer * kNCol + hs * (kNCol / 2), v);     // both halves in flight at once
       tmem_ld_nowait<kNCol / 2>(tlane + tcol + crank * kNCol + hs * (kNCol / 2), u);
       tmem_ld_wait();
-#endif
-      if (prof_warp) PTRACE_L0(1 + (int)crank, 0x80);
-      if (c0_busy) wait(B_C0_FREE);
-      store_transposed<kNCol / 2, true, true>(rem, v, bias, lane, qd * 32, hs * (kNCol / 2), ASYNC ? land_bar(kc) : 0u);
-      if (prof_warp) PTRACE_L0(1 + (int)crank, 0x81);
+      store_transposed<kNCol / 2, true, true>(rem, v, bias, lane, qd * 32, hs * (kNCol / 2), land_bar(kc));
       store_transposed<kNCol / 2, false, true>(loc, u, bias, lane, qd * 32, hs * (kNCol / 2));
-      if (prof_warp) PTRACE_L0(1 + (int)crank, 0x82);
     };
-    auto x_epilogue = [&](int e, bool after_fc) {  // relu(x + cumulative bias) -> bf16 K-chunks; after_fc: an fc_1 layer wrote this x
+    auto x_epilogue = [&](int e) {                 // relu(x + cumulative bias) -> bf16 K-chunks
       for (int mt = 0; mt < kMT; ++mt) {
         // the bias is fetched BEFORE the wait: a global load issued after it sits on the hand-off's critical path
         const float bias = __ldg(bias_x + e * kHidden + mt * 256 + crank * 128 + fl);
         wait(B_X_FULL + mt);
         const int kc = 2 * mt + (int)crank;
-        const long long ts0 = (prof && prof_warp) ? clock64() : 0;
-        convert_unit(mt * 128, kc, bias, order3 && kc == 0 && after_fc);
-        if (prof && prof_warp && lane == 0) prof[14] += clock64() - ts0;
+        convert_unit(mt * 128, kc, bias);
         publish(kc);
       }
     };
@@ -670,7 +490,7 @@ field_pair_kernel(const pnr_scene sc, const pnr_points q, const __grid_constant_
         const float bias = __ldg(bias_h + b * kHidden + mt * 256 + crank * 128 + fl);
         wait(B_H_FULL + mt);
         const int kc = 2 * mt + (int)crank;
-        convert_unit(kHCol + mt * 128, kc, bias, order3 && kc == 0);
+        convert_unit(kHCol + mt * 128, kc, bias);
         publish(kc);
       }
     };
@@ -681,12 +501,11 @@ field_pair_kernel(const pnr_scene sc, const pnr_points q, const __grid_constant_
         const bool live = tile < n_tiles;
         const int obj = tile / tiles_per_obj;
         const int p0 = (tile - obj * tiles_per_obj) * PP;
-        for (int e = 0; e < sch.CL; ++e) { x_epilogue(e, e > 0); h_epilogue(e); }
+        for (int e = 0; e < sch.CL; ++e) { x_epilogue(e); h_epilogue(e); }
         float bias_mean[kMT];
 #pragma unroll
         for (int mt = 0; mt < kMT; ++mt) bias_mean[mt] = __ldg(bias_x + sch.CL * kHidden + mt * 256 + (int)crank * 128 + fl);
         for (int mt = 0; mt < kMT; ++mt) wait(B_X_FULL + mt);
-        if (order3 && crank == 0 && sch.CL > 0) wait(B_C0_FREE);      // keep the phase in step (the last fc_1 signalled it too)
         // view pooling (combine_interleaved) + cumulative bias -> x-bar, column g*PP + p of slot hs.  max(x_v + b) = max(x_v) + b
         // exactly: rounding is monotonic
 #pragma unroll
@@ -737,18 +556,14 @@ field_pair_kernel(const pnr_scene sc, const pnr_points q, const __grid_constant_
           for (int c = 0; c < kNCol / 2; ++c)
             v[c] = (hs * (kNCol / 2) + c < NLIVE) ? __float_as_uint(__ldcg(src + (size_t)c * kHidden)) : 0u;
           tmem_st<kNCol / 2>(tlane + mt * 128 + t * kNCol + hs * (kNCol / 2), v);
-#ifndef PNR_DIAG_NOEPI
-          if (half == 0) store_transposed<kNCol / 2, true, false>(mapa_u32(loc, peer), v, 0.f, lane, qd * 32, hs * (kNCol / 2), ASYNC ? land_bar(kc) : 0u);
+          if (half == 0) store_transposed<kNCol / 2, true, false>(mapa_u32(loc, peer), v, 0.f, lane, qd * 32, hs * (kNCol / 2), land_bar(kc));
           else store_transposed<kNCol / 2, false, false>(loc, v, 0.f, lane, qd * 32, hs * (kNCol / 2));
-#else
-          (void)loc;
-#endif
         }
         publish(kc);
       }
       if (pooled) h_epilogue(sch.CL);
       for (int e = sch.CL + 1; e <= sch.n_blocks; ++e) {
-        x_epilogue(e, true);
+        x_epilogue(e);
         if (e < sch.n_blocks) h_epilogue(e);
       }
       // ---- output: lin_out rows are features 0..d_out-1 -> leader CTA, TMEM lanes 0..d_out-1 of h tile 0
@@ -781,16 +596,10 @@ field_pair_kernel(const pnr_scene sc, const pnr_points q, const __grid_constant_
       }
       tc_fence_before();
     }
-    if (prof && prof_warp && lane == 0) prof[8] += clock64() - t_role0;
-#ifdef PNR_DIAG_OFF_GATHER
-  } else if (false) {
-#else
   } else if (warp == 2 || warp == 3 || warp == 14 || warp == 15) {
-#endif
     // ===================== gather warps: this CTA's 64 columns -> its own z-feature / latent operand rows =======
     const int gw = warp < 4 ? warp - 2 : warp - 12;
     uint32_t par_free = 1;
-    const long long t_role0 = prof ? clock64() : 0;
     const int n_pass = z_passes(sch);
     const int fills = (n_pass > 1 || sch.proj) ? sch.n_linz * n_pass : 1;
     for (int it = 0;; ++it) {                        // tile pairs sg*G + g of super groups sg = pair_id, pair_id + n_pairs, ...
@@ -850,11 +659,7 @@ field_pair_kernel(const pnr_scene sc, const pnr_points q, const __grid_constant_
           for (int k = 0; k < 4; ++k) {
             const int off = __shfl_sync(0xffffffffu, tp.off[k], i);
             w[k] = __shfl_sync(0xffffffffu, tp.w[k], i);
-#ifdef PNR_DIAG_NOGATHER   // timing diagnostic only: no tap loads
-            if (false) {
-#else
             if (off >= 0 && act) {
-#endif
               const uint4* src = reinterpret_cast<const uint4*>(fl0 + vb + off);
               r[2 * k] = __ldg(src); r[2 * k + 1] = __ldg(src + 1);
             } else {
@@ -897,17 +702,7 @@ field_pair_kernel(const pnr_scene sc, const pnr_points q, const __grid_constant_
           float wa[4], wb[4];
           load_col(0, ra, wa);                       // the first two columns' loads go out BEFORE the operand buffers are free:
           load_col(1, rb, wb);                       // they only fill registers
-          {
-            PPROF_T0();
-            if (gw == 0 && crank == 0) PTRACE_L0(4, 0x10 + B_IN_FREE);
-#if PNR_IDLE_WAIT
-            mbar_wait_idle(bar(B_IN_FREE), par_free);
-#else
-            mbar_wait_cluster(bar(B_IN_FREE), par_free);
-#endif
-            if (gw == 0 && crank == 0) PTRACE_L0(4, 0x40 + B_IN_FREE);
-            if (gw == 0) PPROF_ADD(17);
-          }
+          mbar_wait_cluster(bar(B_IN_FREE), par_free);
           par_free ^= 1;
           if (fill == 0) {                           // the sin/cos work runs under the first loads' latency
 #pragma unroll 1
@@ -924,15 +719,12 @@ field_pair_kernel(const pnr_scene sc, const pnr_points q, const __grid_constant_
         fence_proxy_async();                 // the gather writes this CTA's own shared memory only
         __syncwarp();
         if (lane == 0) { if (crank == 0) mbar_arrive(bar(B_IN_READY)); else mbar_arrive_cluster_relaxed(lbar(B_IN_READY)); }
-        if (gw == 0 && crank == 0) PTRACE_L0(4, 0x83);
       }
     }
-    if (prof && gw == 0 && lane == 0) prof[16] += clock64() - t_role0;
   }
 
   tc_fence_before();
   __syncthreads();
-  if (PROF == 1 && g_prof_pair && threadIdx.x < 32) g_prof_pair[(size_t)blockIdx.x * 32 + threadIdx.x] = prof[threadIdx.x];
   cluster_sync_all();                    // no CTA exits (or frees TMEM) while the pair may still touch it
   if (warp == 1) tmem_dealloc_2sm(tmem_base, kTmemCols);
 }
@@ -940,21 +732,8 @@ field_pair_kernel(const pnr_scene sc, const pnr_points q, const __grid_constant_
 }  // namespace pair
 
 // ---- host side ---------------------------------------------------------------------------------------------
-// PNR_ASYNC=0 selects the synchronous epilogue exchange (st.shared::cluster + cluster-scope proxy fence); default 1.
-static bool pair_async() {
-  static int cached = -1;
-  if (cached < 0) { const char* e = getenv("PNR_ASYNC"); cached = (e && atoi(e) == 0) ? 0 : 1; }
-  return cached != 0;
-}
-// PNR_ORDER=0 / 1 select the K-chunk-outer / tile-0-first pair orders (experiments); default 2 (see fc_pair).  Read once: pack
-// and launch must agree.
-static int pair_order() {
-  static int cached = -1;
-  if (cached < 0) { const char* e = getenv("PNR_ORDER"); cached = e ? atoi(e) : 2; if (cached < 0 || cached > 3) cached = 2; }
-  return cached;
-}
 static pair::Sched pair_sched(const pnr_mlp_params* p, int proj) {
-  return pair::Sched{p->n_blocks, p->combine_layer, p->combine_layer, proj ? kHidden / 64 : p->d_latent / 64, pair_order(), proj};
+  return pair::Sched{p->n_blocks, p->combine_layer, p->combine_layer, proj ? kHidden / 64 : p->d_latent / 64, proj};
 }
 size_t pair_stream_bytes(const pnr_mlp_params* p, int proj) {
   pair::Sched s = pair_sched(p, proj);
@@ -1019,30 +798,12 @@ int field_forward_pair(const pnr_scene* sc, const pnr_points* q, const pnr_mlp_p
   cudaGetDevice(&dev);
   cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
   const int G = pair::kNCol / PP;                        // tile pairs per super group (see field_pair_kernel)
-  const bool async_x = pair_async();
   // max over one view is the view itself: NS == 1 runs the average instantiation whatever combine_type says
   const bool vmax = mp->combine_type == PNR_COMBINE_MAX && sc->NS > 1;
-  PNR_REQUIRE(!vmax || (async_x && !getenv("PNR_TRACE") && !getenv("PNR_PROF")), PNR_ERR_UNSUPPORTED,
-              "field_forward_pair: the PNR_ASYNC=0 / PNR_PROF / PNR_TRACE instruments are built for combine_type average only");
   const int n_groups = ((n_tiles + 1) / 2 + G - 1) / G;  // super groups
-  long long* prof_dev = nullptr;
-  long long* trace_dev = nullptr;
-  if (getenv("PNR_TRACE")) {          // event log of pair 0 (takes precedence over the counters)
-    cudaMalloc(&trace_dev, (size_t)11 * pair::kTraceLen * sizeof(long long));
-    cudaMemset(trace_dev, 0, (size_t)11 * pair::kTraceLen * sizeof(long long));
-    cudaMemcpyToSymbol(pair::g_trace_pair, &trace_dev, sizeof(trace_dev));
-    const int ts = getenv("PNR_TRACE_STAGES") ? 1 : 0;
-    cudaMemcpyToSymbol(pair::g_trace_stages, &ts, sizeof(ts));
-  } else if (getenv("PNR_PROF")) {
-    cudaMalloc(&prof_dev, (size_t)4096 * 32 * sizeof(long long));
-    cudaMemset(prof_dev, 0, (size_t)4096 * 32 * sizeof(long long));
-    cudaMemcpyToSymbol(pair::g_prof_pair, &prof_dev, sizeof(prof_dev));
-  }
 #define PNR_LAUNCH_PAIR(NSV)                                                                                     \
   case NSV: {                                                                                                    \
-    auto kern = vmax ? pair::field_pair_kernel<NSV, true, 0, (NSV > 1)>                                          \
-              : async_x ? (trace_dev ? pair::field_pair_kernel<NSV, true, 2> : prof_dev ? pair::field_pair_kernel<NSV, true, 1> : pair::field_pair_kernel<NSV, true, 0>) \
-                        : pair::field_pair_kernel<NSV, false, 0>;                                           \
+    auto kern = vmax ? pair::field_pair_kernel<NSV, (NSV > 1)> : pair::field_pair_kernel<NSV, false>;            \
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pair::Smem::total); \
     PNR_REQUIRE(e == cudaSuccess, PNR_ERR_CUDA, "cudaFuncSetAttribute: %s", cudaGetErrorString(e));             \
     cudaLaunchConfig_t cfg = {};                                                                                 \
@@ -1054,7 +815,6 @@ int field_forward_pair(const pnr_scene* sc, const pnr_points* q, const pnr_mlp_p
     cfg.gridDim = dim3(sms / 2 * 2);                                                                             \
     int max_pairs = sms / 2, mc = 0;                                                                             \
     if (cudaOccupancyMaxActiveClusters(&mc, kern, &cfg) == cudaSuccess && mc > 0 && mc < max_pairs) max_pairs = mc; \
-    if (const char* mp_env = getenv("PNR_MAX_PAIRS")) { const int v = atoi(mp_env); if (v > 0 && v < max_pairs) max_pairs = v; } /* experiments */ \
     const int n_pairs = n_groups < max_pairs ? n_groups : max_pairs;                                             \
     cfg.gridDim = dim3(n_pairs * 2);                                                                             \
     e = cudaLaunchKernelEx(&cfg, kern, *sc, *q, tmap, bx, bh, bo, out, xbar, sch, num_freqs, freq_factor, tiles_per_obj, \
@@ -1067,42 +827,6 @@ int field_forward_pair(const pnr_scene* sc, const pnr_points* q, const pnr_mlp_p
   }
 #undef PNR_LAUNCH_PAIR
   PNR_CHECK_LAUNCH("field_pair_kernel");
-  if (prof_dev) {   // debug only: synchronises and prints the per-role wait breakdown
-    cudaStreamSynchronize(st);
-    std::vector<long long> h((size_t)4096 * 32);
-    cudaMemcpy(h.data(), prof_dev, h.size() * sizeof(long long), cudaMemcpyDeviceToHost);
-    const char* names[32] = {"mma_total", "mma_wait_weights", "mma_wait_gather", 0, "mma_wait_chunk", "mma_wait_x_free", 0, 0,
-                             "epi_total", "epi_wait_x_full", "epi_wait_h_full", 0, 0, 0, "epi_convert_x(x10 units)", 0,
-                             "gather_total", "gather_wait_in_free", "epi_publish(x22)"};
-    int ctas = 0, leaders = 0; double sum[32] = {0};
-    for (int b = 0; b < 4096; ++b) {
-      if (h[(size_t)b * 32 + 8] == 0) continue;
-      ++ctas; if (h[(size_t)b * 32] != 0) ++leaders;
-      for (int k = 0; k < 32; ++k) sum[k] += (double)h[(size_t)b * 32 + k];
-    }
-    const double groups_per_pair = (double)n_groups / (leaders ? leaders : 1);
-    fprintf(stderr, "[pnr pair prof] tiles=%d pairs=%d super-groups/pair=%.1f  (cycles per super group of %d tile pairs)\n", n_tiles, leaders, groups_per_pair, G);
-    for (int k = 0; k < 32; ++k) if (names[k]) fprintf(stderr, "[pnr pair prof]   %-22s %10.0f\n", names[k], sum[k] / ((k < 8) ? (leaders ? leaders : 1) : (ctas ? ctas : 1)) / groups_per_pair);
-    long long* null_ptr = nullptr;
-    cudaMemcpyToSymbol(pair::g_prof_pair, &null_ptr, sizeof(null_ptr));
-    cudaFree(prof_dev);
-
-  }
-  if (trace_dev) {
-    cudaStreamSynchronize(st);
-    long long* null_ptr = nullptr;
-    std::vector<long long> tr((size_t)11 * pair::kTraceLen);
-    cudaMemcpy(tr.data(), trace_dev, tr.size() * sizeof(long long), cudaMemcpyDeviceToHost);
-    if (FILE* f = fopen(getenv("PNR_TRACE"), "a")) {
-      fprintf(f, "# launch tiles=%d\n", n_tiles);
-      for (int r = 0; r < 11; ++r)
-        for (int i = 0; i < pair::kTraceLen && tr[(size_t)r * pair::kTraceLen + i]; ++i)
-          fprintf(f, "%d %lld %lld\n", r, tr[(size_t)r * pair::kTraceLen + i] >> 8, tr[(size_t)r * pair::kTraceLen + i] & 0xFF);
-      fclose(f);
-    }
-    cudaMemcpyToSymbol(pair::g_trace_pair, &null_ptr, sizeof(null_ptr));
-    cudaFree(trace_dev);
-  }
   return PNR_OK;
 }
 

@@ -18,7 +18,6 @@
 #include "umma.cuh"
 #include "train_umma.cuh"
 #include <cuda.h>
-#include <stdlib.h>
 
 namespace pnr {
 namespace tg {
@@ -53,7 +52,8 @@ __host__ __device__ inline uint32_t idesc_2sm(int n, int a_mn, int b_mn) {
 }
 // MN-major SWIZZLE_128B tile made of 64-feature x 64-row boxes (8 KiB each) laid one after the other along MN:
 // LBO = byte distance between 64-element MN atoms = 8 192, SBO = byte distance between 8-row K groups = 1 024
-__device__ __forceinline__ uint64_t smem_desc_mn(uint32_t saddr, uint32_t lbo = 8192, uint32_t sbo = 1024) {
+__device__ __forceinline__ uint64_t smem_desc_mn(uint32_t saddr) {
+  constexpr uint32_t lbo = 8192, sbo = 1024;
   return (uint64_t)((saddr >> 4) & 0x3FFFu) | ((uint64_t)(lbo >> 4) << 16) | ((uint64_t)(sbo >> 4) << 32) | (1ull << 46) | (2ull << 61);
 }
 
@@ -105,9 +105,8 @@ rowgemm_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constant_
           const int kb = second ? s - g.nK0 : s;
           const int nK = second ? g.nK1 : g.nK0;
           mbar_wait_cluster(bar(G_EMPTY + slot), par);
-          if (crank == 0) mbar_arrive_expect_tx(bar(G_FULL + slot), (g.diag & 2) ? kStageG : 2 * kStageG);
+          if (crank == 0) mbar_arrive_expect_tx(bar(G_FULL + slot), 2 * kStageG);
           const uint32_t dst = sbase + SmemG::ring + slot * kStageG;
-          if (!(g.diag & 2))      // timing diagnostic 2: no activation-tile loads (wrong results)
           tma_load_2d_2sm(dst, second ? (const void*)&mapA1 : (const void*)&mapA0, kb * 64, row, bar(G_FULL + slot));
           tma_load_2d_2sm(dst + kHalf, second ? (const void*)&mapW1 : (const void*)&mapW0, 0, ((nh * nK + kb) * 2 + (int)crank) * 128,
                           bar(G_FULL + slot));
@@ -128,7 +127,6 @@ rowgemm_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constant_
         for (int s = 0; s < n_stage_unit; ++s) {
           mbar_wait(bar(G_FULL + slot), fpar);
           const uint32_t a = sbase + SmemG::ring + slot * kStageG;
-          if (!(g.diag & 4))      // timing diagnostic 4: no MMAs
           mma_kblock_desc_2sm(tmem_base + buf * 256, smem_desc(a), smem_desc(a + kHalf), idesc, s > 0);
           mma_commit_2sm(bar(G_EMPTY + slot), 3);
           if (++slot == kStagesG) { slot = 0; fpar ^= 1; }
@@ -209,7 +207,7 @@ rowgemm_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constant_
           if (lane == 0) { if (crank == 0) mbar_arrive(bar(G_ACC_FREE + buf)); else mbar_arrive_cluster_relaxed(lbar(G_ACC_FREE + buf)); }
         }
         __syncwarp();                                    // the staged tiles are complete
-        if (col0 >= g.n_valid || (g.diag & 1)) continue;   // timing diagnostic 1: the epilogue only drains TMEM
+        if (col0 >= g.n_valid) continue;
         float v[32];
 #pragma unroll
         for (int j = 0; j < 32; ++j) v[j] = __uint_as_float(vr[j]);
@@ -399,10 +397,11 @@ wgrad_kernel(const __grid_constant__ CUtensorMap mapY, const __grid_constant__ C
         for (long long s = s0; s < s1; ++s) {
           mbar_wait(bar(G_FULL + slot), fpar);
           const uint32_t a = sbase + SmemG::ring + slot * kStageG;
-          const uint64_t ad = smem_desc_mn(a, g.dbg_lbo, g.dbg_sbo), bd = smem_desc_mn(a + kHalf, g.dbg_lbo, g.dbg_sbo);
+          const uint64_t ad = smem_desc_mn(a), bd = smem_desc_mn(a + kHalf);
+          constexpr uint32_t kKStep = 2048 >> 4;             // 16 rows (contraction) = 2 048 B further into both tiles
 #pragma unroll
-          for (int ks = 0; ks < 4; ++ks)                     // 16 rows (contraction) = 2 048 B further into both tiles
-            mma_bf16_2sm(tmem_base + buf * 256, ad + (uint64_t)(ks * g.dbg_kstep), bd + (uint64_t)(ks * g.dbg_kstep), idesc, (s > s0 || ks > 0) ? 1u : 0u);
+          for (int ks = 0; ks < 4; ++ks)
+            mma_bf16_2sm(tmem_base + buf * 256, ad + (uint64_t)(ks * kKStep), bd + (uint64_t)(ks * kKStep), idesc, (s > s0 || ks > 0) ? 1u : 0u);
           mma_commit_2sm(bar(G_EMPTY + slot), 3);
           if (++slot == kStagesG) { slot = 0; fpar ^= 1; }
         }
@@ -579,7 +578,6 @@ int rowgemm(const RowGemmSrc& s0, const RowGemmSrc* s1, RowGemmArgs g, cudaStrea
   PNR_REQUIRE(g.bias || !g.bias2, PNR_ERR_ARG, "rowgemm: bias2 without bias");
   g.nK0 = s0.K / 64;
   g.nK1 = s1 ? s1->K / 64 : 0;
-  if (const char* e = getenv("PNR_RG_DIAG")) g.diag = atoi(e);
   CUtensorMap mA0, mW0, mA1, mW1;
   int rc;
   if ((rc = make_map(&mA0, s0.A, g.M, s0.K, s0.lda, 64, 128, true))) return rc;
@@ -615,10 +613,6 @@ int wgrad(const __nv_bfloat16* dY, long long ldy, const __nv_bfloat16* X, long l
   WgradArgs g = {};
   g.dW = dW; g.ldw = ldw; g.M = M; g.N = N; g.K = K;
   g.nNb = (N + 255) / 256; g.nKb = (K + 255) / 256;
-  g.dbg_lbo = 8192; g.dbg_sbo = 1024; g.dbg_kstep = 128;
-  if (const char* e = getenv("PNR_WGRAD_LBO")) g.dbg_lbo = (uint32_t)atoi(e);
-  if (const char* e = getenv("PNR_WGRAD_SBO")) g.dbg_sbo = (uint32_t)atoi(e);
-  if (const char* e = getenv("PNR_WGRAD_KSTEP")) g.dbg_kstep = (uint32_t)atoi(e);
   cudaError_t e = cudaFuncSetAttribute(wgrad_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SmemG::total);
   PNR_REQUIRE(e == cudaSuccess, PNR_ERR_CUDA, "cudaFuncSetAttribute: %s", cudaGetErrorString(e));
   int max_pairs = 74;

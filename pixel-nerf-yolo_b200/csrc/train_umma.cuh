@@ -23,7 +23,6 @@ struct RowGemmArgs {
   float* colsum_out;                 // [n_valid] or null: += column sums of v over the rows (bias gradients), fused into the epilogue
   float* colsum_out2;                // a second destination for the same sums (fc_1 bias and lin_z bias see the same gradient)
   int nN, n_pad, nK0, nK1;           // filled in by rowgemm()
-  int diag;                          // timing diagnostics (PNR_RG_DIAG bits: 1 no epilogue work, 2 no activation loads, 4 no MMAs)
 };
 struct RowGemmSrc {
   const __nv_bfloat16* A; long long lda;   // [M, K] row-major bf16, lda multiple of 8
@@ -34,7 +33,6 @@ struct WgradArgs {
   float* dW; int ldw;
   long long M; int N, K;
   int nNb, nKb, n_slabs;
-  uint32_t dbg_lbo, dbg_sbo, dbg_kstep;      // descriptor strides (experiments: PNR_WGRAD_LBO / SBO / KSTEP)
 };
 
 size_t packed_rowgemm_bytes(int n_out, int n_in);

@@ -91,44 +91,6 @@ static __device__ __noinline__ void mbar_wait_slow(uint32_t bar, uint32_t parity
 __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
   if (!mbar_try_wait(bar, parity)) mbar_wait_slow(bar, parity);
 }
-// Wait of a role whose wake-up is not on the issue thread's critical path (epilogue / gather / producer warps waiting for a
-// tcgen05.commit): CTA-scope probe (the data behind these barriers lives in TMEM or is consumed by the async proxy, no generic
-// read follows) that leaves the scheduler's issue slots to the warps that have work.  PNR_IDLE_WAIT selects the flavour:
-// 0 = plain spin on try_wait, 1 = try_wait with a suspend-time hint, 2 = try_wait + __nanosleep back-off.
-#ifndef PNR_IDLE_WAIT
-#define PNR_IDLE_WAIT 0
-#endif
-__device__ __forceinline__ bool mbar_try_wait_hint(uint32_t bar, uint32_t parity, uint32_t ns) {
-  uint32_t ok;
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2, %3;\n\t"
-      "selp.b32 %0, 1, 0, p;\n\t}"
-      : "=r"(ok)
-      : "r"(bar), "r"(parity), "r"(ns)
-      : "memory");
-  return ok != 0;
-}
-static __device__ __noinline__ void mbar_wait_idle_slow(uint32_t bar, uint32_t parity) {
-  const long long t0 = clock64();
-  for (;;) {
-#if PNR_IDLE_WAIT == 1
-    if (mbar_try_wait_hint(bar, parity, 20000u)) return;
-#elif PNR_IDLE_WAIT == 2
-    __nanosleep(100);
-    if (mbar_try_wait(bar, parity)) return;
-#else
-    if (mbar_try_wait(bar, parity)) return;
-#endif
-    if (clock64() - t0 > 4000000000LL) {
-      printf("pnr: mbarrier wait timed out (block %d thread %d bar 0x%x parity %u)\n", (int)blockIdx.x, (int)threadIdx.x, bar, parity);
-      __trap();
-    }
-  }
-}
-__device__ __forceinline__ void mbar_wait_idle(uint32_t bar, uint32_t parity) {
-  if (!mbar_try_wait(bar, parity)) mbar_wait_idle_slow(bar, parity);
-}
 
 // ---- proxies / fences -------------------------------------------------------------------------------
 __device__ __forceinline__ void fence_proxy_async() {   // generic-proxy smem writes -> visible to UMMA/TMA

@@ -203,39 +203,3 @@ def test_render_plan_follows_state_changes():
     net.mlp_fine.lin_out.bias.data.copy_(saved)                            # behind autograd's back: needs invalidate()
     net.mlp_fine.invalidate()
     assert torch.equal(b, go())
-
-
-_ORDER_SCRIPT = r"""
-import sys, torch
-sys.path.insert(0, sys.argv[1]); sys.path.insert(0, sys.argv[2])
-import helpers as H
-import pixel_nerf_yolo_b200.synth as synth
-from pixel_nerf_yolo_b200.conf import ConfigTree
-from pixel_nerf_yolo_b200.render import NeRFRenderer
-scene = H.make_scene_dict(feat=64)
-net = H.build_net(scene, precision="bf16")
-rays = synth.target_rays(128)[:, ::16].contiguous()
-noise = H.make_noise(rays.shape[1], seed=4)
-r = NeRFRenderer.from_conf(ConfigTree.from_dict(dict(H.RENDER_CONF))).eval().cuda()
-r.noise_override = {k: v.cuda() for k, v in noise.items()}
-with torch.no_grad():
-    res = r(net, rays.cuda())
-torch.save({"rgb": res.fine.rgb.cpu(), "depth": res.fine.depth.cpu()}, sys.argv[3])
-"""
-
-
-@pytest.mark.parametrize("order", [0, 1, 3])
-def test_experimental_pair_orders_render_the_same_image(order, tmp_path):
-    """The (chunk, tile) pair orders kept as experiments (PNR_ORDER, read once per process: csrc/mlp_umma_pair.cu fc_pair; order 3
-    adds a chunk-buffer hand-back barrier) render the same image as the default order up to the fp32 accumulation order."""
-    import subprocess
-    import sys
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    outs = {}
-    for o in (2, order):
-        path = str(tmp_path / f"order{o}.pt")
-        env = dict(os.environ, PNR_ORDER=str(o))
-        subprocess.run([sys.executable, "-c", _ORDER_SCRIPT, root, os.path.join(root, "tests"), path], check=True, env=env, timeout=600)
-        outs[o] = torch.load(path)
-    assert (outs[order]["rgb"] - outs[2]["rgb"]).abs().max().item() < 2e-3
-    assert (outs[order]["depth"] - outs[2]["depth"]).abs().max().item() < 2e-3
