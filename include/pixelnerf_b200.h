@@ -61,8 +61,9 @@ typedef struct pnr_scene {
 #define PNR_SCENE_MASK_NONNEG_Z 1
 /* pnr_field_forward returns the raw lin_out values instead of [sigmoid(rgb), relu(sigma)] (models.py:309-310). */
 #define PNR_SCENE_RAW_OUTPUT 2
-/* `feat` holds the lin_z PRE-PROJECTIONS of the encoder output (pnr_project_features): n_linz x d_hidden channels, slice b =
- * latent . lin_z[b].weight^T.  Bilinear interpolation and lin_z are both linear, so lin_z[b](gather(latent)) ==
+/* `feat` holds the lin_z PRE-PROJECTIONS of the encoder output (pnr_project_features): n_linz x d_hidden channels (the
+ * unpadded width, whatever width the packed network is padded to), slice b = latent . lin_z[b].weight^T.  pnr_field_forward
+ * checks C == n_linz * d_hidden.  Bilinear interpolation and lin_z are both linear, so lin_z[b](gather(latent)) ==
  * gather(slice b) (+ bias); the kernel then accumulates the gathered slice with an identity weight instead of streaming a
  * d_latent-wide lin_z.  For wide latents (1 792-channel YOLO backbone maps) this removes 3/4 of the gather traffic and 45 % of
  * the weight stages.  Needs `packed` from pnr_mlp_pack_projected.  bf16 tcgen05 path only. */
@@ -73,7 +74,7 @@ typedef struct pnr_scene {
 #define PNR_SCENE_TRAIN_TF32 8
 /* Training path only: the tcgen05 path -- bf16 operands (activations kept on a bf16 tape, 1 KiB per row and layer), fp32
  * accumulation in TMEM, cta_group::2 GEMMs for the forward layers, the input gradients and the weight gradients
- * (csrc/train_umma.cu).  Gradients within ~2e-2 of autograd (bf16 operand rounding).  d_hidden = 512, C a multiple of 64. */
+ * (csrc/train_umma.cu).  Gradients within ~2e-2 of autograd (bf16 operand rounding).  C a multiple of 64. */
 #define PNR_SCENE_TRAIN_BF16 16
 
 /* Where the query points of a field evaluation come from. */
@@ -203,6 +204,8 @@ typedef struct pnr_mlp_params {
   const float* linz_w[8]; const float* linz_b[8];    /* lin_z.i  (H, d_latent),(H)     */
   /* combine_layer = min(combine_layer, n_blocks): the views are pooled before block combine_layer; combine_layer == n_blocks
    * never pools (the single-view network of conf/default.conf), which is only defined for NS == 1 */
+  /* d_hidden: a multiple of 64 from 64 to 512 on every path; the tcgen05 inference path packs the network zero-padded to
+   * 256 (d_hidden <= 256) or 512 features.  Other widths: PNR_ERR_UNSUPPORTED at the first pack or field call. */
   int32_t d_in, d_latent, d_hidden, d_out, n_blocks, combine_layer;
   int32_t combine_type;                              /* PNR_COMBINE_*; the packed weight stream does not depend on it */
 } pnr_mlp_params;

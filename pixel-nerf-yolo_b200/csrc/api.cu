@@ -60,7 +60,8 @@ extern "C" int pnr_field_forward(const pnr_scene* scene, const pnr_points* pts, 
   cudaStream_t st = (cudaStream_t)stream;
   const int raw = (scene->flags & PNR_SCENE_RAW_OUTPUT) ? 1 : 0;
   if (precision == PNR_PREC_FP32) {
-    PNR_REQUIRE(params->d_hidden == kHidden, PNR_ERR_UNSUPPORTED, "pnr_field_forward: d_hidden=%d", params->d_hidden);
+    PNR_REQUIRE(hidden_width_supported(params->d_hidden), PNR_ERR_UNSUPPORTED,
+                "pnr_field_forward: d_hidden=%d (supported: " PNR_HIDDEN_WIDTHS ")", params->d_hidden);
     return field_forward_fp32(scene, pts, params, out, workspace, workspace_bytes, num_freqs, freq_factor, raw, st);
   }
   if (precision == PNR_PREC_BF16)

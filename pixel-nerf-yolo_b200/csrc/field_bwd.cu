@@ -703,7 +703,9 @@ static int check_train(const pnr_scene* sc, const pnr_points* q, const pnr_mlp_p
   PNR_REQUIRE(!((sc->flags & PNR_SCENE_TRAIN_TF32) && (sc->flags & PNR_SCENE_TRAIN_BF16)), PNR_ERR_ARG, "%s: choose one of PNR_SCENE_TRAIN_TF32 / PNR_SCENE_TRAIN_BF16", who);
   g_use_tf32 = (sc->flags & PNR_SCENE_TRAIN_TF32) ? 1 : 0;
   if (sc->flags & PNR_SCENE_TRAIN_BF16) {
-    PNR_REQUIRE(mp->d_hidden == kHidden && sc->C % 64 == 0, PNR_ERR_UNSUPPORTED, "%s: the tcgen05 training path needs d_hidden = %d and C a multiple of 64 (got %d, %d)", who, kHidden, mp->d_hidden, sc->C);
+    PNR_REQUIRE(hidden_width_supported(mp->d_hidden) && sc->C % 64 == 0, PNR_ERR_UNSUPPORTED,
+                "%s: the tcgen05 training path needs d_hidden in " PNR_HIDDEN_WIDTHS " and C a multiple of 64 (got %d, %d)", who,
+                mp->d_hidden, sc->C);
     PNR_REQUIRE(mp->d_in <= 64, PNR_ERR_UNSUPPORTED, "%s: d_in=%d > 64", who, mp->d_in);
   }
   PNR_REQUIRE(sc->C % 4 == 0, PNR_ERR_UNSUPPORTED, "%s: C=%d must be a multiple of 4", who, sc->C);

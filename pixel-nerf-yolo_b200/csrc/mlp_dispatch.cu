@@ -30,6 +30,8 @@ int field_forward_pair(const pnr_scene* sc, const pnr_points* q, const pnr_mlp_p
                        int num_freqs, float freq_factor, int raw, int proj, cudaStream_t st);
 
 // blob = 1 KiB header | cumulative x biases (n_blocks + 1) x 512 | fc_0 biases n_blocks x 512 | lin_out bias (128) | pair stream
+// The bias tables keep a 512-feature stride whatever d_hidden is; entries at and past d_hidden are zero (the padding to Hp).
+// header: magic, d_in, d_latent, d_hidden, d_out, n_blocks, combine_layer, stages, Hp
 struct PackOffsets { size_t bias_x, bias_h, bias_out, pair_stream, total; };
 static PackOffsets pack_offsets(const Sched& s, const pnr_mlp_params* p, int proj = 0) {
   PackOffsets o;
@@ -44,24 +46,27 @@ static PackOffsets pack_offsets(const Sched& s, const pnr_mlp_params* p, int pro
 __global__ void pack_bias_kernel(pnr_mlp_params mp, Sched sc, int n_stages, float* __restrict__ bias_x, float* __restrict__ bias_h,
                                  float* __restrict__ bias_out, uint32_t* __restrict__ header) {
   const int f = threadIdx.x;   // 512 threads
-  float cum = mp.lin_in_b[f] + (sc.n_linz > 0 ? mp.linz_b[0][f] : 0.f);
+  const bool live = f < mp.d_hidden;               // padded features: every bias 0
+  float cum = live ? mp.lin_in_b[f] + (sc.n_linz > 0 ? mp.linz_b[0][f] : 0.f) : 0.f;
   bias_x[f] = cum;
   for (int e = 1; e <= sc.n_blocks; ++e) {
     if (e - 1 == sc.CL) cum = 0.f;                 // the view-mean epilogue materialises the bias into TMEM
-    cum += mp.fc1_b[e - 1][f] + (e < sc.n_linz ? mp.linz_b[e][f] : 0.f);
+    if (live) cum += mp.fc1_b[e - 1][f] + (e < sc.n_linz ? mp.linz_b[e][f] : 0.f);
     bias_x[e * kHidden + f] = cum;
   }
-  for (int b = 0; b < sc.n_blocks; ++b) bias_h[b * kHidden + f] = mp.fc0_b[b][f];
+  for (int b = 0; b < sc.n_blocks; ++b) bias_h[b * kHidden + f] = live ? mp.fc0_b[b][f] : 0.f;
   if (f < 128) bias_out[f] = f < mp.d_out ? mp.lin_out_b[f] : 0.f;
   if (f == 0) {
     header[0] = kPackMagic; header[1] = mp.d_in; header[2] = mp.d_latent; header[3] = mp.d_hidden;
     header[4] = mp.d_out; header[5] = mp.n_blocks; header[6] = mp.combine_layer; header[7] = n_stages;
+    header[8] = mp.d_hidden <= 256 ? 256 : 512;
   }
 }
 
 static int make_sched(const pnr_mlp_params* p, Sched* s, const char* who) {
   PNR_REQUIRE(p, PNR_ERR_ARG, "%s: null params", who);
-  PNR_REQUIRE(p->d_hidden == kHidden, PNR_ERR_UNSUPPORTED, "%s: d_hidden=%d (tcgen05 path is built for %d)", who, p->d_hidden, kHidden);
+  PNR_REQUIRE(hidden_width_supported(p->d_hidden), PNR_ERR_UNSUPPORTED, "%s: d_hidden=%d (supported: " PNR_HIDDEN_WIDTHS ")", who,
+              p->d_hidden);
   PNR_REQUIRE(p->d_in > 0 && p->d_in <= 64, PNR_ERR_UNSUPPORTED, "%s: d_in=%d must be in (0,64]", who, p->d_in);
   PNR_REQUIRE(p->d_latent > 0 && p->d_latent % 64 == 0, PNR_ERR_UNSUPPORTED, "%s: d_latent=%d must be a positive multiple of 64", who, p->d_latent);
   PNR_REQUIRE(p->n_blocks >= 1 && p->n_blocks <= 8, PNR_ERR_UNSUPPORTED, "%s: n_blocks=%d", who, p->n_blocks);
@@ -87,9 +92,10 @@ int field_forward_umma(const pnr_scene* sc, const pnr_points* q, const pnr_mlp_p
   PNR_REQUIRE(!sc->feat_fp32, PNR_ERR_ARG, "field_forward_umma: needs bf16 channels-last feature maps");
   const int proj = (sc->flags & PNR_SCENE_PROJECTED) ? 1 : 0;
   if (proj) {
-    PNR_REQUIRE(sc->C == sch.n_linz * kHidden, PNR_ERR_ARG, "field_forward_umma: projected maps must have n_linz x %d = %d channels (got %d)",
-                kHidden, sch.n_linz * kHidden, sc->C);
-    sch.KBz = kHidden / 64;              // blob from pnr_mlp_pack_projected: identity lin_z over 512 channels
+    PNR_REQUIRE(sc->C == sch.n_linz * mp->d_hidden, PNR_ERR_ARG,
+                "field_forward_umma: projected maps must have n_linz x d_hidden = %d x %d = %d channels (got %d)", sch.n_linz,
+                mp->d_hidden, sch.n_linz * mp->d_hidden, sc->C);
+    sch.KBz = mp->d_hidden / 64;         // blob from pnr_mlp_pack_projected: identity lin_z over d_hidden channels
   } else {
     PNR_REQUIRE(sc->C == mp->d_latent, PNR_ERR_ARG, "field_forward_umma: feature maps have %d channels, the MLP expects %d", sc->C, mp->d_latent);
   }
@@ -111,7 +117,7 @@ using namespace pnr;
 static size_t mlp_pack_bytes(const pnr_mlp_params* p, int proj) {
   Sched s;
   if (make_sched(p, &s, "pnr_mlp_pack_bytes")) return 0;
-  if (proj) s.KBz = kHidden / 64;
+  if (proj) s.KBz = p->d_hidden / 64;
   return pack_offsets(s, p, proj).total;
 }
 extern "C" size_t pnr_mlp_pack_bytes(const pnr_mlp_params* p) { return mlp_pack_bytes(p, 0); }
@@ -122,7 +128,7 @@ static int mlp_pack(const pnr_mlp_params* p, void* packed, int proj, void* strea
   Sched s;
   int rc = make_sched(p, &s, "pnr_mlp_pack");
   if (rc) return rc;
-  if (proj) s.KBz = kHidden / 64;
+  if (proj) s.KBz = p->d_hidden / 64;
   PNR_REQUIRE(packed && ((uintptr_t)packed & 1023) == 0, PNR_ERR_ARG, "pnr_mlp_pack: packed must be non-null and 1024-byte aligned");
   PNR_REQUIRE(p->lin_in_w && p->lin_in_b && p->lin_out_w && p->lin_out_b, PNR_ERR_ARG, "pnr_mlp_pack: null lin_in/lin_out");
   for (int b = 0; b < p->n_blocks; ++b)

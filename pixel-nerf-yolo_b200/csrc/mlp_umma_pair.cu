@@ -7,7 +7,10 @@
 //     the single-CTA N=64 MMA, and N=128 runs the tensor pipe at its full rate (scripts/umma_bench.py);
 //   * each CTA streams only ITS half (128 rows) of every 256-row weight slab (tensor-map TMA, cta_group::2, completion
 //     on the leader's mbarrier);
-//   * TMEM per CTA: x^T = 2 feature tiles x 128 columns (cols [0,256)), h^T likewise (cols [256,512)).
+//   * TMEM per CTA: x^T = MT feature tiles x 128 columns (cols [0,256)), h^T likewise (cols [256,512)).
+// Hidden widths: the network is zero-padded to Hp = 256 * MT features (pnr_mlp_pack): MT = 2 (Hp = 512) for d_hidden in
+// (256, 512], MT = 1 (Hp = 256) for d_hidden <= 256.  Padded weight rows / columns and bias entries are zero, so the padded
+// features stay exactly 0 through every layer and both pooling modes.
 // The price: D rows are FEATURES (CTA c holds features 256*mt + 128*c + lane of all 128 columns) while the B operand
 // needs COLUMNS (CTA c holds the rows of its own 64 columns for all K).  So every epilogue unit sends half of its
 // bf16 output to the peer CTA's shared memory: values are transposed 8x8 across lanes (shuffles) into 16-byte chunks
@@ -35,8 +38,8 @@ using namespace umma;
 namespace pair {
 
 constexpr int kNCol = 64;                    // columns per CTA tile
-constexpr int kMT = 2;                       // 256-feature tiles per 512-wide layer
-constexpr int kKBlocksH = kHidden / kBlockK; // 8
+constexpr int kMaxMT = kHidden / 256;        // 256-feature tiles of the widest (512) hidden layer
+constexpr int kKBlocksLat = 512 / kBlockK;   // 8 k-blocks: one pass over 512 latent channels
 constexpr int kStages = 5;                   // weight ring depth (16 KiB each): the most that fits the shared-memory budget
 constexpr int kThreads = 512;
 constexpr int kProducers = 3;                // warps 0,12,13
@@ -49,86 +52,107 @@ constexpr int kHCol = 256;
 constexpr int kMaxStages = 1024;
 
 struct Sched { int n_blocks, CL, n_linz, KBz, proj; };
-// proj: the feature maps hold the lin_z pre-projections (512 channels per lin_z layer, PNR_SCENE_PROJECTED): every lin_z[b]
-// is an IDENTITY-weight accumulate of its own freshly gathered 512-channel slice (KBz = 8)
+// proj: the feature maps hold the lin_z pre-projections (d_hidden channels per lin_z layer, PNR_SCENE_PROJECTED): every
+// lin_z[b] is an IDENTITY-weight accumulate of its own freshly gathered d_hidden-channel slice (KBz = d_hidden / 64)
+// MT = 256-feature tiles of the padded hidden width Hp = 256 * MT.  Stages of one layer: lin_in MT, lin_z MT * KBz,
+// fc_0 / fc_1 (2 MT K-chunks x MT tiles x 2 k-blocks) 4 MT^2, lin_out 4 MT.
 enum { MAT_LIN_IN = 0, MAT_LINZ = 1, MAT_FC0 = 2, MAT_FC1 = 3, MAT_LIN_OUT = 4 };
 struct Seg { int kind, blk, t, len; };
 struct StageSrc { int mat, blk, row0, k0; };   // row0 = first row of the 256-row slab
 
+template <int MT> constexpr int kSquareStages = 4 * MT * MT;   // stages of one fc_0 / fc_1 layer
 __host__ __device__ inline int z_passes(const Sched& s) { return (s.KBz + 7) / 8; }
+template <int MT>
 __host__ __device__ inline int sched_total(const Sched& s) {
-  return kMT + s.n_linz * kMT * s.KBz + s.n_blocks * 32 + kKBlocksH;
+  return MT + s.n_linz * MT * s.KBz + s.n_blocks * 2 * kSquareStages<MT> + 4 * MT;
 }
 // stages [0, sched_pre) are the pre-combine part (run once per tile), the rest the post-combine part
-__host__ __device__ inline int sched_pre(const Sched& s) { return kMT + s.n_linz * kMT * s.KBz + s.CL * 32; }
+template <int MT>
+__host__ __device__ inline int sched_pre(const Sched& s) { return MT + s.n_linz * MT * s.KBz + s.CL * 2 * kSquareStages<MT>; }
 // per-tile stage order = MMA issue order:
-//   lin_in (2) | lin_z[0] | per block: fc_0 (8 (chunk, tile) pairs x kk(2), see fc_pair) | lin_z[b+1] | fc_1 (same) | lin_out (8)
-// Order of the (K-chunk kc, feature tile mt) pairs inside a 512x512 layer: (c1,t0)(c0,t0)(c1,t1)(c0,t1)(c3,t0)(c2,t0)(c3,t1)(c2,t1).
+//   lin_in (MT) | lin_z[0] | per block: fc_0 (2 MT^2 (chunk, tile) pairs x kk(2), see fc_pair) | lin_z[b+1] | fc_1 (same) |
+//   lin_out (4 MT)
+// Order of the (K-chunk kc, feature tile mt) pairs inside a 512x512 layer: (c1,t0)(c0,t0)(c1,t1)(c0,t1)(c3,t0)(c2,t0)(c3,t1)(c2,t1);
+// inside a 256x256 layer (MT = 1): (c1,t0)(c0,t0).
 // Chunks 0,1 come from the previous layer's tile 0 and arrive first, so both output tiles consume them first; then tile 0 is
 // finished (its completion is signalled on its own barrier, so its epilogue overlaps the last two pairs), then tile 1.
 // Each pair of chunks starts with its ODD chunk: odd chunks are produced by the non-leader CTA and their remote rows land in
 // the leader, on the very barrier the MMA warp waits on, while even chunks need the relay hop from the non-leader -- that hop
 // then overlaps the MMAs of the odd chunk.
 // first / last: this is the first / last (k-block of the) pair that touches output tile mt.
+template <int MT>
 __host__ __device__ inline void fc_pair(int t, int& kc, int& mt, int& kk, bool& first, bool& last) {
-  const int pr = t >> 1;                       // 0..7
+  const int pr = t >> 1;                       // 0..2 MT^2 - 1
   kk = t & 1;
-  kc = ((pr < 4) ? (pr & 1) : (2 + (pr & 1))) ^ 1;
-  mt = (pr >> 1) & 1;
-  first = (pr == 0 || pr == 2) && kk == 0;
-  last = (pr == 5 || pr == 7) && kk == 1;
+  if constexpr (MT == 1) {
+    kc = pr ^ 1;
+    mt = 0;
+    first = pr == 0 && kk == 0;
+    last = pr == 1 && kk == 1;
+  } else {
+    kc = ((pr < 4) ? (pr & 1) : (2 + (pr & 1))) ^ 1;
+    mt = (pr >> 1) & 1;
+    first = (pr == 0 || pr == 2) && kk == 0;
+    last = (pr == 5 || pr == 7) && kk == 1;
+  }
 }
-// chunk order of lin_out (one output tile): 1,0,3,2, odd chunk first as in fc_pair
+// chunk order of lin_out (one output tile): 1,0,3,2 (MT = 2) or 1,0 (MT = 1), odd chunk first as in fc_pair
 __host__ __device__ inline int out_chunk(int t) { return (t >> 1) ^ 1; }
+template <int MT>
 __host__ __device__ inline Seg walk_stage(const Sched& sc, int s) {
+  constexpr int sq = kSquareStages<MT>;
   Seg g;
-  const int s1 = kMT * sc.KBz;
-  if (s < kMT) { g.kind = MAT_LIN_IN; g.blk = 0; g.t = s; g.len = kMT; return g; }
-  s -= kMT;
+  const int s1 = MT * sc.KBz;
+  if (s < MT) { g.kind = MAT_LIN_IN; g.blk = 0; g.t = s; g.len = MT; return g; }
+  s -= MT;
   if (s < s1) { g.kind = MAT_LINZ; g.blk = 0; g.t = s; g.len = s1; return g; }
   s -= s1;
   for (int b = 0; b < sc.n_blocks; ++b) {
     const bool has_z = b + 1 < sc.n_linz;
-    if (s < 16) { g.kind = MAT_FC0; g.blk = b; g.t = s; g.len = 16; return g; }
-    s -= 16;
+    if (s < sq) { g.kind = MAT_FC0; g.blk = b; g.t = s; g.len = sq; return g; }
+    s -= sq;
     if (has_z) {
       if (s < s1) { g.kind = MAT_LINZ; g.blk = b + 1; g.t = s; g.len = s1; return g; }
       s -= s1;
     }
-    if (s < 16) { g.kind = MAT_FC1; g.blk = b; g.t = s; g.len = 16; return g; }
-    s -= 16;
+    if (s < sq) { g.kind = MAT_FC1; g.blk = b; g.t = s; g.len = sq; return g; }
+    s -= sq;
   }
-  g.kind = MAT_LIN_OUT; g.blk = 0; g.t = s; g.len = kKBlocksH;
+  g.kind = MAT_LIN_OUT; g.blk = 0; g.t = s; g.len = 4 * MT;
   return g;
 }
 struct ZPos { int pass, mt, kbi, kp; };
+template <int MT>
 __host__ __device__ inline ZPos z_position(int KBz, int t) {
   ZPos z;
-  z.pass = t / (kMT * 8);
-  const int tt = t - z.pass * kMT * 8;
+  z.pass = t / (MT * 8);
+  const int tt = t - z.pass * MT * 8;
   z.kp = KBz - z.pass * 8 < 8 ? KBz - z.pass * 8 : 8;
   z.mt = tt / z.kp;
   z.kbi = tt - z.mt * z.kp;
   return z;
 }
+template <int MT>
 __host__ __device__ inline StageSrc decode_stage(const Sched& sc, int s) {
-  const Seg g = walk_stage(sc, s);
+  const Seg g = walk_stage<MT>(sc, s);
   StageSrc r;
   r.mat = g.kind; r.blk = g.blk;
   switch (g.kind) {
     case MAT_LIN_IN: r.row0 = g.t * 256; r.k0 = 0; break;
-    case MAT_LINZ: { const ZPos z = z_position(sc.KBz, g.t); r.row0 = z.mt * 256; r.k0 = (z.pass * 8 + z.kbi) * 64; } break;
+    case MAT_LINZ: { const ZPos z = z_position<MT>(sc.KBz, g.t); r.row0 = z.mt * 256; r.k0 = (z.pass * 8 + z.kbi) * 64; } break;
     case MAT_FC0:
-    case MAT_FC1: { int kc, mt, kk; bool f, l; fc_pair(g.t, kc, mt, kk, f, l); r.row0 = mt * 256; r.k0 = kc * 128 + kk * 64; } break;
+    case MAT_FC1: { int kc, mt, kk; bool f, l; fc_pair<MT>(g.t, kc, mt, kk, f, l); r.row0 = mt * 256; r.k0 = kc * 128 + kk * 64; } break;
     default: r.row0 = 0; r.k0 = out_chunk(g.t) * 128 + (g.t & 1) * 64; break;
   }
   return r;
 }
 
-// Packed pair stream: stage s = [CTA0 half: 128 rows x 64 k][CTA1 half], both pre-swizzled 16 KiB k-blocks.
+// Packed pair stream: stage s = [CTA0 half: 128 rows x 64 k][CTA1 half], both pre-swizzled 16 KiB k-blocks.  Rows and k
+// past the layer's true size (the padding to Hp, d_in < 64, d_out < 128) are zero.
+template <int MT>
 __global__ void pack_stages_kernel(pnr_mlp_params mp, Sched sc, uint8_t* __restrict__ stages) {
   const int s = blockIdx.x >> 1, half = blockIdx.x & 1;
-  const StageSrc src = decode_stage(sc, s);
+  const StageSrc src = decode_stage<MT>(sc, s);
   const float* W; int rows, cols;
   switch (src.mat) {
     case MAT_LIN_IN: W = mp.lin_in_w; rows = mp.d_hidden; cols = mp.d_in; break;
@@ -151,25 +175,27 @@ struct Smem {
   static constexpr uint32_t w = 0;
   static constexpr uint32_t ring = w + kStages * kStageBytes;             // 4 K-chunk buffers (16 KiB each): chunk kc -> buffer kc
   static constexpr uint32_t lat = ring + 4 * kChunkBytes;
-  static constexpr uint32_t zf = lat + kKBlocksH * kOperandKB;
+  static constexpr uint32_t zf = lat + kKBlocksLat * kOperandKB;
   static constexpr uint32_t bars = zf + kOperandKB;
   static constexpr uint32_t prog = bars + 512;
   static constexpr uint32_t total = prog + 8 * kMaxStages;
 };
 enum {
   B_W_FULL = 0, B_W_EMPTY = B_W_FULL + kStages, B_IN_READY = B_W_EMPTY + kStages, B_IN_FREE,
-  B_X_FULL, B_H_FULL = B_X_FULL + kMT,          // one per feature tile
-  B_RDY = B_H_FULL + kMT, B_X_FREE = B_RDY + 4,  // one per feature tile: the view-mean epilogue has read x tile mt out of TMEM
-  B_LAND = B_X_FREE + kMT,                                       // non-leader CTA only: remote rows of chunk 2*i have landed (st.async bytes)
-  B_OUT_FREE = B_LAND + kMT,                    // leader: the output epilogue has read lin_out's result out of the h region
+  // laid out for MT = 2; MT = 1 uses the first of each group (feature tile 0, K-chunks 0 and 1)
+  B_X_FULL, B_H_FULL = B_X_FULL + kMaxMT,          // one per feature tile
+  B_RDY = B_H_FULL + kMaxMT, B_X_FREE = B_RDY + 2 * kMaxMT,  // one per feature tile: the view-mean epilogue has read x tile mt out of TMEM
+  B_LAND = B_X_FREE + kMaxMT,                                    // non-leader CTA only: remote rows of chunk 2*i have landed (st.async bytes)
+  B_OUT_FREE = B_LAND + kMaxMT,                 // leader: the output epilogue has read lin_out's result out of the h region
   B_COUNT
 };
 static_assert(B_COUNT <= 30, "barrier parity bits live in one 32-bit word");
 static_assert(Smem::total <= 227 * 1024, "shared memory budget");
 
 struct ProgEntry { uint32_t w0, w1; };
+template <int MT>
 __device__ inline ProgEntry make_prog(const Sched& sc, int s, uint32_t sbase) {
-  const Seg g = walk_stage(sc, s);
+  const Seg g = walk_stage<MT>(sc, s);
   uint32_t b_addr = 0, dcol = 0, acc = 1, wait_id = 0, c1 = 0, c2 = 0, c3 = 0;
   const bool last = g.t == g.len - 1;
   switch (g.kind) {
@@ -178,19 +204,19 @@ __device__ inline ProgEntry make_prog(const Sched& sc, int s, uint32_t sbase) {
       if (g.t == 0) wait_id = B_IN_READY + 1;
       break;
     case MAT_LINZ: {
-      const ZPos z = z_position(sc.KBz, g.t);
+      const ZPos z = z_position<MT>(sc.KBz, g.t);
       const bool streaming = z_passes(sc) > 1 || sc.proj;      // the latent tile is refilled for every pass / lin_z layer
-      const bool pass_first = z.mt == 0 && z.kbi == 0, pass_last = z.mt == kMT - 1 && z.kbi == z.kp - 1;
+      const bool pass_first = z.mt == 0 && z.kbi == 0, pass_last = z.mt == MT - 1 && z.kbi == z.kp - 1;
       b_addr = sbase + Smem::lat + z.kbi * kOperandKB; dcol = z.mt * 128;
       if (streaming && pass_first && !(g.blk == 0 && z.pass == 0)) wait_id = B_IN_READY + 1;
       if (pass_last && (streaming || g.blk == sc.n_linz - 1)) c1 = B_IN_FREE + 1;
-      if (last && g.blk == 0) { c2 = B_X_FULL + 1; c3 = B_X_FULL + 2; }
+      if (last && g.blk == 0) { c2 = B_X_FULL + 1; if (MT > 1) c3 = B_X_FULL + 2; }
     } break;
     case MAT_FC0:
     case MAT_FC1: {
       int kc, mt, kk;
       bool first_of_tile, last_of_tile;
-      fc_pair(g.t, kc, mt, kk, first_of_tile, last_of_tile);
+      fc_pair<MT>(g.t, kc, mt, kk, first_of_tile, last_of_tile);
       const bool fc0 = g.kind == MAT_FC0;
       b_addr = sbase + Smem::ring + (kc * 2 + kk) * kOperandKB; dcol = (fc0 ? kHCol : 0) + mt * 128;
       if (fc0) acc = first_of_tile ? 0 : 1;                      // fc_1 always accumulates into x
@@ -271,8 +297,8 @@ __device__ __forceinline__ void store_transposed(uint32_t base, const uint32_t* 
 // waiting for their remote rows to be performed (14.5 % of all warp-stall samples of a synchronous exchange).  Rows landing
 // in the leader are counted directly on the chunk barrier the MMA warp waits on; rows landing in the non-leader are counted
 // on its B_LAND barrier, and its otherwise idle warp 1 relays that to the leader.
-// VMAX: combine_type "max".
-template <int NS, bool VMAX>
+// VMAX: combine_type "max".  MT: 256-feature tiles of the padded hidden width (1 or 2, see Sched).
+template <int NS, bool VMAX, int MT>
 __global__ void __launch_bounds__(kThreads, 1)
 field_pair_kernel(const pnr_scene sc, const pnr_points q, const __grid_constant__ CUtensorMap wmap,
                   const float* __restrict__ bias_x, const float* __restrict__ bias_h,
@@ -286,7 +312,8 @@ field_pair_kernel(const pnr_scene sc, const pnr_points q, const __grid_constant_
   constexpr int NLIVE = G * PP;                        // live columns of a post-combine tile (<= 64)
   const bool pooled = NS > 1 || sch.CL < sch.n_blocks;   // false: no block after the combine step, lin_out follows it
   const int n_sg = ((n_tiles + 1) / 2 + G - 1) / G;
-  float* const xbar = xbar_all + (size_t)pair_id * (2 * kNCol * kHidden);   // [tile slot 2][column 64][feature 512]
+  // [tile slot 2][column 64][feature 512]: laid out for the widest hidden layer whatever MT is (features >= Hp unused)
+  float* const xbar = xbar_all + (size_t)pair_id * (2 * kNCol * kHidden);
   extern __shared__ __align__(1024) uint8_t smem[];
   const uint32_t sbase = smem_u32(smem);
   volatile uint32_t* tmem_base_slot = reinterpret_cast<volatile uint32_t*>(smem + Smem::bars + 8 * B_COUNT);
@@ -300,19 +327,19 @@ field_pair_kernel(const pnr_scene sc, const pnr_points q, const __grid_constant_
     for (int i = 0; i < kStages; ++i) { mbar_init(bar(B_W_FULL + i), 1); mbar_init(bar(B_W_EMPTY + i), 1); }
     mbar_init(bar(B_IN_READY), 2 * kGatherWarps);
     mbar_init(bar(B_IN_FREE), 1);
-    for (int i = 0; i < kMT; ++i) { mbar_init(bar(B_X_FULL + i), 1); mbar_init(bar(B_H_FULL + i), 1); }
+    for (int i = 0; i < MT; ++i) { mbar_init(bar(B_X_FULL + i), 1); mbar_init(bar(B_H_FULL + i), 1); }
     // chunk kc is produced by CTA kc % 2; even chunks need one more arrival: the relay of the non-leader CTA
-    for (int i = 0; i < 4; ++i) mbar_init(bar(B_RDY + i), kEpiWarps + ((i & 1) == 0 ? 1 : 0));
-    for (int i = 0; i < kMT; ++i) mbar_init(bar(B_LAND + i), kEpiWarps);
+    for (int i = 0; i < 2 * MT; ++i) mbar_init(bar(B_RDY + i), kEpiWarps + ((i & 1) == 0 ? 1 : 0));
+    for (int i = 0; i < MT; ++i) mbar_init(bar(B_LAND + i), kEpiWarps);
     mbar_init(bar(B_OUT_FREE), 2);
-    for (int i = 0; i < kMT; ++i) mbar_init(bar(B_X_FREE + i), 2 * kEpiWarps);
+    for (int i = 0; i < MT; ++i) mbar_init(bar(B_X_FREE + i), 2 * kEpiWarps);
     fence_barrier_init();
   }
-  const int n_stages = sched_total(sch);
-  const int s_pre = sched_pre(sch);                 // stages [0, s_pre) run per pre-combine tile, [s_pre, n_stages) per super group
+  const int n_stages = sched_total<MT>(sch);
+  const int s_pre = sched_pre<MT>(sch);                 // stages [0, s_pre) run per pre-combine tile, [s_pre, n_stages) per super group
   const int n_flat = G * s_pre + (n_stages - s_pre);   // weight stages one super group consumes
   for (int i = threadIdx.x; i < n_stages; i += kThreads) {
-    const ProgEntry pe = make_prog(sch, i, sbase);
+    const ProgEntry pe = make_prog<MT>(sch, i, sbase);
     reinterpret_cast<ProgEntry*>(smem + Smem::prog)[i] = pe;
     if (i == n_stages - 1) reinterpret_cast<ProgEntry*>(smem + Smem::prog)[n_stages] = pe;   // pad: the issuer prefetches entry st + 1
   }
@@ -369,7 +396,7 @@ field_pair_kernel(const pnr_scene sc, const pnr_points q, const __grid_constant_
             const bool after_mean = seg > 0 && seg < G;
             if (after_mean) {
               // the view-mean epilogue of the previous tile must have read x tile 0 out of TMEM before lin_in (stage 0) overwrites
-              // it; tile 1 is first written by stage 1 (see below)
+              // it; tile 1 (MT = 2) is first written by stage 1 (see below)
               mbar_wait_cluster(bar(B_X_FREE), (ph >> B_X_FREE) & 1u);
               ph ^= (1u << B_X_FREE);
               tc_fence_after();
@@ -410,7 +437,7 @@ field_pair_kernel(const pnr_scene sc, const pnr_points q, const __grid_constant_
               cur = nxt;
             };
             int st = st_beg;
-            if (after_mean) {                               // lin_in's second stage is the first write into x tile 1
+            if (MT > 1 && after_mean) {                     // lin_in's second stage is the first write into x tile 1
               issue_stage(st++);
               mbar_wait_cluster(bar(B_X_FREE + 1), (ph >> (B_X_FREE + 1)) & 1u);
               ph ^= (1u << (B_X_FREE + 1));
@@ -428,7 +455,7 @@ field_pair_kernel(const pnr_scene sc, const pnr_points q, const __grid_constant_
       for (int sg = pair_id; sg < n_sg; sg += n_pairs) {
         for (int i = 0; i < n_pub; ++i) {
 #pragma unroll
-          for (int mt = 0; mt < kMT; ++mt) {
+          for (int mt = 0; mt < MT; ++mt) {
             mbar_wait_cluster(bar(B_LAND + mt), par);
             fence_proxy_async();
             __syncwarp();
@@ -476,7 +503,7 @@ field_pair_kernel(const pnr_scene sc, const pnr_points q, const __grid_constant_
       store_transposed<kNCol / 2, false, true>(loc, u, bias, lane, qd * 32, hs * (kNCol / 2));
     };
     auto x_epilogue = [&](int e) {                 // relu(x + cumulative bias) -> bf16 K-chunks
-      for (int mt = 0; mt < kMT; ++mt) {
+      for (int mt = 0; mt < MT; ++mt) {
         // the bias is fetched BEFORE the wait: a global load issued after it sits on the hand-off's critical path
         const float bias = __ldg(bias_x + e * kHidden + mt * 256 + crank * 128 + fl);
         wait(B_X_FULL + mt);
@@ -486,7 +513,7 @@ field_pair_kernel(const pnr_scene sc, const pnr_points q, const __grid_constant_
       }
     };
     auto h_epilogue = [&](int b) {                 // relu(fc_0 out + b) -> bf16 K-chunks for fc_1
-      for (int mt = 0; mt < kMT; ++mt) {
+      for (int mt = 0; mt < MT; ++mt) {
         const float bias = __ldg(bias_h + b * kHidden + mt * 256 + crank * 128 + fl);
         wait(B_H_FULL + mt);
         const int kc = 2 * mt + (int)crank;
@@ -502,14 +529,14 @@ field_pair_kernel(const pnr_scene sc, const pnr_points q, const __grid_constant_
         const int obj = tile / tiles_per_obj;
         const int p0 = (tile - obj * tiles_per_obj) * PP;
         for (int e = 0; e < sch.CL; ++e) { x_epilogue(e); h_epilogue(e); }
-        float bias_mean[kMT];
+        float bias_mean[MT];
 #pragma unroll
-        for (int mt = 0; mt < kMT; ++mt) bias_mean[mt] = __ldg(bias_x + sch.CL * kHidden + mt * 256 + (int)crank * 128 + fl);
-        for (int mt = 0; mt < kMT; ++mt) wait(B_X_FULL + mt);
+        for (int mt = 0; mt < MT; ++mt) bias_mean[mt] = __ldg(bias_x + sch.CL * kHidden + mt * 256 + (int)crank * 128 + fl);
+        for (int mt = 0; mt < MT; ++mt) wait(B_X_FULL + mt);
         // view pooling (combine_interleaved) + cumulative bias -> x-bar, column g*PP + p of slot hs.  max(x_v + b) = max(x_v) + b
         // exactly: rounding is monotonic
 #pragma unroll
-        for (int mt = 0; mt < kMT; ++mt) {
+        for (int mt = 0; mt < MT; ++mt) {
           const int f = mt * 256 + (int)crank * 128 + fl;
           const float bias = bias_mean[mt];
           uint32_t v[kNCol];
@@ -543,7 +570,7 @@ field_pair_kernel(const pnr_scene sc, const pnr_points q, const __grid_constant_
       tc_fence_before();
       asm volatile("bar.sync %0, 64;" ::"r"(1 + qd) : "memory");
       tc_fence_after();
-      for (int mt = 0; mt < kMT; ++mt) {
+      for (int mt = 0; mt < MT; ++mt) {
         const int kc = 2 * mt + (int)crank;
         const int f = mt * 256 + (int)crank * 128 + fl;
         const uint32_t loc = sbase + Smem::ring + kc * kChunkBytes;
@@ -648,7 +675,8 @@ field_pair_kernel(const pnr_scene sc, const pnr_points q, const __grid_constant_
       for (int fill = 0; fill < fills; ++fill) {
         const int pass = fill % n_pass;
         const int kp = sch.KBz - pass * 8 < 8 ? sch.KBz - pass * 8 : 8;
-        const int ch0 = sch.proj ? (fill / n_pass) * kHidden : pass * 512;   // projected maps: lin_z[b]'s own 512-channel slice
+        // projected maps: lin_z[b]'s own d_hidden-channel slice (one pass, KBz = d_hidden / 64)
+        const int ch0 = sch.proj ? (fill / n_pass) * (sch.KBz * kBlockK) : pass * 512;
         // ---- 4 taps x 1 KiB per column, two columns in flight per warp (the loads are L2 hits with ~1-2 k cycles of
         // latency under the weight stream's load; one column at a time left the tensor cores waiting for the gather)
         const bool act = (lane >> 2) < kp;
@@ -733,25 +761,27 @@ field_pair_kernel(const pnr_scene sc, const pnr_points q, const __grid_constant_
 
 // ---- host side ---------------------------------------------------------------------------------------------
 static pair::Sched pair_sched(const pnr_mlp_params* p, int proj) {
-  return pair::Sched{p->n_blocks, p->combine_layer, p->combine_layer, proj ? kHidden / 64 : p->d_latent / 64, proj};
+  return pair::Sched{p->n_blocks, p->combine_layer, p->combine_layer, proj ? p->d_hidden / 64 : p->d_latent / 64, proj};
 }
-size_t pair_stream_bytes(const pnr_mlp_params* p, int proj) {
-  pair::Sched s = pair_sched(p, proj);
-  return (size_t)pair::sched_total(s) * 2 * kStageBytes;
-}
+// padded hidden width Hp of the packed network: 256 * hidden_tiles
+int hidden_tiles(const pnr_mlp_params* p) { return p->d_hidden <= 256 ? 1 : 2; }
 int pair_stages(const pnr_mlp_params* p, int proj) {
   pair::Sched s = pair_sched(p, proj);
-  return pair::sched_total(s);
+  return hidden_tiles(p) == 1 ? pair::sched_total<1>(s) : pair::sched_total<2>(s);
 }
+size_t pair_stream_bytes(const pnr_mlp_params* p, int proj) { return (size_t)pair_stages(p, proj) * 2 * kStageBytes; }
 int pair_pack(const pnr_mlp_params* p, uint8_t* stream, int proj, cudaStream_t st) {
   pair::Sched s = pair_sched(p, proj);
-  PNR_REQUIRE(pair::sched_total(s) < pair::kMaxStages, PNR_ERR_UNSUPPORTED, "pair_pack: %d stages exceed the stage program (one padding entry is needed)", pair::sched_total(s));
-  pair::pack_stages_kernel<<<pair::sched_total(s) * 2, 256, 0, st>>>(*p, s, stream);
+  const int n = pair_stages(p, proj);
+  PNR_REQUIRE(n < pair::kMaxStages, PNR_ERR_UNSUPPORTED, "pair_pack: %d stages exceed the stage program (one padding entry is needed)", n);
+  if (hidden_tiles(p) == 1) pair::pack_stages_kernel<1><<<n * 2, 256, 0, st>>>(*p, s, stream);
+  else pair::pack_stages_kernel<2><<<n * 2, 256, 0, st>>>(*p, s, stream);
   PNR_CHECK_LAUNCH("pair::pack_stages_kernel");
   return PNR_OK;
 }
 
-// scratch for the view means: 2 tiles x 64 columns x 512 features fp32 per resident CTA pair
+// scratch for the view means: 2 tiles x 64 columns x 512 features fp32 per resident CTA pair.  Sized for the widest hidden
+// layer: an upper bound for narrower networks (pnr_field_workspace_bytes has no parameters to size it from).
 size_t pair_workspace_bytes() {
   int dev = 0, sms = 148;
   cudaGetDevice(&dev);
@@ -786,7 +816,7 @@ int field_forward_pair(const pnr_scene* sc, const pnr_points* q, const pnr_mlp_p
     encode = (EncodeFn)fn;
   }
   CUtensorMap tmap;
-  cuuint64_t gdim[2] = {64, (cuuint64_t)pair::sched_total(sch) * 256};
+  cuuint64_t gdim[2] = {64, (cuuint64_t)pair_stages(mp, proj) * 256};
   cuuint64_t gstride[1] = {128};
   cuuint32_t box[2] = {64, 128};
   cuuint32_t estr[2] = {1, 1};
@@ -801,9 +831,11 @@ int field_forward_pair(const pnr_scene* sc, const pnr_points* q, const pnr_mlp_p
   // max over one view is the view itself: NS == 1 runs the average instantiation whatever combine_type says
   const bool vmax = mp->combine_type == PNR_COMBINE_MAX && sc->NS > 1;
   const int n_groups = ((n_tiles + 1) / 2 + G - 1) / G;  // super groups
+  const bool mt1 = hidden_tiles(mp) == 1;
 #define PNR_LAUNCH_PAIR(NSV)                                                                                     \
   case NSV: {                                                                                                    \
-    auto kern = vmax ? pair::field_pair_kernel<NSV, (NSV > 1)> : pair::field_pair_kernel<NSV, false>;            \
+    auto kern = mt1 ? (vmax ? pair::field_pair_kernel<NSV, (NSV > 1), 1> : pair::field_pair_kernel<NSV, false, 1>)  \
+                    : (vmax ? pair::field_pair_kernel<NSV, (NSV > 1), 2> : pair::field_pair_kernel<NSV, false, 2>); \
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pair::Smem::total); \
     PNR_REQUIRE(e == cudaSuccess, PNR_ERR_CUDA, "cudaFuncSetAttribute: %s", cudaGetErrorString(e));             \
     cudaLaunchConfig_t cfg = {};                                                                                 \

@@ -33,7 +33,12 @@ void reset_launch_count();
   } while (0)
 
 constexpr int kZFeat = 42;      // 39 positional-encoding values + 3 rotated view-direction values
-constexpr int kHidden = 512;    // ResnetFC d_hidden of every shipped conf (conf/default*.conf)
+constexpr int kHidden = 512;    // widest ResnetFC d_hidden the library runs (that of every shipped conf, conf/default*.conf)
+// ResnetFC hidden widths the field and training paths run: the multiples of 64 up to kHidden
+__host__ __device__ inline bool hidden_width_supported(int d_hidden) {
+  return d_hidden >= 64 && d_hidden <= kHidden && d_hidden % 64 == 0;
+}
+#define PNR_HIDDEN_WIDTHS "64, 128, ..., 512 (multiples of 64)"
 
 // Per-point camera-space quantities for one source view (models.py:168-230, encoder.py:94-98).
 struct Projection {
