@@ -35,9 +35,8 @@ EXPORTS = [
     "pnr_mlp_pack_projected_bytes", "pnr_mlp_pack_projected", "pnr_project_features",
     "pnr_render_workspace_bytes", "pnr_render_forward",
 ]
-# lab equipment (csrc/pnr_lab.h, internal): micro-benchmarks and the tcgen05 self test; not part of the product ABI
-LAB_EXPORTS = ["pnr_umma_selftest", "pnr_ingest_bench", "pnr_ingest_bench_tma", "pnr_umma_bench", "pnr_umma2_bench", "pnr_tma_latency_bench", "pnr_dsmem_bench",
-               "pnr_lab_gemm_workspace_bytes", "pnr_lab_rowgemm", "pnr_lab_wgrad"]
+# test hooks of the training GEMMs (csrc/pnr_lab.h, internal); not part of the product ABI
+LAB_EXPORTS = ["pnr_lab_gemm_workspace_bytes", "pnr_lab_rowgemm", "pnr_lab_wgrad"]
 ABI_VERSION = 3
 
 
@@ -139,18 +138,11 @@ def load() -> C.CDLL:
     lib.pnr_field_workspace_bytes.restype = C.c_size_t
     lib.pnr_field_forward.argtypes = [C.POINTER(Scene), C.POINTER(Points), C.POINTER(MlpParams), vp, vp, vp,
                                       C.c_size_t, i32, i32, f32, vp]
-    lib.pnr_umma_selftest.argtypes = [vp, vp, vp, vp, i32, i32, vp]
     lib.pnr_resnetfc_workspace_bytes.argtypes = [C.POINTER(MlpParams), C.c_longlong]
     lib.pnr_resnetfc_workspace_bytes.restype = C.c_size_t
     lib.pnr_resnetfc_forward.argtypes = [C.POINTER(MlpParams), vp, C.c_longlong, i32, i32, vp, vp, C.c_size_t, vp]
     lib.pnr_positional_encoding.argtypes = [vp, vp, C.c_longlong, i32, i32, f32, i32, vp]
     lib.pnr_index_features.argtypes = [C.POINTER(Scene), vp, i32, i32, vp, vp]
-    lib.pnr_ingest_bench.argtypes = [vp, i32, i32, i32, i32, vp, i32, i32, i32, vp]
-    lib.pnr_ingest_bench_tma.argtypes = [vp, i32, i32, i32, i32, vp, i32, i32, vp]
-    lib.pnr_umma_bench.argtypes = [i32, i32, i32, i32, i32, vp, i32, vp]
-    lib.pnr_umma2_bench.argtypes = [i32, i32, i32, i32, i32, i32, vp, vp, vp]
-    lib.pnr_tma_latency_bench.argtypes = [vp, i32, i32, i32, i32, i32, vp, vp]
-    lib.pnr_dsmem_bench.argtypes = [i32, i32, i32, i32, vp, vp]
     lib.pnr_lab_gemm_workspace_bytes.argtypes = [C.c_longlong, i32, i32]
     lib.pnr_lab_gemm_workspace_bytes.restype = C.c_size_t
     lib.pnr_lab_rowgemm.argtypes = [vp, vp, vp, vp, vp, vp, vp, C.c_longlong, i32, i32, i32, vp, C.c_size_t, vp]

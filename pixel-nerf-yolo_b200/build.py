@@ -15,7 +15,7 @@ from concurrent.futures import ThreadPoolExecutor
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT = os.path.join(CSRC, "libpixelnerf_b200.so")
-SOURCES = ["api.cu", "ray_tile.cu", "gather_pe.cu", "mlp_fp32.cu", "mlp_dispatch.cu", "mlp_umma_pair.cu", "field_bwd.cu", "encode_rays.cu", "lab.cu", "train_umma.cu"]
+SOURCES = ["api.cu", "ray_tile.cu", "gather_pe.cu", "mlp_fp32.cu", "mlp_dispatch.cu", "mlp_umma_pair.cu", "field_bwd.cu", "encode_rays.cu", "train_umma.cu"]
 HEADERS = ["pnr_common.cuh", "umma.cuh", "pnr_lab.h", "train_umma.cuh", os.path.join("..", "..", "include", "pixelnerf_b200.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "-Xptxas", "-v"]

@@ -4,7 +4,7 @@
 // the two SMs of a cluster of 2:  M = 256 features (128 per CTA), N = 128 columns (64 per CTA: each CTA gathers and
 // owns its own tile of 64 columns = PP points x NS views), K = 16.
 //   * per MMA each CTA reads 4 KiB of weights + 2 KiB of activations from its own shared memory for 4x the MACs of
-//     the single-CTA N=64 MMA, and N=128 runs the tensor pipe at its full rate (scripts/umma_bench.py);
+//     the single-CTA N=64 MMA, and N=128 runs the tensor pipe at its full rate (DESIGN.md section 4.1);
 //   * each CTA streams only ITS half (128 rows) of every 256-row weight slab (tensor-map TMA, cta_group::2, completion
 //     on the leader's mbarrier);
 //   * TMEM per CTA: x^T = MT feature tiles x 128 columns (cols [0,256)), h^T likewise (cols [256,512)).
@@ -30,7 +30,6 @@
 //   OUT_FREE   @L    : the output epilogue has read lin_out's result
 #include "pnr_common.cuh"
 #include "umma.cuh"
-#include <cuda.h>
 
 namespace pnr {
 using namespace umma;
@@ -804,62 +803,30 @@ int field_forward_pair(const pnr_scene* sc, const pnr_points* q, const pnr_mlp_p
   const int n_tiles = (int)n_tiles_ll;
   // tensor map over the packed pair stream: rows = stages x 256, 64 bf16 per row (128 B), box = 64 x 128, no swizzle
   // (the stream is already stored in the swizzled operand layout)
-  typedef CUresult (*EncodeFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                               const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                               CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-  static EncodeFn encode = nullptr;
-  if (!encode) {
-    void* fn = nullptr;
-    cudaDriverEntryPointQueryResult qres;
-    cudaError_t e = cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres);
-    PNR_REQUIRE(e == cudaSuccess && fn, PNR_ERR_CUDA, "cuTensorMapEncodeTiled entry point not found");
-    encode = (EncodeFn)fn;
-  }
   CUtensorMap tmap;
-  cuuint64_t gdim[2] = {64, (cuuint64_t)pair_stages(mp, proj) * 256};
-  cuuint64_t gstride[1] = {128};
-  cuuint32_t box[2] = {64, 128};
-  cuuint32_t estr[2] = {1, 1};
-  CUresult r = encode(&tmap, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, (void*)stream, gdim, gstride, box, estr,
-                      CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                      CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  PNR_REQUIRE(r == CUDA_SUCCESS, PNR_ERR_CUDA, "cuTensorMapEncodeTiled failed (%d)", (int)r);
-  int dev = 0, sms = 148;
-  cudaGetDevice(&dev);
-  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+  int rc = make_map(&tmap, stream, (long long)pair_stages(mp, proj) * 256, 64, 64, 64, 128, false);
+  if (rc) return rc;
   const int G = pair::kNCol / PP;                        // tile pairs per super group (see field_pair_kernel)
   // max over one view is the view itself: NS == 1 runs the average instantiation whatever combine_type says
   const bool vmax = mp->combine_type == PNR_COMBINE_MAX && sc->NS > 1;
   const int n_groups = ((n_tiles + 1) / 2 + G - 1) / G;  // super groups
   const bool mt1 = hidden_tiles(mp) == 1;
-#define PNR_LAUNCH_PAIR(NSV)                                                                                     \
-  case NSV: {                                                                                                    \
-    auto kern = mt1 ? (vmax ? pair::field_pair_kernel<NSV, (NSV > 1), 1> : pair::field_pair_kernel<NSV, false, 1>)  \
-                    : (vmax ? pair::field_pair_kernel<NSV, (NSV > 1), 2> : pair::field_pair_kernel<NSV, false, 2>); \
-    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pair::Smem::total); \
-    PNR_REQUIRE(e == cudaSuccess, PNR_ERR_CUDA, "cudaFuncSetAttribute: %s", cudaGetErrorString(e));             \
-    cudaLaunchConfig_t cfg = {};                                                                                 \
-    cudaLaunchAttribute attr[1];                                                                                 \
-    attr[0].id = cudaLaunchAttributeClusterDimension;                                                            \
-    attr[0].val.clusterDim.x = 2; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;                    \
-    cfg.blockDim = dim3(pair::kThreads); cfg.dynamicSmemBytes = pair::Smem::total; cfg.stream = st;              \
-    cfg.attrs = attr; cfg.numAttrs = 1;                                                                          \
-    cfg.gridDim = dim3(sms / 2 * 2);                                                                             \
-    int max_pairs = sms / 2, mc = 0;                                                                             \
-    if (cudaOccupancyMaxActiveClusters(&mc, kern, &cfg) == cudaSuccess && mc > 0 && mc < max_pairs) max_pairs = mc; \
-    const int n_pairs = n_groups < max_pairs ? n_groups : max_pairs;                                             \
-    cfg.gridDim = dim3(n_pairs * 2);                                                                             \
-    e = cudaLaunchKernelEx(&cfg, kern, *sc, *q, tmap, bx, bh, bo, out, xbar, sch, num_freqs, freq_factor, tiles_per_obj, \
-                           n_tiles, (int)mp->d_out, raw);                                                        \
-    PNR_REQUIRE(e == cudaSuccess, PNR_ERR_CUDA, "field_pair_kernel launch: %s", cudaGetErrorString(e));          \
-  } break;
+  decltype(&pair::field_pair_kernel<1, false, 1>) kern = nullptr;
+#define PNR_PAIR_KERNEL(NSV)                                                                                     \
+  case NSV:                                                                                                      \
+    kern = mt1 ? (vmax ? pair::field_pair_kernel<NSV, (NSV > 1), 1> : pair::field_pair_kernel<NSV, false, 1>)     \
+               : (vmax ? pair::field_pair_kernel<NSV, (NSV > 1), 2> : pair::field_pair_kernel<NSV, false, 2>);    \
+    break;
   switch (sc->NS) {
-    PNR_LAUNCH_PAIR(1) PNR_LAUNCH_PAIR(2) PNR_LAUNCH_PAIR(3) PNR_LAUNCH_PAIR(4) PNR_LAUNCH_PAIR(5) PNR_LAUNCH_PAIR(6) PNR_LAUNCH_PAIR(8)
+    PNR_PAIR_KERNEL(1) PNR_PAIR_KERNEL(2) PNR_PAIR_KERNEL(3) PNR_PAIR_KERNEL(4) PNR_PAIR_KERNEL(5) PNR_PAIR_KERNEL(6) PNR_PAIR_KERNEL(8)
     default: PNR_REQUIRE(false, PNR_ERR_UNSUPPORTED, "field_forward_pair: NS=%d", sc->NS);
   }
-#undef PNR_LAUNCH_PAIR
-  PNR_CHECK_LAUNCH("field_pair_kernel");
-  return PNR_OK;
+#undef PNR_PAIR_KERNEL
+  int max_pairs;
+  if ((rc = pair_capacity(kern, pair::kThreads, pair::Smem::total, &max_pairs))) return rc;
+  const int n_pairs = n_groups < max_pairs ? n_groups : max_pairs;
+  return launch_pairs(kern, n_pairs, pair::kThreads, pair::Smem::total, st, "field_pair_kernel", *sc, *q, tmap, bx, bh, bo, out,
+                      xbar, sch, num_freqs, freq_factor, tiles_per_obj, n_tiles, (int)mp->d_out, raw);
 }
 
 }  // namespace pnr

@@ -1,33 +1,11 @@
-/* Internal header: design-aid micro-benchmarks and the tcgen05 building-block self test (lab.cu).  NOT part of the product
- * ABI (include/pixelnerf_b200.h); used by scripts/{ingest,umma,dsmem}_bench.py and tests/test_gpu_parity.py::test_umma_selftest. */
+/* Internal header, NOT part of the product ABI (include/pixelnerf_b200.h): test hooks of the training GEMMs, used by
+ * tests/test_gpu_train.py, scripts/rowgemm_bench.py and scripts/wgrad_probe.py. */
 #ifndef PNR_LAB_H
 #define PNR_LAB_H
 #include <stddef.h>
 #ifdef __cplusplus
 extern "C" {
 #endif
-/* D(128 x N) = A(128 x K) * B(N x K)^T with bf16 operands staged exactly like the fused kernel (bulk-copied pre-swizzled A,
- * thread-written swizzled B, TMEM accumulator, tcgen05.ld epilogue).  a (128,K), b (N,K) fp32 device inputs, d (128,N) fp32
- * device output; workspace: K/64 * 16 KiB, 1024-byte aligned.  N in {16,32,48,64}, K multiple of 64 <= 512. */
-int pnr_umma_selftest(const float* a, const float* b, float* d, void* workspace, int N, int K, void* stream);
-/* per-SM cp.async.bulk ingest (16 KiB stages, `depth`-slot ring, `grid` CTAs streaming `n_stages` stages each from a buffer of
- * `src_stages` stages).  out[grid] = elapsed SM cycles per CTA. */
-int pnr_ingest_bench(const void* src, int src_stages, int n_stages, int depth, int grid, long long* out,
-                     int n_prod, int n_cons, int stage_bytes, void* stream);
-/* same through a 2-D tensor map (cp.async.bulk.tensor.2d), box = 64 x box_rows bf16, optional 128B swizzle. */
-int pnr_ingest_bench_tma(const void* src, int src_stages, int n_stages, int depth, int grid, long long* out,
-                         int box_rows, int swizzle, void* stream);
-/* latency of k 16 KiB loads issued back to back per CTA of a cluster of 2 (mode 0 bulk 1-D, 1 tensor-map box, 2 the field kernel's
- * cta_group::2 form completing on the leader's barrier); out[2 * pairs] = cycles summed over iters. */
-int pnr_tma_latency_bench(const void* src, int src_stages, int iters, int mode, int k, int pairs, long long* out, void* stream);
-/* cycles for `iters` x 8 tcgen05.mma (kind::f16, bf16, K=16) of shape M x N issued back to back from shared-memory operands. */
-int pnr_umma_bench(int M, int N, int iters, int a_stride_kb, int grid, long long* out, int commit_every, void* stream);
-/* the CTA-pair MMA (cta_group::2, M = 256, N) in isolation: out[pairs] = cycles for iters x 8 MMAs; bg bit 0 = concurrent 16 KiB
- * bulk copies from src (pairs * 4 MiB) into shared memory, bit 1 = concurrent st.shared traffic. */
-int pnr_umma2_bench(int N, int iters, int commit_every, int a_slots, int bg, int pairs, const void* src, long long* out, void* stream);
-/* distributed-shared-memory ping-pong of `bytes` between the two CTAs of a cluster.  mode 0: st.shared::cluster.v4 by `warps`
- * warps + proxy fence + remote arrive; mode 1: one cp.async.bulk smem->peer smem.  out[2] = cycles for `iters` transfers. */
-int pnr_dsmem_bench(int mode, int bytes, int iters, int warps, long long* out, void* stream);
 /* Stand-alone entry points of the tcgen05 training GEMMs (train_umma.cu): fp32 device inputs are rounded to bf16, then
  * out[M,N] = epilogue(A[M,K] W[N,K]^T) (rowgemm: optional bias [N], relu mask source [M,N], residual [M,N]; fp32 and / or bf16
  * outputs) and dW[N,K] += dY[M,N]^T X[M,K] (wgrad).  workspace: pnr_lab_gemm_workspace_bytes(M, N, K). */

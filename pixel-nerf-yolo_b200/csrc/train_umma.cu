@@ -17,7 +17,7 @@
 #include "pnr_common.cuh"
 #include "umma.cuh"
 #include "train_umma.cuh"
-#include <cuda.h>
+#include "pnr_lab.h"
 
 namespace pnr {
 namespace tg {
@@ -41,21 +41,6 @@ struct SmemG {
 };
 enum { G_FULL = 0, G_EMPTY = G_FULL + kStagesG, G_ACC_FULL = G_EMPTY + kStagesG, G_ACC_FREE = G_ACC_FULL + 2, G_COUNT = G_ACC_FREE + 2 };
 static_assert(SmemG::total <= 227 * 1024, "shared memory budget");
-
-__device__ __forceinline__ void tma_load_2d_2sm_sw(uint32_t dst, const void* tmap, int c0, int c1, uint32_t bar) {
-  tma_load_2d_2sm(dst, tmap, c0, c1, bar);
-}
-// kind::f16, bf16 x bf16 -> f32, M = 256 (pair), N = n; a_mn / b_mn: operand is MN-major instead of K-major
-__host__ __device__ inline uint32_t idesc_2sm(int n, int a_mn, int b_mn) {
-  return (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)a_mn << 15) | ((uint32_t)b_mn << 16) | ((uint32_t)(n >> 3) << 17) |
-         ((uint32_t)(256 >> 4) << 24);
-}
-// MN-major SWIZZLE_128B tile made of 64-feature x 64-row boxes (8 KiB each) laid one after the other along MN:
-// LBO = byte distance between 64-element MN atoms = 8 192, SBO = byte distance between 8-row K groups = 1 024
-__device__ __forceinline__ uint64_t smem_desc_mn(uint32_t saddr) {
-  constexpr uint32_t lbo = 8192, sbo = 1024;
-  return (uint64_t)((saddr >> 4) & 0x3FFFu) | ((uint64_t)(lbo >> 4) << 16) | ((uint64_t)(sbo >> 4) << 32) | (1ull << 46) | (2ull << 61);
-}
 
 // ------------------------------------------------------------------------------------------------------------------------
 template <bool kDummy>
@@ -117,7 +102,7 @@ rowgemm_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constant_
     __syncwarp();
   } else if (warp == 1) {
     if (crank == 0 && elect_one()) {
-      const uint32_t idesc = idesc_2sm(256, 0, 0);
+      const uint32_t idesc = instr_desc_bf16_2sm(256);
       uint32_t slot = 0, fpar = 0;
       long long i = 0;
       for (long long u = pair_id; u < n_units; u += n_pairs, ++i) {
@@ -385,7 +370,7 @@ wgrad_kernel(const __grid_constant__ CUtensorMap mapY, const __grid_constant__ C
     __syncwarp();
   } else if (warp == 1) {
     if (crank == 0 && elect_one()) {
-      const uint32_t idesc = idesc_2sm(256, 1, 1);
+      const uint32_t idesc = instr_desc_bf16_2sm(256, 1, 1);
       uint32_t slot = 0, fpar = 0;
       long long i = 0;
       for (long long u = pair_id; u < n_units; u += n_pairs, ++i) {
@@ -488,53 +473,6 @@ __global__ void pack_rowgemm_many_kernel(const PackJobs jobs) {
   }
 }
 
-typedef CUresult (*EncodeFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                             const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                             CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-static EncodeFn get_encode() {
-  static EncodeFn encode = nullptr;
-  if (!encode) {
-    void* fn = nullptr;
-    cudaDriverEntryPointQueryResult qres;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres) == cudaSuccess) encode = (EncodeFn)fn;
-  }
-  return encode;
-}
-// 2-D bf16 tensor map over a row-major [rows x cols] matrix with leading dimension ld (elements); box = box_c x box_r
-static int make_map(CUtensorMap* m, const void* base, long long rows, long long cols, long long ld, int box_c, int box_r, bool swizzle) {
-  EncodeFn enc = get_encode();
-  PNR_REQUIRE(enc, PNR_ERR_CUDA, "cuTensorMapEncodeTiled entry point not found");
-  PNR_REQUIRE(((uintptr_t)base & 15) == 0 && (ld * 2) % 16 == 0, PNR_ERR_ARG, "tensor map: base / row pitch must be 16-byte aligned");
-  cuuint64_t gdim[2] = {(cuuint64_t)cols, (cuuint64_t)rows};
-  cuuint64_t gstride[1] = {(cuuint64_t)ld * 2};
-  cuuint32_t box[2] = {(cuuint32_t)box_c, (cuuint32_t)box_r};
-  cuuint32_t estr[2] = {1, 1};
-  CUresult r = enc(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(base), gdim, gstride, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                   swizzle ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  PNR_REQUIRE(r == CUDA_SUCCESS, PNR_ERR_CUDA, "cuTensorMapEncodeTiled failed (%d)", (int)r);
-  return PNR_OK;
-}
-
-// CTA pairs that can be co-resident (persistent kernels with a static round-robin over units must not exceed it)
-template <typename K>
-static int launch_pairs(K kern, int threads, int* n_pairs_out) {
-  int dev = 0, sms = 148;
-  cudaGetDevice(&dev);
-  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-  int pairs = sms / 2;
-  cudaLaunchConfig_t cfg = {};
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = 2; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
-  cfg.gridDim = dim3(pairs * 2); cfg.blockDim = dim3(threads); cfg.dynamicSmemBytes = SmemG::total;
-  cfg.attrs = attr; cfg.numAttrs = 1;
-  int mc = 0;
-  if (cudaOccupancyMaxActiveClusters(&mc, kern, &cfg) == cudaSuccess && mc > 0 && mc < pairs) pairs = mc;
-  *n_pairs_out = pairs;
-  return PNR_OK;
-}
-
 size_t packed_rowgemm_bytes(int n_out, int n_in) {
   const int nN = (n_out + 255) / 256, nK = (n_in + 63) / 64;
   return (size_t)nN * nK * 2 * kHalf;
@@ -588,22 +526,11 @@ int rowgemm(const RowGemmSrc& s0, const RowGemmSrc* s1, RowGemmArgs g, cudaStrea
     if ((rc = make_map(&mW1, s1->Wp, (long long)g.nN * g.nK1 * 256, 64, 64, 64, 128, false))) return rc;
   } else { mA1 = mA0; mW1 = mW0; }
   auto kern = rowgemm_kernel<false>;
-  cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SmemG::total);
-  PNR_REQUIRE(e == cudaSuccess, PNR_ERR_CUDA, "cudaFuncSetAttribute: %s", cudaGetErrorString(e));
-  int max_pairs = 74;
-  launch_pairs(kern, kThreadsR, &max_pairs);
+  int max_pairs;
+  if ((rc = pair_capacity(kern, kThreadsR, SmemG::total, &max_pairs))) return rc;
   const long long n_units = ((g.M + 255) / 256) * g.nN;
   const int n_pairs = (int)(n_units < max_pairs ? n_units : max_pairs);
-  cudaLaunchConfig_t cfg = {};
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = 2; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
-  cfg.gridDim = dim3(n_pairs * 2); cfg.blockDim = dim3(kThreadsR); cfg.dynamicSmemBytes = SmemG::total; cfg.stream = st;
-  cfg.attrs = attr; cfg.numAttrs = 1;
-  e = cudaLaunchKernelEx(&cfg, kern, mA0, mW0, mA1, mW1, g);
-  PNR_REQUIRE(e == cudaSuccess, PNR_ERR_CUDA, "rowgemm_kernel launch: %s", cudaGetErrorString(e));
-  PNR_CHECK_LAUNCH("tg::rowgemm_kernel");
-  return PNR_OK;
+  return launch_pairs(kern, n_pairs, kThreadsR, SmemG::total, st, "tg::rowgemm_kernel", mA0, mW0, mA1, mW1, g);
 }
 
 int wgrad(const __nv_bfloat16* dY, long long ldy, const __nv_bfloat16* X, long long ldx, float* dW, int ldw, long long M, int N, int K,
@@ -613,10 +540,8 @@ int wgrad(const __nv_bfloat16* dY, long long ldy, const __nv_bfloat16* X, long l
   WgradArgs g = {};
   g.dW = dW; g.ldw = ldw; g.M = M; g.N = N; g.K = K;
   g.nNb = (N + 255) / 256; g.nKb = (K + 255) / 256;
-  cudaError_t e = cudaFuncSetAttribute(wgrad_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SmemG::total);
-  PNR_REQUIRE(e == cudaSuccess, PNR_ERR_CUDA, "cudaFuncSetAttribute: %s", cudaGetErrorString(e));
-  int max_pairs = 74;
-  launch_pairs(wgrad_kernel, kThreadsG, &max_pairs);
+  int max_pairs, rc;
+  if ((rc = pair_capacity(wgrad_kernel, kThreadsG, SmemG::total, &max_pairs))) return rc;
   const long long steps = (M + 63) / 64;
   long long slabs = (2LL * max_pairs + g.nNb * g.nKb - 1) / (g.nNb * g.nKb);      // ~2 units per CTA pair
   if (slabs > steps) slabs = steps;
@@ -624,7 +549,6 @@ int wgrad(const __nv_bfloat16* dY, long long ldy, const __nv_bfloat16* X, long l
   g.n_slabs = (int)slabs;
   // boxes of 64 features x 64 rows; the feature extent is padded to the boxes by the caller's leading dimension (zero-filled OOB)
   CUtensorMap mY, mX;
-  int rc;
   // declared widths are rounded up to whole 64-feature boxes where the leading dimension has room (the caller's padding
   // columns are zero); anything beyond the declared width is zero-filled by the TMA unit
   auto width = [](int n, long long ld) -> long long { const long long r = (n + 63) / 64 * 64; return r <= ld ? r : n; };
@@ -632,17 +556,65 @@ int wgrad(const __nv_bfloat16* dY, long long ldy, const __nv_bfloat16* X, long l
   if ((rc = make_map(&mX, X, M, width(K, ldx), ldx, 64, 64, true))) return rc;
   const long long n_units = (long long)g.nNb * g.nKb * g.n_slabs;
   const int n_pairs = (int)(n_units < max_pairs ? n_units : max_pairs);
-  cudaLaunchConfig_t cfg = {};
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = 2; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
-  cfg.gridDim = dim3(n_pairs * 2); cfg.blockDim = dim3(kThreadsG); cfg.dynamicSmemBytes = SmemG::total; cfg.stream = st;
-  cfg.attrs = attr; cfg.numAttrs = 1;
-  e = cudaLaunchKernelEx(&cfg, wgrad_kernel, mY, mX, g);
-  PNR_REQUIRE(e == cudaSuccess, PNR_ERR_CUDA, "wgrad_kernel launch: %s", cudaGetErrorString(e));
-  PNR_CHECK_LAUNCH("tg::wgrad_kernel");
-  return PNR_OK;
+  return launch_pairs(wgrad_kernel, n_pairs, kThreadsG, SmemG::total, st, "tg::wgrad_kernel", mY, mX, g);
 }
 
 }  // namespace tg
 }  // namespace pnr
+
+// ---- stand-alone entry points of the two GEMMs (csrc/pnr_lab.h), for tests/test_gpu_train.py and scripts/ ------------------------
+namespace pnr {
+__global__ void lab_to_bf16_kernel(const float* __restrict__ src, __nv_bfloat16* __restrict__ dst, long long rows, int cols, int ld) {
+  const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= rows * ld) return;
+  const long long r = i / ld;
+  const int c = (int)(i - r * ld);
+  dst[i] = __float2bfloat16_rn(c < cols ? src[r * cols + c] : 0.f);
+}
+}  // namespace pnr
+
+extern "C" size_t pnr_lab_gemm_workspace_bytes(long long M, int N, int K) {
+  const size_t ldk = (size_t)((K + 63) / 64 * 64), ldn = (size_t)((N + 63) / 64 * 64);
+  return (size_t)M * ldk * 2 + (size_t)M * ldn * 2 + pnr::tg::packed_rowgemm_bytes(N, K) + 4096;
+}
+
+// out[M, N] = epilogue(A[M, K] W[N, K]^T): A, W fp32 device inputs rounded to bf16; optional bias [N], mask_src [M, N] (fp32,
+// rounded to bf16), res_in [M, N]; out_f32 and / or out_bf16_as_f32 ([M, N] fp32 copy of the bf16 output) may be null.
+extern "C" int pnr_lab_rowgemm(const float* A, const float* W, const float* bias, const float* mask_src, const float* res_in,
+                               float* out_f32, void* out_bf16, long long M, int N, int K, int relu_out, void* workspace,
+                               size_t workspace_bytes, void* stream) {
+  using namespace pnr;
+  reset_launch_count();
+  PNR_REQUIRE(A && W && workspace && workspace_bytes >= pnr_lab_gemm_workspace_bytes(M, N, K), PNR_ERR_ARG, "pnr_lab_rowgemm: bad arguments");
+  cudaStream_t st = (cudaStream_t)stream;
+  const int ldk = (K + 63) / 64 * 64, ldn = (N + 63) / 64 * 64;
+  uint8_t* p = (uint8_t*)(((uintptr_t)workspace + 1023) & ~(uintptr_t)1023);
+  __nv_bfloat16* A16 = (__nv_bfloat16*)p; p += ((size_t)M * ldk * 2 + 1023) & ~(size_t)1023;
+  __nv_bfloat16* M16 = (__nv_bfloat16*)p; p += ((size_t)M * ldn * 2 + 1023) & ~(size_t)1023;
+  uint8_t* Wp = p;
+  lab_to_bf16_kernel<<<(unsigned)((M * ldk + 255) / 256), 256, 0, st>>>(A, A16, M, K, ldk);
+  if (mask_src) lab_to_bf16_kernel<<<(unsigned)((M * ldn + 255) / 256), 256, 0, st>>>(mask_src, M16, M, N, ldn);
+  int rc = tg::pack_rowgemm(W, N, K, K, 0, Wp, st);
+  if (rc) return rc;
+  tg::RowGemmArgs g = {};
+  g.M = M; g.n_valid = N; g.bias = bias; g.mask_src = mask_src ? M16 : nullptr; g.ld_mask = ldn; g.res_in = res_in; g.ld_res = N;
+  g.out_f32 = out_f32; g.ld_f32 = N; g.out_bf16 = (__nv_bfloat16*)out_bf16; g.ld_bf16 = N; g.relu_out = relu_out;
+  tg::RowGemmSrc s0 = {A16, ldk, ldk, Wp};
+  return tg::rowgemm(s0, nullptr, g, st);
+}
+
+// dW[N, K] += dY[M, N]^T X[M, K] (fp32 device inputs rounded to bf16)
+extern "C" int pnr_lab_wgrad(const float* dY, const float* X, float* dW, long long M, int N, int K, void* workspace,
+                             size_t workspace_bytes, void* stream) {
+  using namespace pnr;
+  reset_launch_count();
+  PNR_REQUIRE(dY && X && dW && workspace && workspace_bytes >= pnr_lab_gemm_workspace_bytes(M, N, K), PNR_ERR_ARG, "pnr_lab_wgrad: bad arguments");
+  cudaStream_t st = (cudaStream_t)stream;
+  const int ldk = (K + 63) / 64 * 64, ldn = (N + 63) / 64 * 64;
+  uint8_t* p = (uint8_t*)(((uintptr_t)workspace + 1023) & ~(uintptr_t)1023);
+  __nv_bfloat16* X16 = (__nv_bfloat16*)p; p += ((size_t)M * ldk * 2 + 1023) & ~(size_t)1023;
+  __nv_bfloat16* Y16 = (__nv_bfloat16*)p;
+  lab_to_bf16_kernel<<<(unsigned)((M * ldk + 255) / 256), 256, 0, st>>>(X, X16, M, K, ldk);
+  lab_to_bf16_kernel<<<(unsigned)((M * ldn + 255) / 256), 256, 0, st>>>(dY, Y16, M, N, ldn);
+  return tg::wgrad(Y16, ldn, X16, ldk, dW, K, M, N, K, st);
+}

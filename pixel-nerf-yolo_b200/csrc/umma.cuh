@@ -1,14 +1,17 @@
-// sm_100a building blocks: mbarrier, bulk (TMA) copies, TMEM allocation, tcgen05.mma / ld / st, and the
-// shared-memory operand layout used by every tensor-core tile in this library.
+// sm_100a building blocks of the CTA-pair kernels: mbarrier, tensor-map (TMA) loads, TMEM allocation, tcgen05.mma / ld / st,
+// the shared-memory operand layout used by every tensor-core tile in this library, and the host side of a pair launch
+// (tensor maps, co-resident pair count, cluster launch).
 //
-// Operand layout (both A and B of D = A * B^T are "K-major"): a k-block is [rows x 64] bf16, one row =
+// Operand layout (K-major, the default for both A and B of D = A * B^T): a k-block is [rows x 64] bf16, one row =
 // 128 bytes, rows packed densely, 16-byte chunks XOR-swizzled with (row % 8) -- the canonical
 // SWIZZLE_128B layout that tcgen05 smem descriptors (layout_type = 2, SBO = 1024 B) and TMA share.
 // Every k-block base is 1024-byte aligned.
 #pragma once
+#include <cuda.h>
 #include <cuda_runtime.h>
 #include <cuda_bf16.h>
 #include <stdint.h>
+#include "pnr_common.cuh"
 
 namespace pnr {
 namespace umma {
@@ -64,18 +67,6 @@ __device__ __forceinline__ bool mbar_try_wait(uint32_t bar, uint32_t parity) {
       : "memory");
   return ok != 0;
 }
-// non-blocking probe (never suspends the warp)
-__device__ __forceinline__ bool mbar_test_wait(uint32_t bar, uint32_t parity) {
-  uint32_t ok;
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "mbarrier.test_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-      "selp.b32 %0, 1, 0, p;\n\t}"
-      : "=r"(ok)
-      : "r"(bar), "r"(parity)
-      : "memory");
-  return ok != 0;
-}
 // Bounded wait: a protocol bug traps (launch error) instead of hanging the GPU.  The spin lives out of line so
 // that the (latency-critical, single-thread) MMA issue loop stays small.
 static __device__ __noinline__ void mbar_wait_slow(uint32_t bar, uint32_t parity) {
@@ -99,32 +90,10 @@ __device__ __forceinline__ void fence_proxy_async() {   // generic-proxy smem wr
 __device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
 __device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
 
-// ---- bulk copy global -> shared (TMA engine, 1-D), completion on an mbarrier --------------------------
-__device__ __forceinline__ void bulk_g2s(uint32_t dst_smem, const void* src, uint32_t bytes, uint32_t bar) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(dst_smem),
-               "l"(src), "r"(bytes), "r"(bar)
-               : "memory");
-}
-
-// same, delivered to the same CTA-relative offset (data AND mbarrier signal) of every CTA in cta_mask
-__device__ __forceinline__ void bulk_g2s_multicast(uint32_t dst_smem, const void* src, uint32_t bytes, uint32_t bar,
-                                                   uint16_t cta_mask) {
-  asm volatile(
-      "cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1], %2, [%3], %4;" ::"r"(
-          dst_smem),
-      "l"(src), "r"(bytes), "r"(bar), "h"(cta_mask)
-      : "memory");
-}
-
 // ---- thread-block cluster -------------------------------------------------------------------------
 __device__ __forceinline__ uint32_t cluster_ctarank() {
   uint32_t r;
   asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-  return r;
-}
-__device__ __forceinline__ uint32_t cluster_nctarank() {
-  uint32_t r;
-  asm volatile("mov.u32 %0, %%cluster_nctarank;" : "=r"(r));
   return r;
 }
 __device__ __forceinline__ void cluster_sync_all() {
@@ -132,63 +101,16 @@ __device__ __forceinline__ void cluster_sync_all() {
   asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
 }
 
-// ---- TMEM ---------------------------------------------------------------------------------------
-__device__ __forceinline__ void tmem_alloc(uint32_t dst_smem, uint32_t ncols) {   // one full warp
-  asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(dst_smem), "r"(ncols) : "memory");
-  asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tmem_dealloc(uint32_t taddr, uint32_t ncols) {    // same warp as alloc
-  asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols) : "memory");
-}
-
 // ---- descriptors ------------------------------------------------------------------------------------
 // K-major, SWIZZLE_128B: start>>4 | LBO(1)<<16 | SBO(1024>>4)<<32 | version(1)<<46 | layout(2)<<61
 __device__ __forceinline__ uint64_t smem_desc(uint32_t saddr) {
   return (uint64_t)((saddr >> 4) & 0x3FFFu) | (1ull << 16) | (64ull << 32) | (1ull << 46) | (2ull << 61);
 }
-// kind::f16, A=B=bf16, D=f32, both K-major, M=128, N=n
-__host__ __device__ __forceinline__ uint32_t instr_desc_bf16(int n) {
-  return (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(n >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);
-}
-
-// D[tmem] (+)= A[smem] * B[smem]^T, one K=16 step.  Issued by ONE thread.
-__device__ __forceinline__ void mma_bf16(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc,
-                                         uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}" ::"r"(d_tmem),
-      "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-// all prior tcgen05 ops of this thread complete -> arrive(1) on the mbarrier (implies fence::before_thread_sync)
-__device__ __forceinline__ void mma_commit(uint32_t bar) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
-}
-
-// same, arriving on the barrier at this CTA-relative offset in every CTA of cta_mask
-__device__ __forceinline__ void mma_commit_multicast(uint32_t bar, uint16_t cta_mask) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(bar),
-               "h"(cta_mask)
-               : "memory");
-}
-
-// Same with precomputed descriptors: advancing K by 16 elements (32 B) adds 2 to the start-address field.
-__device__ __forceinline__ void mma_kblock_desc(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc,
-                                                bool accumulate_first) {
-#pragma unroll
-  for (int ks = 0; ks < kBlockK / kUmmaK; ++ks)
-    mma_bf16(d_tmem, a_desc + 2 * ks, b_desc + 2 * ks, idesc, (accumulate_first || ks > 0) ? 1u : 0u);
-}
-
-// A k-block-wide (64) slab: 4 MMAs of K=16.  a_base/b_base are k-block bases in shared memory.
-__device__ __forceinline__ void mma_kblock(uint32_t d_tmem, uint32_t a_base, uint32_t b_base, uint32_t idesc,
-                                           bool accumulate_first) {
-#pragma unroll
-  for (int ks = 0; ks < kBlockK / kUmmaK; ++ks) {
-    mma_bf16(d_tmem, smem_desc(a_base + ks * 32), smem_desc(b_base + ks * 32), idesc,
-             (accumulate_first || ks > 0) ? 1u : 0u);
-  }
+// MN-major SWIZZLE_128B tile made of 64-feature x 64-row boxes (8 KiB each) laid one after the other along MN:
+// LBO = byte distance between 64-element MN atoms = 8 192, SBO = byte distance between 8-row K groups = 1 024
+__device__ __forceinline__ uint64_t smem_desc_mn(uint32_t saddr) {
+  constexpr uint32_t lbo = 8192, sbo = 1024;
+  return (uint64_t)((saddr >> 4) & 0x3FFFu) | ((uint64_t)(lbo >> 4) << 16) | ((uint64_t)(sbo >> 4) << 32) | (1ull << 46) | (2ull << 61);
 }
 
 // ---- TMEM <-> registers (32 lanes x 32-bit, N consecutive columns per thread) ---------------------------
@@ -245,12 +167,8 @@ __device__ __forceinline__ uint32_t mapa_u32(uint32_t smem_addr, uint32_t cta_ra
   asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(smem_addr), "r"(cta_rank));
   return r;
 }
-// arrive (count 1) on an mbarrier anywhere in the cluster; release at cluster scope publishes this thread's prior writes
-__device__ __forceinline__ void mbar_arrive_cluster(uint32_t cluster_addr) {
-  asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(cluster_addr) : "memory");
-}
-// same without the (costly, ~1k cycles) cluster-scope release: only valid after an explicit fence that already made
-// the data visible where it will be consumed (fence.proxy.async on the writer side)
+// arrive (count 1) on an mbarrier anywhere in the cluster, without the (costly, ~1k cycles) cluster-scope release: only valid
+// after an explicit fence that already made the data visible where it will be consumed (fence.proxy.async on the writer side)
 __device__ __forceinline__ void mbar_arrive_cluster_relaxed(uint32_t cluster_addr) {
   asm volatile("mbarrier.arrive.relaxed.cluster.shared::cluster.b64 _, [%0];" ::"r"(cluster_addr) : "memory");
 }
@@ -278,17 +196,8 @@ static __device__ __noinline__ void mbar_wait_cluster_slow(uint32_t bar, uint32_
 __device__ __forceinline__ void mbar_wait_cluster(uint32_t bar, uint32_t parity) {
   if (!mbar_try_wait_cluster(bar, parity)) mbar_wait_cluster_slow(bar, parity);
 }
-__device__ __forceinline__ void fence_proxy_async_all() {   // generic-proxy writes (any space) -> async proxy; expensive (~2k cycles)
-  asm volatile("fence.proxy.async;" ::: "memory");
-}
-__device__ __forceinline__ void fence_proxy_async_cluster() {   // generic-proxy writes to shared memory of any CTA of the cluster
-  asm volatile("fence.proxy.async.shared::cluster;" ::: "memory");
-}
 __device__ __forceinline__ void st_shared_v4(uint32_t addr, uint32_t a, uint32_t b, uint32_t c, uint32_t d) {
   asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(addr), "r"(a), "r"(b), "r"(c), "r"(d) : "memory");
-}
-__device__ __forceinline__ void st_cluster_v4(uint32_t cluster_addr, uint32_t a, uint32_t b, uint32_t c, uint32_t d) {
-  asm volatile("st.shared::cluster.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(cluster_addr), "r"(a), "r"(b), "r"(c), "r"(d) : "memory");
 }
 
 // Asynchronous 16-byte store into a peer CTA's shared memory: the bytes are counted on an mbarrier of the DESTINATION CTA
@@ -311,9 +220,10 @@ __device__ __forceinline__ void tmem_alloc_2sm(uint32_t dst_smem, uint32_t ncols
 __device__ __forceinline__ void tmem_dealloc_2sm(uint32_t taddr, uint32_t ncols) {
   asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols) : "memory");
 }
-// kind::f16, A=B=bf16, D=f32, both K-major, M=256 (pair), N=n
-__host__ __device__ __forceinline__ uint32_t instr_desc_bf16_2sm(int n) {
-  return (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(n >> 3) << 17) | ((uint32_t)(256 >> 4) << 24);
+// kind::f16, A=B=bf16, D=f32, M=256 (pair), N=n; a_mn / b_mn: that operand is MN-major instead of K-major
+__host__ __device__ __forceinline__ uint32_t instr_desc_bf16_2sm(int n, int a_mn = 0, int b_mn = 0) {
+  return (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)a_mn << 15) | ((uint32_t)b_mn << 16) | ((uint32_t)(n >> 3) << 17) |
+         ((uint32_t)(256 >> 4) << 24);
 }
 __device__ __forceinline__ void mma_bf16_2sm(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc,
                                              uint32_t accumulate) {
@@ -359,6 +269,70 @@ __device__ __forceinline__ void transpose8x8(uint32_t (&a)[8], int lane) {
       if (up) a[k] = recv; else a[k | d] = recv;
     }
   }
+}
+
+// ---- host side of a pair launch ---------------------------------------------------------------------------------------
+typedef CUresult (*EncodeFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
+                             const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
+                             CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
+// 2-D bf16 tensor map over a row-major [rows x cols] matrix with leading dimension ld (elements); box = box_c x box_r
+inline int make_map(CUtensorMap* m, const void* base, long long rows, long long cols, long long ld, int box_c, int box_r, bool swizzle) {
+  static EncodeFn enc = nullptr;
+  if (!enc) {
+    void* fn = nullptr;
+    cudaDriverEntryPointQueryResult qres;
+    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres) == cudaSuccess) enc = (EncodeFn)fn;
+  }
+  PNR_REQUIRE(enc, PNR_ERR_CUDA, "cuTensorMapEncodeTiled entry point not found");
+  PNR_REQUIRE(((uintptr_t)base & 15) == 0 && (ld * 2) % 16 == 0, PNR_ERR_ARG, "tensor map: base / row pitch must be 16-byte aligned");
+  cuuint64_t gdim[2] = {(cuuint64_t)cols, (cuuint64_t)rows};
+  cuuint64_t gstride[1] = {(cuuint64_t)ld * 2};
+  cuuint32_t box[2] = {(cuuint32_t)box_c, (cuuint32_t)box_r};
+  cuuint32_t estr[2] = {1, 1};
+  CUresult r = enc(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(base), gdim, gstride, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                   swizzle ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  PNR_REQUIRE(r == CUDA_SUCCESS, PNR_ERR_CUDA, "cuTensorMapEncodeTiled failed (%d)", (int)r);
+  return PNR_OK;
+}
+
+// launch configuration of n_pairs clusters of 2 CTAs; attr must outlive the returned configuration
+inline cudaLaunchConfig_t pair_config(cudaLaunchAttribute* attr, int n_pairs, int threads, int smem_bytes, cudaStream_t st) {
+  attr->id = cudaLaunchAttributeClusterDimension;
+  attr->val.clusterDim.x = 2; attr->val.clusterDim.y = 1; attr->val.clusterDim.z = 1;
+  cudaLaunchConfig_t cfg = {};
+  cfg.gridDim = dim3(2 * n_pairs); cfg.blockDim = dim3(threads); cfg.dynamicSmemBytes = smem_bytes; cfg.stream = st;
+  cfg.attrs = attr; cfg.numAttrs = 1;
+  return cfg;
+}
+
+// Sets kern's dynamic shared-memory limit to smem_bytes and returns in *n_pairs the CTA pairs of kern that can be resident at
+// once: cudaOccupancyMaxActiveClusters, at most SMs / 2.  The pair kernels are persistent with a static round-robin over
+// their units, so they must not be launched with more pairs than that.
+template <typename Kern>
+int pair_capacity(Kern kern, int threads, int smem_bytes, int* n_pairs) {
+  cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes);
+  PNR_REQUIRE(e == cudaSuccess, PNR_ERR_CUDA, "cudaFuncSetAttribute: %s", cudaGetErrorString(e));
+  int dev = 0, sms = 148;
+  cudaGetDevice(&dev);
+  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+  int pairs = sms / 2, mc = 0;
+  cudaLaunchAttribute attr;
+  const cudaLaunchConfig_t cfg = pair_config(&attr, pairs, threads, smem_bytes, 0);
+  if (cudaOccupancyMaxActiveClusters(&mc, kern, &cfg) == cudaSuccess && mc > 0 && mc < pairs) pairs = mc;
+  *n_pairs = pairs;
+  return PNR_OK;
+}
+
+// Launches 2 x n_pairs CTAs of kern (after pair_capacity) as clusters of 2; `name` names the kernel in error messages.
+template <typename Kern, typename... Args>
+int launch_pairs(Kern kern, int n_pairs, int threads, int smem_bytes, cudaStream_t st, const char* name, const Args&... args) {
+  cudaLaunchAttribute attr;
+  const cudaLaunchConfig_t cfg = pair_config(&attr, n_pairs, threads, smem_bytes, st);
+  const cudaError_t e = cudaLaunchKernelEx(&cfg, kern, args...);
+  PNR_REQUIRE(e == cudaSuccess, PNR_ERR_CUDA, "%s launch: %s", name, cudaGetErrorString(e));
+  PNR_CHECK_LAUNCH(name);
+  return PNR_OK;
 }
 
 }  // namespace umma

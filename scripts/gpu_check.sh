@@ -6,7 +6,6 @@ cd "$(dirname "$0")/.."
 nvidia-smi --query-gpu=name,clocks.max.sm,memory.total --format=csv > gpurun_out/gpu.txt 2>&1
 run() { name=$1; shift; timeout 900 python -m pytest tests -m gpu -q --timeout 600 -k "$@" > gpurun_out/test_$name.log 2>&1; echo "$name exit $?" >> gpurun_out/summary.txt; tail -3 gpurun_out/test_$name.log >> gpurun_out/summary.txt; }
 : > gpurun_out/summary.txt
-run umma "umma_building"
 run raytile "sample_coarse or composite or resample"
 run ops "positional or index_operator or resnetfc_operator or gather_encode"
 run field_fp32 "field and fp32"

@@ -41,27 +41,6 @@ def _renderer(**kw):
     return NeRFRenderer.from_conf(ConfigTree.from_dict(conf)).eval().cuda()
 
 
-# ------------------------------------------------------------------------------------------------ tcgen05
-@pytest.mark.parametrize("N,K", [(64, 64), (64, 512), (32, 128), (16, 512), (48, 256)])
-def test_umma_building_blocks(lib, N, K):
-    """bulk copy + swizzled operands + smem/instruction descriptors + TMEM accumulate + tcgen05.ld."""
-    from pixel_nerf_yolo_b200 import _lib
-    g = torch.Generator().manual_seed(N * 1000 + K)
-    a = torch.randn(128, K, generator=g)
-    b = torch.randn(N, K, generator=g)
-    ref = a.bfloat16().float() @ b.bfloat16().float().t()
-    ad, bd = a.cuda(), b.cuda()
-    d = torch.full((128, N), float("nan"), device="cuda")
-    ws = torch.empty(K // 64 * 16384 + 1024, dtype=torch.uint8, device="cuda")
-    off = (-ws.data_ptr()) % 1024
-    rc = lib.pnr_umma_selftest(ad.data_ptr(), bd.data_ptr(), d.data_ptr(), ws.data_ptr() + off, N, K,
-                               _lib.stream_ptr(torch.device("cuda", 0)))
-    _lib.check(rc, "pnr_umma_selftest")
-    torch.cuda.synchronize()
-    np.testing.assert_allclose(d.cpu().numpy(), ref.numpy(), atol=2e-3 * K ** 0.5, rtol=1e-3)
-    assert (d.cpu() - ref).abs().max() < 1e-3 * K ** 0.5
-
-
 # ------------------------------------------------------------------------------------------------ ray tile
 @pytest.mark.parametrize("Kc,lindisp", [(64, False), (128, False), (256, False), (96, False), (64, True)])
 def test_sample_coarse_bit_exact(lib, Kc, lindisp):
