@@ -23,6 +23,7 @@
 // Hand-offs (L = leader CTA 0; "mc" = tcgen05.commit.cta_group::2 multicast to both CTAs):
 //   W_FULL[s]  @L    : leader producer's expect_tx(32 KiB) + TMA bytes of both CTAs      W_EMPTY[s] @both : mc
 //   IN_READY   @L    : gather warps of both CTAs (remote arrive)                         IN_FREE    @both : mc
+//   ZF_FREE    @both : mc, lin_in has read the z-feature tile (the latent tile stays busy until the last lin_z)
 //   RDY[kc]    @L    : chunk kc (produced by CTA kc % 2) is in place in both CTAs: the producing warps' arrivals, plus
 //                      the st.async bytes landing in L (odd kc) or the relay's arrival for bytes that landed in CTA 1 (even kc)
 //   LAND[mt]   @CTA1 : st.async bytes of chunk 2*mt from L have landed (+ L's warps' remote arrive.expect_tx)
@@ -186,6 +187,7 @@ enum {
   B_RDY = B_H_FULL + kMaxMT, B_X_FREE = B_RDY + 2 * kMaxMT,  // one per feature tile: the view-mean epilogue has read x tile mt out of TMEM
   B_LAND = B_X_FREE + kMaxMT,                                    // non-leader CTA only: remote rows of chunk 2*i have landed (st.async bytes)
   B_OUT_FREE = B_LAND + kMaxMT,                 // leader: the output epilogue has read lin_out's result out of the h region
+  B_ZF_FREE,                                    // both: lin_in has read the z-feature tile
   B_COUNT
 };
 static_assert(B_COUNT <= 30, "barrier parity bits live in one 32-bit word");
@@ -201,6 +203,7 @@ __device__ inline ProgEntry make_prog(const Sched& sc, int s, uint32_t sbase) {
     case MAT_LIN_IN:
       b_addr = sbase + Smem::zf; dcol = g.t * 128; acc = 0;
       if (g.t == 0) wait_id = B_IN_READY + 1;
+      if (g.t == MT - 1) c1 = B_ZF_FREE + 1;
       break;
     case MAT_LINZ: {
       const ZPos z = z_position<MT>(sc.KBz, g.t);
@@ -209,7 +212,9 @@ __device__ inline ProgEntry make_prog(const Sched& sc, int s, uint32_t sbase) {
       b_addr = sbase + Smem::lat + z.kbi * kOperandKB; dcol = z.mt * 128;
       if (streaming && pass_first && !(g.blk == 0 && z.pass == 0)) wait_id = B_IN_READY + 1;
       if (pass_last && (streaming || g.blk == sc.n_linz - 1)) c1 = B_IN_FREE + 1;
-      if (last && g.blk == 0) { c2 = B_X_FULL + 1; if (MT > 1) c3 = B_X_FULL + 2; }
+      // x tile 0 is complete after the last pass's tile-0 k-blocks: at MT = 2 its epilogue overlaps tile 1's lin_z stages
+      if (g.blk == 0 && z.pass == z_passes(sc) - 1 && z.mt == 0 && z.kbi == z.kp - 1) c2 = B_X_FULL + 1;
+      if (last && g.blk == 0 && MT > 1) c3 = B_X_FULL + 2;
     } break;
     case MAT_FC0:
     case MAT_FC1: {
@@ -331,6 +336,7 @@ field_pair_kernel(const pnr_scene sc, const pnr_points q, const __grid_constant_
     for (int i = 0; i < 2 * MT; ++i) mbar_init(bar(B_RDY + i), kEpiWarps + ((i & 1) == 0 ? 1 : 0));
     for (int i = 0; i < MT; ++i) mbar_init(bar(B_LAND + i), kEpiWarps);
     mbar_init(bar(B_OUT_FREE), 2);
+    mbar_init(bar(B_ZF_FREE), 1);
     for (int i = 0; i < MT; ++i) mbar_init(bar(B_X_FREE + i), 2 * kEpiWarps);
     fence_barrier_init();
   }
@@ -729,12 +735,15 @@ field_pair_kernel(const pnr_scene sc, const pnr_points q, const __grid_constant_
           float wa[4], wb[4];
           load_col(0, ra, wa);                       // the first two columns' loads go out BEFORE the operand buffers are free:
           load_col(1, rb, wb);                       // they only fill registers
-          mbar_wait_cluster(bar(B_IN_FREE), par_free);
-          par_free ^= 1;
-          if (fill == 0) {                           // the sin/cos work runs under the first loads' latency
+          if (fill == 0) {
+            // the z-feature tile is free once the previous tile's lin_in has read it, long before the latent tile is: the
+            // sin/cos work runs under the first loads' latency and off the path from IN_FREE to IN_READY
+            mbar_wait_cluster(bar(B_ZF_FREE), (~it) & 1);   // one phase per tile, the first wait passes at once
 #pragma unroll 1
             for (int i = 0; i < 16; ++i) zfeat_col(i);
           }
+          mbar_wait_cluster(bar(B_IN_FREE), par_free);
+          par_free ^= 1;
 #pragma unroll 1
           for (int i = 0; i < 16; i += 2) {
             blend_col(i, ra, wa);
