@@ -76,6 +76,19 @@ typedef struct pnr_scene {
  * accumulation in TMEM, cta_group::2 GEMMs for the forward layers, the input gradients and the weight gradients
  * (csrc/train_umma.cu).  Gradients within ~2e-2 of autograd (bf16 operand rounding).  C a multiple of 64. */
 #define PNR_SCENE_TRAIN_BF16 16
+/* z-feature layout: the non-latent part of each MLP input row, as PixelNeRFNet's switches shape it (models.py:16-90,
+ * 183-209).  All bits clear is the layout of every shipped conf: [PE(R x) (3 + 6 num_freqs), R d (3)].  In general, with
+ * x_rot = R x and x_cam = R x + t of the source view:
+ *   u  = x_rot (x_cam with CAM_COORDS), or the one value -u_z with Z_ONLY;  u ++= R d with CODE_VIEWDIRS (unless NO_VIEWDIRS);
+ *   zf = PE(u) = [u (unless NO_CODE_INPUT), sin(f_0 u), cos(f_0 u), sin(f_1 u), ...], or u itself with NO_CODE;
+ *   zf ++= R d unless NO_VIEWDIRS or CODE_VIEWDIRS.
+ * Its width is pnr_zfeat_width(flags, num_freqs); every field, gather and training entry point requires d_in to equal it. */
+#define PNR_SCENE_ZF_NO_VIEWDIRS 32      /* use_viewdirs = False                                                       */
+#define PNR_SCENE_ZF_CODE_VIEWDIRS 64    /* use_code_viewdirs = True: R d goes through the positional encoding          */
+#define PNR_SCENE_ZF_CAM_COORDS 128      /* normalize_z = False: camera coordinates R x + t instead of R x             */
+#define PNR_SCENE_ZF_Z_ONLY 256          /* use_xyz = False: the single coordinate -z                                  */
+#define PNR_SCENE_ZF_NO_CODE 512         /* use_code = False: no positional encoding                                   */
+#define PNR_SCENE_ZF_NO_CODE_INPUT 1024  /* code.include_input = False: the encoding drops its raw input columns        */
 
 /* Where the query points of a field evaluation come from. */
 typedef struct pnr_points {
@@ -173,10 +186,15 @@ int pnr_rgb_loss(const float* rgb, const float* gt, float* loss, float* d_rgb, l
 
 /* ---- project + 4-tap gather + positional encoding, stand-alone ---------------------------------- */
 /* models.py:168-230 + encoder.py:79-108 + code.py:30-42.  For every (object, view, point) row
- * r = (s*NS + v)*P + p writes latent_out[r, 0:C] (bf16 if out_fp32=0 else fp32) and zfeat_out[r, 0:42]
- * fp32 = [PE(R x) (39), R d (3)].  Either output may be NULL. */
+ * r = (s*NS + v)*P + p writes latent_out[r, 0:C] (bf16 if out_fp32=0 else fp32) and zfeat_out[r, 0:W] fp32, the z-feature in
+ * the layout of the scene's PNR_SCENE_ZF_* bits, W = pnr_zfeat_width(scene->flags, num_freqs) (default: [PE(R x) (39),
+ * R d (3)] at 6 frequencies).  Either output may be NULL. */
 int pnr_gather_encode(const pnr_scene* scene, const pnr_points* pts, void* latent_out, float* zfeat_out,
                       int out_fp32, int num_freqs, float freq_factor, void* stream);
+
+/* Width of the z-feature (PixelNeRFNet's d_in) that the PNR_SCENE_ZF_* bits of `flags` give at num_freqs frequencies
+ * (num_freqs is ignored with PNR_SCENE_ZF_NO_CODE).  Default layout: 6 * num_freqs + 6.  Host function, no device work. */
+int pnr_zfeat_width(int flags, int num_freqs);
 
 /* PositionalEncoding.forward as a stand-alone operator (src/model/code.py:30-42):
  * x (n, d) -> out (n, d * (2*num_freqs + include_input)) = [x, sin(f0 x), cos(f0 x), sin(f1 x), ...]. */

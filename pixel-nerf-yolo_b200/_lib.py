@@ -22,6 +22,13 @@ SCENE_RAW_OUTPUT = 2
 SCENE_PROJECTED = 4
 SCENE_TRAIN_TF32 = 8
 SCENE_TRAIN_BF16 = 16
+# z-feature layout bits (PNR_SCENE_ZF_*): the PixelNeRFNet switches that shape the non-latent part of the MLP input
+SCENE_ZF_NO_VIEWDIRS = 32
+SCENE_ZF_CODE_VIEWDIRS = 64
+SCENE_ZF_CAM_COORDS = 128
+SCENE_ZF_Z_ONLY = 256
+SCENE_ZF_NO_CODE = 512
+SCENE_ZF_NO_CODE_INPUT = 1024
 COMBINE_TYPES = {"average": 0, "max": 1}     # pnr_mlp_params.combine_type
 
 # every symbol include/pixelnerf_b200.h declares
@@ -33,7 +40,7 @@ EXPORTS = [
     "pnr_field_tape_bytes", "pnr_field_forward_train", "pnr_field_backward_workspace_bytes", "pnr_field_backward",
     "pnr_composite_backward", "pnr_sample_fine_depth_backward", "pnr_pyramid_pack", "pnr_gen_rays", "pnr_yolo_reduce", "pnr_image_output", "pnr_rgb_loss",
     "pnr_mlp_pack_projected_bytes", "pnr_mlp_pack_projected", "pnr_project_features",
-    "pnr_render_workspace_bytes", "pnr_render_forward",
+    "pnr_render_workspace_bytes", "pnr_render_forward", "pnr_zfeat_width",
 ]
 # test hooks of the training GEMMs (csrc/pnr_lab.h, internal); not part of the product ABI
 LAB_EXPORTS = ["pnr_lab_gemm_workspace_bytes", "pnr_lab_rowgemm", "pnr_lab_wgrad"]
@@ -141,6 +148,8 @@ def load() -> C.CDLL:
     lib.pnr_resnetfc_workspace_bytes.argtypes = [C.POINTER(MlpParams), C.c_longlong]
     lib.pnr_resnetfc_workspace_bytes.restype = C.c_size_t
     lib.pnr_resnetfc_forward.argtypes = [C.POINTER(MlpParams), vp, C.c_longlong, i32, i32, vp, vp, C.c_size_t, vp]
+    lib.pnr_zfeat_width.argtypes = [i32, i32]
+    lib.pnr_zfeat_width.restype = i32
     lib.pnr_positional_encoding.argtypes = [vp, vp, C.c_longlong, i32, i32, f32, i32, vp]
     lib.pnr_index_features.argtypes = [C.POINTER(Scene), vp, i32, i32, vp, vp]
     lib.pnr_lab_gemm_workspace_bytes.argtypes = [C.c_longlong, i32, i32]

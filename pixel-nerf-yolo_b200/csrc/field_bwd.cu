@@ -559,7 +559,7 @@ lin_out_bwd_kernel(const T* __restrict__ x, const float* __restrict__ W, const f
 }
 
 // Backward of projection + bilinear gather + positional encoding for one (object, view, point) row per warp.
-//   dlat (rows, C), dzf (rows, d_in)  ->  d_feat (fp32 channels-last maps, atomics; may be null),
+//   dlat (rows, C), dzf (rows, d_in = z-feature width)  ->  d_feat (fp32 channels-last maps, atomics; may be null),
 //   d_xyz (SB*P, 3) (mode 0) or d_z (SB*B*K) (mode 1: x = o + z d  =>  dz = dx . d), atomics; may be null.
 __global__ void __launch_bounds__(256)
 gather_encode_bwd_kernel(pnr_scene sc, pnr_points q, const float* __restrict__ dlat, const float* __restrict__ dzf,
@@ -569,7 +569,7 @@ gather_encode_bwd_kernel(pnr_scene sc, pnr_points q, const float* __restrict__ d
   const long long warp = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const long long n_warps = ((long long)gridDim.x * blockDim.x) >> 5;
   const int NS = sc.NS, P = q.P, C = sc.C;
-  const int d_in = 6 * num_freqs + 6;
+  const ZfLayout L = zf_layout(sc.flags, num_freqs);
   const bool want_x = d_xyz || d_z;
   for (long long row = warp; row < n_rows; row += n_warps) {
     const int view = (int)(row / P);
@@ -612,18 +612,24 @@ gather_encode_bwd_kernel(pnr_scene sc, pnr_points q, const float* __restrict__ d
       }
     }
     if (!want_x) continue;
-    // positional encoding: element j of the z-feature row depends on coordinate d = (j - 3) % 3 of R x
+    // z-feature: column j < n_code depends on encoder input i of u (zfeat_value).  Inputs i < n_xyz are coordinates of R x
+    // (R x + t with CAM_COORDS: same derivative), or -z alone with Z_ONLY; the view-direction values carry no gradient to
+    // the points.
     float gx[3] = {0.f, 0.f, 0.f};
-    const int n_pe = 3 + 6 * num_freqs;
-    for (int j = lane; j < n_pe && j < d_in; j += 32) {
-      const float gj = dzf[row * d_in + j];
-      if (j < 3) { gx[j] += gj; continue; }
-      const int qq = j - 3, k = qq / 6, r = qq - k * 6, d = r % 3;
-      const float xv = d == 0 ? pr.xr : (d == 1 ? pr.yr : pr.zr);
-      const float f = freq_factor * (float)(1 << k);
-      const float ph = r >= 3 ? 1.57079637050628662109375f : 0.0f;
-      const float dv = gj * f * cosf(fmaf(xv, f, ph));           // d/dx sin(f x + ph)
-      gx[d] += dv;
+    for (int j = lane; j < L.n_code; j += 32) {
+      const float gj = dzf[row * L.width + j];
+      int i = j;
+      float dv = gj;
+      if (j >= L.n_raw) {
+        const ZfCode c = zf_code(L, j);
+        const float f = freq_factor * (float)(1 << c.k);
+        const float ph = c.cos ? 1.57079637050628662109375f : 0.0f;
+        i = c.i;
+        dv = gj * f * cosf(fmaf(zf_input(pr, L, i), f, ph));    // d/du sin(f u + ph)
+      }
+      if (i >= L.n_xyz) continue;
+      if (L.n_xyz == 1) gx[2] -= dv;                             // u = -z
+      else gx[i] += dv;
     }
 #pragma unroll
     for (int d = 16; d > 0; d >>= 1) {
@@ -635,7 +641,7 @@ gather_encode_bwd_kernel(pnr_scene sc, pnr_points q, const float* __restrict__ d
     }
     if (lane == 0) {
       const float* M = sc.poses + (size_t)view * 12;
-      const float xc = pr.xr + M[3], yc = pr.yr + M[7], zc = pr.zr + M[11];
+      const float xc = pr.xc, yc = pr.yc, zc = pr.zc;
       const float fxv = sc.focal[view * 2 + 0], fyv = sc.focal[view * 2 + 1];
       // ix = u * (lat_scale_x / image_w) * 0.5 * (Wl - 1),  u = -xc / zc * fx + cx
       const float du = gix * (sc.lat_scale_x / sc.image_w) * 0.5f * (float)(sc.Wl - 1);
@@ -710,7 +716,9 @@ static int check_train(const pnr_scene* sc, const pnr_points* q, const pnr_mlp_p
   }
   PNR_REQUIRE(sc->C % 4 == 0, PNR_ERR_UNSUPPORTED, "%s: C=%d must be a multiple of 4", who, sc->C);
   PNR_REQUIRE(mp->d_latent == sc->C, PNR_ERR_ARG, "%s: d_latent=%d but maps have C=%d", who, mp->d_latent, sc->C);
-  PNR_REQUIRE(mp->d_in == 6 * num_freqs + 6, PNR_ERR_ARG, "%s: d_in/num_freqs mismatch", who);
+  PNR_REQUIRE(mp->d_in == pnr_zfeat_width(sc->flags, num_freqs), PNR_ERR_ARG,
+              "%s: d_in=%d but the z-feature layout of the scene flags has width %d at num_freqs=%d", who, mp->d_in,
+              pnr_zfeat_width(sc->flags, num_freqs), num_freqs);
   PNR_REQUIRE(mp->n_blocks >= 1 && mp->n_blocks <= 8, PNR_ERR_UNSUPPORTED, "%s: n_blocks=%d", who, mp->n_blocks);
   PNR_REQUIRE(mp->combine_layer >= 1 && mp->combine_layer <= mp->n_blocks, PNR_ERR_ARG, "%s: combine_layer=%d", who, mp->combine_layer);
   PNR_REQUIRE(mp->combine_layer < mp->n_blocks || sc->NS == 1, PNR_ERR_UNSUPPORTED, "%s: combine_layer >= n_blocks needs NS=1", who);

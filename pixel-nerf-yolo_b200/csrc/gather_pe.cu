@@ -49,8 +49,8 @@ gather_encode_kernel(pnr_scene sc, pnr_points q, void* __restrict__ latent_out, 
     fetch_point(q, (long long)s * P + p, px, py, pz, vx, vy, vz);
     const Projection pr = project_point(sc, view, px, py, pz, vx, vy, vz);
     if (zfeat_out) {
-      for (int j = lane; j < 3 + 6 * num_freqs + 3; j += 32)
-        zfeat_out[row * (3 + 6 * num_freqs + 3) + j] = zfeat_value(pr, j, num_freqs, freq_factor);
+      const ZfLayout L = zf_layout(sc.flags, num_freqs);
+      for (int j = lane; j < L.width; j += 32) zfeat_out[row * L.width + j] = zfeat_value<false>(pr, L, j, num_freqs, freq_factor);
     }
     if (latent_out) {
       const Taps t = make_taps(pr.ix, pr.iy, sc.Hl, sc.Wl, C);
@@ -204,6 +204,8 @@ extern "C" int pnr_gather_encode(const pnr_scene* scene, const pnr_points* pts, 
   PNR_CHECK_LAUNCH("gather_encode_kernel");
   return PNR_OK;
 }
+
+extern "C" int pnr_zfeat_width(int flags, int num_freqs) { return zf_layout(flags, num_freqs).width; }
 
 extern "C" int pnr_positional_encoding(const float* x, float* out, long long n, int d, int num_freqs,
                                        float freq_factor, int include_input, void* stream) {

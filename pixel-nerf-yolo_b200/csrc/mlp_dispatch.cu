@@ -99,7 +99,9 @@ int field_forward_umma(const pnr_scene* sc, const pnr_points* q, const pnr_mlp_p
   } else {
     PNR_REQUIRE(sc->C == mp->d_latent, PNR_ERR_ARG, "field_forward_umma: feature maps have %d channels, the MLP expects %d", sc->C, mp->d_latent);
   }
-  PNR_REQUIRE(mp->d_in == 6 * num_freqs + 6, PNR_ERR_ARG, "field_forward_umma: d_in/num_freqs mismatch");
+  PNR_REQUIRE(mp->d_in == pnr_zfeat_width(sc->flags, num_freqs), PNR_ERR_ARG,
+              "field_forward_umma: d_in=%d but the z-feature layout of the scene flags has width %d at num_freqs=%d", mp->d_in,
+              pnr_zfeat_width(sc->flags, num_freqs), num_freqs);
   PNR_REQUIRE(sc->NS >= 1 && sc->NS <= 8 && sc->NS != 7, PNR_ERR_UNSUPPORTED, "field_forward_umma: NS=%d source views", sc->NS);
   PNR_REQUIRE(mp->combine_layer < mp->n_blocks || sc->NS == 1, PNR_ERR_UNSUPPORTED,
               "field_forward_umma: combine_layer >= n_blocks never pools the views; only valid with one source view");

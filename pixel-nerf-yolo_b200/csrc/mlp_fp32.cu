@@ -187,7 +187,9 @@ int field_forward_fp32(const pnr_scene* sc, const pnr_points* q, const pnr_mlp_p
   int rc = check_mlp(mp, sc->NS, "field_forward_fp32");
   if (rc) return rc;
   const int H = mp->d_hidden, d_in = mp->d_in, C = sc->C;
-  PNR_REQUIRE(d_in == 6 * num_freqs + 6, PNR_ERR_ARG, "field_forward_fp32: d_in=%d does not match num_freqs=%d", d_in, num_freqs);
+  PNR_REQUIRE(d_in == pnr_zfeat_width(sc->flags, num_freqs), PNR_ERR_ARG,
+              "field_forward_fp32: d_in=%d but the z-feature layout of the scene flags has width %d at num_freqs=%d", d_in,
+              pnr_zfeat_width(sc->flags, num_freqs), num_freqs);
   PNR_REQUIRE(mp->d_latent == C, PNR_ERR_ARG, "field_forward_fp32: d_latent=%d but feature maps have C=%d", mp->d_latent, C);
   PNR_REQUIRE(ws && ws_bytes >= field_workspace_fp32(sc, q, d_in, H), PNR_ERR_ARG, "field_forward_fp32: workspace too small");
   const long long rows = (long long)sc->SB * sc->NS * q->P, pts = (long long)sc->SB * q->P;

@@ -301,8 +301,10 @@ __device__ __forceinline__ void store_transposed(uint32_t base, const uint32_t* 
 // waiting for their remote rows to be performed (14.5 % of all warp-stall samples of a synchronous exchange).  Rows landing
 // in the leader are counted directly on the chunk barrier the MMA warp waits on; rows landing in the non-leader are counted
 // on its B_LAND barrier, and its otherwise idle warp 1 relays that to the leader.
-// VMAX: combine_type "max".  MT: 256-feature tiles of the padded hidden width (1 or 2, see Sched).
-template <int NS, bool VMAX, int MT>
+// VMAX: combine_type "max".  MT: 256-feature tiles of the padded hidden width (1 or 2, see Sched).  ZF: the scene's
+// PNR_SCENE_ZF_* bits shape the z-feature; without it the layout is the default one as a compile-time constant (reading the
+// layout at run time costs the gather warps 16 bytes of stack frame and spills at flags = 0).
+template <int NS, bool VMAX, int MT, bool ZF>
 __global__ void __launch_bounds__(kThreads, 1)
 field_pair_kernel(const pnr_scene sc, const pnr_points q, const __grid_constant__ CUtensorMap wmap,
                   const float* __restrict__ bias_x, const float* __restrict__ bias_h,
@@ -650,7 +652,7 @@ field_pair_kernel(const pnr_scene sc, const pnr_points q, const __grid_constant_
         const int c = gather_col(gw, lane & 15);
         const int v = c / PP, p = c - v * PP;
         const bool valid = (tile < n_tiles) && (v < NS) && (p0 + p < q.P);
-        pr.xr = pr.yr = pr.zr = pr.dx = pr.dy = pr.dz = pr.ix = pr.iy = 0.f;
+        pr.xr = pr.yr = pr.zr = pr.xc = pr.yc = pr.zc = pr.dx = pr.dy = pr.dz = pr.ix = pr.iy = 0.f;
 #pragma unroll
         for (int k = 0; k < 4; ++k) { tp.off[k] = -1; tp.w[k] = 0.f; }
         if (valid) {
@@ -667,13 +669,18 @@ field_pair_kernel(const pnr_scene sc, const pnr_points q, const __grid_constant_
         pi.xr = __shfl_sync(0xffffffffu, pr.xr, i); pi.yr = __shfl_sync(0xffffffffu, pr.yr, i);
         pi.zr = __shfl_sync(0xffffffffu, pr.zr, i); pi.dx = __shfl_sync(0xffffffffu, pr.dx, i);
         pi.dy = __shfl_sync(0xffffffffu, pr.dy, i); pi.dz = __shfl_sync(0xffffffffu, pr.dz, i);
+        if constexpr (ZF) {
+          pi.xc = __shfl_sync(0xffffffffu, pr.xc, i); pi.yc = __shfl_sync(0xffffffffu, pr.yc, i);
+          pi.zc = __shfl_sync(0xffffffffu, pr.zc, i);
+        }
         pi.ix = pi.iy = 0.f;
         const bool vi = __shfl_sync(0xffffffffu, vbase, i) >= 0;
-        const int j0 = lane * 2, d_in = 6 * num_freqs + 6;
+        const int j0 = lane * 2;
+        const ZfLayout zl = zf_layout(ZF ? sc.flags : 0, num_freqs);
         float a = 0.f, b = 0.f;
         if (vi) {
-          if (j0 < d_in) a = zfeat_value_fast(pi, j0, num_freqs, freq_factor);
-          if (j0 + 1 < d_in) b = zfeat_value_fast(pi, j0 + 1, num_freqs, freq_factor);
+          if (j0 < zl.width) a = zfeat_value<true>(pi, zl, j0, num_freqs, freq_factor);
+          if (j0 + 1 < zl.width) b = zfeat_value<true>(pi, zl, j0 + 1, num_freqs, freq_factor);
         }
         *reinterpret_cast<__nv_bfloat162*>(smem + Smem::zf + swz_offset(gather_col(gw, i), j0)) = __floats2bfloat162_rn(a, b);
       };
@@ -820,16 +827,20 @@ int field_forward_pair(const pnr_scene* sc, const pnr_points* q, const pnr_mlp_p
   const bool vmax = mp->combine_type == PNR_COMBINE_MAX && sc->NS > 1;
   const int n_groups = ((n_tiles + 1) / 2 + G - 1) / G;  // super groups
   const bool mt1 = hidden_tiles(mp) == 1;
-  decltype(&pair::field_pair_kernel<1, false, 1>) kern = nullptr;
+  const bool zf = (sc->flags & kZfFlags) != 0;
+  decltype(&pair::field_pair_kernel<1, false, 1, false>) kern = nullptr;
+#define PNR_PAIR_KERNEL_ZF(NSV, ZFV)                                                                                   \
+  kern = mt1 ? (vmax ? pair::field_pair_kernel<NSV, (NSV > 1), 1, ZFV> : pair::field_pair_kernel<NSV, false, 1, ZFV>)  \
+             : (vmax ? pair::field_pair_kernel<NSV, (NSV > 1), 2, ZFV> : pair::field_pair_kernel<NSV, false, 2, ZFV>);
 #define PNR_PAIR_KERNEL(NSV)                                                                                     \
   case NSV:                                                                                                      \
-    kern = mt1 ? (vmax ? pair::field_pair_kernel<NSV, (NSV > 1), 1> : pair::field_pair_kernel<NSV, false, 1>)     \
-               : (vmax ? pair::field_pair_kernel<NSV, (NSV > 1), 2> : pair::field_pair_kernel<NSV, false, 2>);    \
+    if (zf) { PNR_PAIR_KERNEL_ZF(NSV, true) } else { PNR_PAIR_KERNEL_ZF(NSV, false) }                            \
     break;
   switch (sc->NS) {
     PNR_PAIR_KERNEL(1) PNR_PAIR_KERNEL(2) PNR_PAIR_KERNEL(3) PNR_PAIR_KERNEL(4) PNR_PAIR_KERNEL(5) PNR_PAIR_KERNEL(6) PNR_PAIR_KERNEL(8)
     default: PNR_REQUIRE(false, PNR_ERR_UNSUPPORTED, "field_forward_pair: NS=%d", sc->NS);
   }
+#undef PNR_PAIR_KERNEL_ZF
 #undef PNR_PAIR_KERNEL
   int max_pairs;
   if ((rc = pair_capacity(kern, pair::kThreads, pair::Smem::total, &max_pairs))) return rc;

@@ -32,7 +32,6 @@ void reset_launch_count();
     ::pnr::count_launch();                                                            \
   } while (0)
 
-constexpr int kZFeat = 42;      // 39 positional-encoding values + 3 rotated view-direction values
 constexpr int kHidden = 512;    // widest ResnetFC d_hidden the library runs (that of every shipped conf, conf/default*.conf)
 // ResnetFC hidden widths the field and training paths run: the multiples of 64 up to kHidden
 __host__ __device__ inline bool hidden_width_supported(int d_hidden) {
@@ -43,6 +42,7 @@ __host__ __device__ inline bool hidden_width_supported(int d_hidden) {
 // Per-point camera-space quantities for one source view (models.py:168-230, encoder.py:94-98).
 struct Projection {
   float xr, yr, zr;   // R x            (positional-encoding input, normalize_z=True)
+  float xc, yc, zc;   // R x + t        (camera coordinates, normalize_z=False)
   float dx, dy, dz;   // R d            (view direction in the source view frame)
   float ix, iy;       // feature-map pixel coordinates (align_corners=True un-normalised)
 };
@@ -58,7 +58,8 @@ __device__ __forceinline__ Projection project_point(const pnr_scene& sc, int row
   o.dx = M[0] * vx + M[1] * vy + M[2] * vz;
   o.dy = M[4] * vx + M[5] * vy + M[6] * vz;
   o.dz = M[8] * vx + M[9] * vy + M[10] * vz;
-  const float xc = o.xr + M[3], yc = o.yr + M[7], zc = o.zr + M[11];
+  o.xc = o.xr + M[3]; o.yc = o.yr + M[7]; o.zc = o.zr + M[11];
+  const float xc = o.xc, yc = o.yc, zc = o.zc;
   // uv = -xy / z * focal + c                      models.py:220-230
   float u = __fdiv_rn(-xc, zc) * sc.focal[row * 2 + 0] + sc.center[row * 2 + 0];
   float v = __fdiv_rn(-yc, zc) * sc.focal[row * 2 + 1] + sc.center[row * 2 + 1];
@@ -99,40 +100,70 @@ __device__ __forceinline__ Taps make_taps(float ix, float iy, int Hl, int Wl, in
   return t;
 }
 
-// z-feature element j in [0,42): [x,y,z, sin/cos(f_k * x,y,z)..., R d]   code.py:30-42, models.py:183-209
-__device__ __forceinline__ float zfeat_value(const Projection& p, int j, int num_freqs, float freq_factor) {
-  const int n_pe = 3 + 6 * num_freqs;
-  if (j < 3) return j == 0 ? p.xr : (j == 1 ? p.yr : p.zr);
-  if (j < n_pe) {
-    int q = j - 3;
-    int k = q / 6;             // frequency index
-    int r = q - k * 6;         // 0..2 sin(x,y,z), 3..5 cos(x,y,z)
-    int d = r % 3;
-    float x = d == 0 ? p.xr : (d == 1 ? p.yr : p.zr);
-    float f = freq_factor * (float)(1 << k);
-    float ph = r >= 3 ? 1.57079637050628662109375f : 0.0f;   // float32(pi/2), code.py:26-27
-    return sinf(fmaf(x, f, ph));                             // sin(addcmul(phase, x, freq)): ATen fuses the multiply-add
-  }
-  int d = j - n_pe;
-  return d == 0 ? p.dx : (d == 1 ? p.dy : p.dz);
+// z-feature layout of the PNR_SCENE_ZF_* bits (include/pixelnerf_b200.h; models.py:16-90, 183-209).  A row is
+//   [u (n_raw columns), sin(f_0 u), cos(f_0 u), sin(f_1 u), ... (up to n_code), R d (up to width)]
+// where u (n_u values) is the encoder input: the coordinates (3, or -z alone), then R d with CODE_VIEWDIRS.  Without the
+// encoder (NO_CODE) the row is u itself, n_raw = n_code = n_u.  All bits clear: [x, y, z, sin/cos(f_k x,y,z)..., R d].
+struct ZfLayout {
+  int n_xyz;    // coordinate values of u: 3, or 1 (-z, Z_ONLY)
+  int n_u;      // encoder input width: n_xyz, + 3 with CODE_VIEWDIRS
+  int n_raw;    // leading columns that are u itself: n_u, or 0 with NO_CODE_INPUT
+  int n_code;   // columns of the (encoded) u block
+  int width;    // n_code, + 3 raw view-direction columns unless NO_VIEWDIRS or CODE_VIEWDIRS (= d_in)
+  bool cam;     // coordinates are R x + t (CAM_COORDS) instead of R x
+};
+constexpr int kZfFlags = PNR_SCENE_ZF_NO_VIEWDIRS | PNR_SCENE_ZF_CODE_VIEWDIRS | PNR_SCENE_ZF_CAM_COORDS | PNR_SCENE_ZF_Z_ONLY |
+                         PNR_SCENE_ZF_NO_CODE | PNR_SCENE_ZF_NO_CODE_INPUT;
+__host__ __device__ inline ZfLayout zf_layout(int flags, int num_freqs) {
+  const bool dirs = !(flags & PNR_SCENE_ZF_NO_VIEWDIRS);
+  const bool code_dirs = dirs && (flags & PNR_SCENE_ZF_CODE_VIEWDIRS);      // models.py: use_viewdirs and use_code_viewdirs
+  const bool code = !(flags & PNR_SCENE_ZF_NO_CODE);
+  ZfLayout L;
+  L.n_xyz = (flags & PNR_SCENE_ZF_Z_ONLY) ? 1 : 3;
+  L.n_u = L.n_xyz + (code_dirs ? 3 : 0);
+  L.n_raw = (code && (flags & PNR_SCENE_ZF_NO_CODE_INPUT)) ? 0 : L.n_u;
+  L.n_code = L.n_raw + (code ? 2 * num_freqs * L.n_u : 0);
+  L.width = L.n_code + (dirs && !code_dirs ? 3 : 0);
+  L.cam = (flags & PNR_SCENE_ZF_CAM_COORDS) != 0;
+  return L;
 }
 
-// Same element for the bf16 tensor-core path, where the value is rounded to bf16 (2^-9 relative) right after: explicit
-// range reduction in turns + the SFU sine (abs error < 1e-5 for |f x| < 128) instead of the ~40-instruction libm sinf,
-// which was 45 % of the gather warps' issue slots in the fused kernel (ncu source page, profiles/).
-__device__ __forceinline__ float zfeat_value_fast(const Projection& p, int j, int num_freqs, float freq_factor) {
-  const int n_pe = 3 + 6 * num_freqs;
-  if (j < 3) return j == 0 ? p.xr : (j == 1 ? p.yr : p.zr);
-  if (j < n_pe) {
-    const int q = j - 3, k = q / 6, r = q - k * 6, d = r % 3;
-    const float x = d == 0 ? p.xr : (d == 1 ? p.yr : p.zr);
-    const float f_turns = freq_factor * (float)(1 << k) * 0.15915494309189535f;      // f / (2 pi)
-    float t = fmaf(x, f_turns, r >= 3 ? 0.25f : 0.0f);
-    t -= rintf(t);                                                                    // [-0.5, 0.5] turns
-    return __sinf(t * 6.283185307179586f);
+__device__ __forceinline__ float zf_dir(const Projection& p, int d) { return d == 0 ? p.dx : (d == 1 ? p.dy : p.dz); }
+// value i of the encoder input u.  The tests are ordered so that a layout known at compile time keeps only its own case.
+__device__ __forceinline__ float zf_input(const Projection& p, const ZfLayout& L, int i) {
+  if (L.n_u > L.n_xyz && i >= L.n_xyz) return zf_dir(p, i - L.n_xyz);
+  if (L.n_xyz == 1) return -(L.cam ? p.zc : p.zr);
+  return L.cam ? (i == 0 ? p.xc : (i == 1 ? p.yc : p.zc)) : (i == 0 ? p.xr : (i == 1 ? p.yr : p.zr));
+}
+// Encoded column j in [n_raw, n_code): input value index i, frequency index k, and whether it is the cosine.
+struct ZfCode { int i, k; bool cos; };
+__device__ __forceinline__ ZfCode zf_code(const ZfLayout& L, int j) {
+  const int q = j - L.n_raw, k = q / (2 * L.n_u), r = q - k * 2 * L.n_u;
+  return ZfCode{r % L.n_u, k, r >= L.n_u};
+}
+
+// z-feature element j in [0, L.width)   code.py:30-42, models.py:183-209
+// FAST = false: sinf of the fp32 argument, as ATen computes it (the fp32 paths).  FAST = true, for the bf16 tensor-core path
+// where the value is rounded to bf16 (2^-9 relative) right after: explicit range reduction in turns + the SFU sine (abs error
+// < 1e-5 for |f x| < 128) instead of the ~40-instruction libm sinf, which was 45 % of the gather warps' issue slots in the
+// fused kernel (ncu source page, profiles/).
+template <bool FAST>
+__device__ __forceinline__ float zfeat_value(const Projection& p, const ZfLayout& L, int j, int num_freqs, float freq_factor) {
+  if (j < L.n_raw) return zf_input(p, L, j);
+  if (j < L.n_code) {
+    const ZfCode c = zf_code(L, j);
+    const float x = zf_input(p, L, c.i);
+    if (FAST) {
+      const float f_turns = freq_factor * (float)(1 << c.k) * 0.15915494309189535f;      // f / (2 pi)
+      float t = fmaf(x, f_turns, c.cos ? 0.25f : 0.0f);
+      t -= rintf(t);                                                                      // [-0.5, 0.5] turns
+      return __sinf(t * 6.283185307179586f);
+    }
+    const float f = freq_factor * (float)(1 << c.k);
+    const float ph = c.cos ? 1.57079637050628662109375f : 0.0f;   // float32(pi/2), code.py:26-27
+    return sinf(fmaf(x, f, ph));                                   // sin(addcmul(phase, x, freq)): ATen fuses the multiply-add
   }
-  const int d = j - n_pe;
-  return d == 0 ? p.dx : (d == 1 ? p.dy : p.dz);
+  return zf_dir(p, j - L.n_code);
 }
 
 // near * (1 - s) + far * s (nerf.py:119,151: separately rounded), or the linear-in-disparity variant (nerf.py:121,153)

@@ -34,7 +34,7 @@ class _FieldTrainFn(torch.autograd.Function):
         tape = torch.empty(lib.pnr_field_tape_bytes(sc, pts, cp), dtype=torch.uint8, device=dev)
         with torch.cuda.device(dev):
             rc = lib.pnr_field_forward_train(sc, pts, cp, out.data_ptr(), tape.data_ptr(), tape.numel(),
-                                             net.code.num_freqs, net.code.freq_factor, _lib.stream_ptr(dev))
+                                             *net.code_args(), _lib.stream_ptr(dev))
         _lib.check(rc, "pnr_field_forward_train")
         net.last_launches = lib.pnr_last_launch_count()
         ctx.net, ctx.mlp, ctx.mode, ctx.sb, ctx.P = net, mlp, mode, sb, P
@@ -65,7 +65,7 @@ class _FieldTrainFn(torch.autograd.Function):
         with torch.cuda.device(dev):
             rc = lib.pnr_field_backward(sc, pts, cp, tape.data_ptr(), out.data_ptr(), d_out.data_ptr(),
                                         mlp.c_grads(grads), _lib.ptr(d_feat), _lib.ptr(d_xyz), _lib.ptr(d_z),
-                                        ws.data_ptr(), ws.numel(), net.code.num_freqs, net.code.freq_factor,
+                                        ws.data_ptr(), ws.numel(), *net.code_args(),
                                         _lib.stream_ptr(dev))
         _lib.check(rc, "pnr_field_backward")
         net.last_bwd_launches = getattr(net, "last_bwd_launches", 0) + lib.pnr_last_launch_count()
@@ -87,25 +87,38 @@ class PixelNeRFNet(torch.nn.Module):
         self.use_code_viewdirs = conf.get_bool("use_code_viewdirs", True)
         self.use_viewdirs = conf.get_bool("use_viewdirs", False)
         self.use_global_encoder = conf.get_bool("use_global_encoder", False)
-        # The fused kernels implement the switch set of every shipped conf (conf/default*.conf, conf/exp/*.conf), and both
+        # The fused kernels implement every switch that shapes the z-feature (the non-latent part of each MLP input row:
+        # use_xyz, normalize_z, use_code, code.include_input, use_viewdirs, use_code_viewdirs; PNR_SCENE_ZF_* bits) and both
         # view-pooling modes of ResnetFC: combine_type average / max before block combine_layer, or no pooling at all
-        # (combine_layer >= n_blocks, the single-view conf/default.conf network; one source view only).
+        # (combine_layer >= n_blocks, the single-view conf/default.conf network; one source view only).  Not built: the
+        # network without pixel-aligned features (use_encoder = False), the global encoder, and z-features wider than the
+        # one K = 64 slab of lin_in.
         unsupported = []
         if not self.use_encoder: unsupported.append("use_encoder=False")
-        if not self.use_xyz: unsupported.append("use_xyz=False")
-        if not self.normalize_z: unsupported.append("normalize_z=False")
-        if not self.use_code: unsupported.append("use_code=False")
-        if self.use_code_viewdirs: unsupported.append("use_code_viewdirs=True")
-        if not self.use_viewdirs: unsupported.append("use_viewdirs=False")
         if self.use_global_encoder: unsupported.append("use_global_encoder=True")
         if unsupported:
             raise NotImplementedError("PixelNeRFNet (B200 path) does not build: " + ", ".join(unsupported))
 
         d_latent = self.encoder.latent_size
-        self.code = PositionalEncoding.from_conf(conf["code"], d_in=3)
-        if not self.code.include_input:
-            raise NotImplementedError("PixelNeRFNet (B200 path): code.include_input=False is not built")
-        d_in = self.code.d_out + 3            # PE(xyz) ++ raw view directions (models.py:47-59)
+        # z-feature width and encoder exactly as models.py:16-90 (no `code` module, and no code.* state, without use_code)
+        d_in = 3 if self.use_xyz else 1
+        if self.use_viewdirs and self.use_code_viewdirs:
+            d_in += 3
+        if self.use_code and d_in > 0:
+            self.code = PositionalEncoding.from_conf(conf["code"], d_in=d_in)
+            d_in = self.code.d_out
+        if self.use_viewdirs and not self.use_code_viewdirs:
+            d_in += 3
+        if d_in > 64:
+            raise NotImplementedError(
+                f"PixelNeRFNet (B200 path): these switches give a z-feature of d_in={d_in} values; the fused kernels take at "
+                f"most 64 (one K = 64 slab of lin_in)")
+        self.zf_flags = ((0 if self.use_viewdirs else _lib.SCENE_ZF_NO_VIEWDIRS)
+                         | (_lib.SCENE_ZF_CODE_VIEWDIRS if self.use_viewdirs and self.use_code_viewdirs else 0)
+                         | (0 if self.normalize_z else _lib.SCENE_ZF_CAM_COORDS)
+                         | (0 if self.use_xyz else _lib.SCENE_ZF_Z_ONLY)
+                         | (0 if self.use_code else _lib.SCENE_ZF_NO_CODE)
+                         | (_lib.SCENE_ZF_NO_CODE_INPUT if self.use_code and not self.code.include_input else 0))
         self.latent_size = self.encoder.latent_size
         self.mlp_coarse = make_mlp(conf["mlp_coarse"], d_in, d_latent)
         self.mlp_fine = make_mlp(conf["mlp_fine"], d_in, d_latent, allow_empty=True)
@@ -226,13 +239,19 @@ class PixelNeRFNet(torch.nn.Module):
         sc.feat, sc.poses, sc.focal, sc.center = feat.data_ptr(), poses.data_ptr(), focal.data_ptr(), center.data_ptr()
         sc.SB, sc.NS, sc.C, sc.Hl, sc.Wl = SB, NS, feat.shape[3], feat.shape[1], feat.shape[2]
         sc.feat_fp32 = int(fp32_maps)
-        sc.flags = (_lib.SCENE_MASK_NONNEG_Z | _lib.SCENE_RAW_OUTPUT) if self.yolo else 0
+        sc.flags = ((_lib.SCENE_MASK_NONNEG_Z | _lib.SCENE_RAW_OUTPUT) if self.yolo else 0) | self.zf_flags
         if fp32_maps and self.train_precision == "tf32":
             sc.flags |= _lib.SCENE_TRAIN_TF32            # read by the training entry points only
         elif fp32_maps and self.train_precision == "bf16":
             sc.flags |= _lib.SCENE_TRAIN_BF16
         sc.image_w, sc.image_h, sc.lat_scale_x, sc.lat_scale_y = iw, ih, lsx, lsy
         return sc, (poses, focal, center, iw, ih, lsx, lsy)
+
+    def code_args(self):
+        """(num_freqs, freq_factor) of the z-feature's positional encoding for the C entry points; (0, 0.0) without one."""
+        if not self.use_code:
+            return 0, 0.0
+        return self.code.num_freqs, float(self.code.freq_factor)
 
     def projects_latent(self) -> bool:
         """True when the tcgen05 path gathers lin_z PRE-PROJECTIONS of the maps (PNR_SCENE_PROJECTED): automatic for latents
@@ -289,7 +308,7 @@ class PixelNeRFNet(torch.nn.Module):
                 if ws is None or ws.numel() < max(ws_bytes, 16) or ws.device != dev:
                     ws = self._field_ws = torch.empty(max(ws_bytes, 16), dtype=torch.uint8, device=dev)
                 rc = lib.pnr_field_forward(sc, pts, mlp.c_params(), mlp.packed(projected=proj).data_ptr(), out.data_ptr(),
-                                           ws.data_ptr(), ws_bytes, _lib.PREC_BF16, self.code.num_freqs, self.code.freq_factor,
+                                           ws.data_ptr(), ws_bytes, _lib.PREC_BF16, *self.code_args(),
                                            _lib.stream_ptr(dev))
                 _lib.check(rc, "pnr_field_forward(bf16)")
                 launches = lib.pnr_last_launch_count()
@@ -299,7 +318,7 @@ class PixelNeRFNet(torch.nn.Module):
                 ws_bytes = lib.pnr_field_workspace_bytes(sc, pts, _lib.PREC_FP32)
                 ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
                 rc = lib.pnr_field_forward(sc, pts, cp, None, out.data_ptr(), ws.data_ptr(), ws_bytes,
-                                           _lib.PREC_FP32, self.code.num_freqs, self.code.freq_factor,
+                                           _lib.PREC_FP32, *self.code_args(),
                                            _lib.stream_ptr(dev))
                 _lib.check(rc, "pnr_field_forward(fp32)")
                 launches = lib.pnr_last_launch_count()
@@ -309,22 +328,26 @@ class PixelNeRFNet(torch.nn.Module):
         return out
 
     def forward(self, xyz, coarse=True, viewdirs=None, far=False):
-        """(r, g, b, sigma) at world points xyz (SB, B, 3) given view directions (SB, B, 3) -> (SB, B, 4)."""
+        """(r, g, b, sigma) at world points xyz (SB, B, 3) given view directions (SB, B, 3) -> (SB, B, 4).  viewdirs may be
+        None when the network does not use them (use_viewdirs = False)."""
         SB, B, _ = xyz.shape
-        assert viewdirs is not None
+        if self.use_viewdirs:
+            assert viewdirs is not None
         _lib.require_cuda(xyz, "xyz")
+        if viewdirs is not None:
+            viewdirs = viewdirs.detach().reshape(SB, B, 3).contiguous().float()
         if self._wants_grad(coarse, xyz):
             assert SB * self.num_views_per_obj == self.poses.shape[0], "call encode() first"
             mlp = self._mlp(coarse)
-            return _FieldTrainFn.apply(self, mlp, "xyz", SB, self._train_feat(), xyz.contiguous().float(),
-                                       viewdirs.detach().reshape(SB, B, 3).contiguous().float(), *mlp.ordered_params())
+            return _FieldTrainFn.apply(self, mlp, "xyz", SB, self._train_feat(), xyz.contiguous().float(), viewdirs,
+                                       *mlp.ordered_params())
         xyz = xyz.detach().contiguous().float()
-        viewdirs = viewdirs.detach().reshape(SB, B, 3).contiguous().float()
         assert SB * self.num_views_per_obj == self.poses.shape[0], "call encode() first"
         outs = []
         step = B if self.precision == "bf16" else max(1, self.fp32_chunk_points // max(SB * self.num_views_per_obj, 1))
         for b0 in range(0, max(B, 1), max(step, 1)):
-            xs, ds = xyz[:, b0:b0 + step].contiguous(), viewdirs[:, b0:b0 + step].contiguous()
+            xs = xyz[:, b0:b0 + step].contiguous()
+            ds = None if viewdirs is None else viewdirs[:, b0:b0 + step].contiguous()
             pts = _lib.points_xyz(xs, ds)
             outs.append(self._run_field(pts, SB, xs.shape[1], coarse, (xs, ds)))
         return outs[0] if len(outs) == 1 else torch.cat(outs, dim=1)

@@ -306,7 +306,7 @@ class NeRFRenderer(torch.nn.Module):
                     a.mlp_fine, a.packed_fine = C.pointer(cpf), pk_f.data_ptr()
                 a.n_coarse, a.n_fine, a.n_fine_depth = kc, (self.n_fine if fine else 0), (kfd if fine else 0)
                 a.depth_std, a.white_bkgd, a.lindisp = float(self.depth_std), int(bool(self.white_bkgd)), int(bool(self.lindisp))
-                a.precision, a.num_freqs, a.freq_factor = _lib.PREC_BF16, model.code.num_freqs, float(model.code.freq_factor)
+                a.precision, (a.num_freqs, a.freq_factor) = _lib.PREC_BF16, model.code_args()
                 a.n_splits = 1 if self.field_events is not None else int(self.n_splits)
                 nbytes = lib.pnr_render_workspace_bytes(a)
                 ws = self._ws_cache.get(key[0])                # one persistent workspace per (renderer, device)
