@@ -279,11 +279,55 @@ int pnr_field_backward(const pnr_scene* scene, const pnr_points* pts, const pnr_
                        const float* out, const float* d_out, const pnr_mlp_grads* grads, float* d_feat, float* d_xyz,
                        float* d_z, void* workspace, size_t workspace_bytes, int num_freqs, float freq_factor,
                        void* stream);
+/* Camera gradients of the field function: what autograd sends, for the reference, into the camera inputs of
+ * PixelNeRFNet.encode / forward and of the renderers.  Optional outputs that pnr_field_backward_cameras ADDS into (the caller
+ * zeroes them); NULL = not wanted.
+ *   d_poses  (SB*NS, 3, 4): with respect to the world->camera matrices of scene->poses (R | t);
+ *   d_focal  (SB*NS, 2)   : with respect to scene->focal, the per-view values the kernels read (fy sign convention and YOLO
+ *                           negation already applied: uv = -xy / z * focal + center);
+ *   d_center (SB*NS, 2)   : with respect to scene->center;
+ *   d_dirs   (SB, P, 3)   : point mode 0: with respect to pts->dirs (used only by z-feature layouts with view directions);
+ *   d_rays   (SB*B, 8)    : point mode 1: columns 0-5, origin and direction of pts->rays (points o + z d, view direction d).
+ *                           Near and far reach the depths only through the samplers: pnr_sample_bounds_backward.
+ * image_shape and latent_scaling are constants (buffers in the reference). */
+typedef struct pnr_camera_grads {
+  float* d_poses;
+  float* d_focal;
+  float* d_center;
+  float* d_dirs;
+  float* d_rays;
+} pnr_camera_grads;
+/* pnr_field_backward plus the camera gradients of `cams` (NULL, or all of its pointers NULL: exactly pnr_field_backward).
+ * The gradient of the projection x_cam = R x + t, uv = -x_cam.xy / x_cam.z * focal + center, of the bilinear tap position
+ * (a row whose latent is zeroed -- YOLO z >= 0 -- or whose taps all fall outside the map has none) and of the z-feature
+ * inputs (R x, R x + t, -z, R d, raw or encoded) of every (object, view, point) row, summed over rows per view and over
+ * views per point or ray. */
+int pnr_field_backward_cameras(const pnr_scene* scene, const pnr_points* pts, const pnr_mlp_params* params, const void* tape,
+                               const float* out, const float* d_out, const pnr_mlp_grads* grads, float* d_feat, float* d_xyz,
+                               float* d_z, const pnr_camera_grads* cams, void* workspace, size_t workspace_bytes, int num_freqs,
+                               float freq_factor, void* stream);
 /* Backward of pnr_composite (nerf.py:184-188, 229-255): d_rgb (B,3), d_depth (B, may be NULL), d_weights (B,K, may be
  * NULL) -> d_rgb_sigma (B,K,4) and, if non-NULL, d_z (B,K) (both overwritten). */
 int pnr_composite_backward(const float* rgb_sigma, const float* z, const float* rays, const float* d_rgb,
                            const float* d_depth, const float* d_weights, float* d_rgb_sigma, float* d_z, int B, int K,
                            int white_bkgd, void* stream);
+/* pnr_composite_backward that also adds d far (the last interval is far - z_K, nerf.py:187) into column 7 of d_rays (B, 8)
+ * when d_rays is non-NULL. */
+int pnr_composite_backward_rays(const float* rgb_sigma, const float* z, const float* rays, const float* d_rgb,
+                                const float* d_depth, const float* d_weights, float* d_rgb_sigma, float* d_z, float* d_rays,
+                                int B, int K, int white_bkgd, void* stream);
+/* Near / far gradients of the sample depths (nerf.py:104-167, 300-301), added into columns 6 and 7 of d_rays (B, 8).
+ *   z_sorted == NULL, the coarse samples: z = near (1 - s) + far s (lindisp: 1 / ((1 - s) / near + s / far)) with
+ *     s = steps_k + noise_coarse / Kc (as pnr_sample_coarse), given their gradient d_z_coarse (B, Kc).
+ *   z_sorted != NULL, the fine pass: the merged row z_sorted (B, Kc+Kf+Kfd) of pnr_sample_fine and its gradient d_z_sorted.
+ *     Each sample is found at the position of its value (equal values in concatenation order).  Importance samples have
+ *     s = (inds + jitter) / Kc (inds (B, Kf) int32 from pnr_sample_fine's inds_out); depth samples clamped at near or far
+ *     send their gradient there; the coarse samples' share is written to d_z_coarse_out (B, Kc; may be NULL).  The
+ *     unclamped depth samples' share is pnr_sample_fine_depth_backward's. */
+int pnr_sample_bounds_backward(const float* rays, const float* steps, const float* noise_coarse, const float* d_z_coarse,
+                               const float* z_coarse, const float* z_sorted, const float* d_z_sorted, const int32_t* inds,
+                               const float* jitter, const float* depth, const float* gauss, float* d_rays, float* d_z_coarse_out,
+                               int B, int Kc, int Kf, int Kfd, float depth_std, int lindisp, void* stream);
 /* Backward of sample_fine_depth + cat + sort (nerf.py:156-167, 296-301) with respect to the coarse depth:
  * d_depth[b] = sum of d_z_sorted over the positions of the unclamped depth samples (overwritten). */
 int pnr_sample_fine_depth_backward(const float* z_sorted, const float* d_z_sorted, const float* depth,

@@ -40,7 +40,8 @@ EXPORTS = [
     "pnr_field_tape_bytes", "pnr_field_forward_train", "pnr_field_backward_workspace_bytes", "pnr_field_backward",
     "pnr_composite_backward", "pnr_sample_fine_depth_backward", "pnr_pyramid_pack", "pnr_gen_rays", "pnr_yolo_reduce", "pnr_image_output", "pnr_rgb_loss",
     "pnr_mlp_pack_projected_bytes", "pnr_mlp_pack_projected", "pnr_project_features",
-    "pnr_render_workspace_bytes", "pnr_render_forward", "pnr_zfeat_width",
+    "pnr_render_workspace_bytes", "pnr_render_forward", "pnr_zfeat_width", "pnr_field_backward_cameras",
+    "pnr_composite_backward_rays", "pnr_sample_bounds_backward",
 ]
 # test hooks of the training GEMMs (csrc/pnr_lab.h, internal); not part of the product ABI
 LAB_EXPORTS = ["pnr_lab_gemm_workspace_bytes", "pnr_lab_rowgemm", "pnr_lab_wgrad"]
@@ -94,6 +95,12 @@ class MlpGrads(C.Structure):
                 ("lin_out_b", C.c_void_p), ("fc0_w", C.c_void_p * 8), ("fc0_b", C.c_void_p * 8),
                 ("fc1_w", C.c_void_p * 8), ("fc1_b", C.c_void_p * 8), ("linz_w", C.c_void_p * 8),
                 ("linz_b", C.c_void_p * 8)]
+
+
+class CameraGrads(C.Structure):
+    """pnr_camera_grads: optional camera-gradient accumulators of pnr_field_backward_cameras (None = not wanted)."""
+    _fields_ = [("d_poses", C.c_void_p), ("d_focal", C.c_void_p), ("d_center", C.c_void_p), ("d_dirs", C.c_void_p),
+                ("d_rays", C.c_void_p)]
 
 
 class RenderArgs(C.Structure):
@@ -164,7 +171,12 @@ def load() -> C.CDLL:
     lib.pnr_field_backward_workspace_bytes.restype = C.c_size_t
     lib.pnr_field_backward.argtypes = [C.POINTER(Scene), C.POINTER(Points), C.POINTER(MlpParams), vp, vp, vp,
                                        C.POINTER(MlpGrads), vp, vp, vp, vp, C.c_size_t, i32, f32, vp]
+    lib.pnr_field_backward_cameras.argtypes = [C.POINTER(Scene), C.POINTER(Points), C.POINTER(MlpParams), vp, vp, vp,
+                                               C.POINTER(MlpGrads), vp, vp, vp, C.POINTER(CameraGrads), vp, C.c_size_t, i32,
+                                               f32, vp]
     lib.pnr_composite_backward.argtypes = [vp] * 8 + [i32, i32, i32, vp]
+    lib.pnr_composite_backward_rays.argtypes = [vp] * 9 + [i32, i32, i32, vp]
+    lib.pnr_sample_bounds_backward.argtypes = [vp] * 13 + [i32, i32, i32, i32, f32, i32, vp]
     lib.pnr_sample_fine_depth_backward.argtypes = [vp] * 6 + [i32, i32, i32, f32, vp]
     lib.pnr_pyramid_pack.argtypes = [C.POINTER(vp), C.POINTER(C.c_int32), C.POINTER(C.c_int32), C.POINTER(C.c_int32),
                                      i32, i32, vp, i32, vp]

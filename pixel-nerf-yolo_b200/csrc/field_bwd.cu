@@ -561,17 +561,71 @@ lin_out_bwd_kernel(const T* __restrict__ x, const float* __restrict__ W, const f
 // Backward of projection + bilinear gather + positional encoding for one (object, view, point) row per warp.
 //   dlat (rows, C), dzf (rows, d_in = z-feature width)  ->  d_feat (fp32 channels-last maps, atomics; may be null),
 //   d_xyz (SB*P, 3) (mode 0) or d_z (SB*B*K) (mode 1: x = o + z d  =>  dz = dx . d), atomics; may be null.
+// CAM adds the camera inputs (pnr_camera_grads; every pointer may be null).  With x_rot = R x, x_cam = R x + t, d_rot = R d of
+// the row's view and u = -x_cam / z_cam * f + c (per axis):
+//   d R += d(x_rot) x^T + d(d_rot) d^T,  d t += d(x_cam),  d f = d u * (-x_cam / z_cam),  d c = d u,
+//   d d (world) = R^T d(d_rot)  (point mode: d_dirs; ray mode: with x = o + z d, d o += R^T d(x_rot), d d += z R^T d(x_rot) too).
+// Per-view sums (16 values) stay in the registers of lane 0 while a warp's rows stay in one view, then go to a shared-memory
+// slot of the block's first kCamSlots views and leave the block in one reduction per (block, view); per-ray sums likewise
+// leave a warp once per ray.  CAM gives every warp a contiguous run of rows so that these runs are long.
+struct CamGrads { float *d_poses, *d_focal, *d_center, *d_dirs, *d_rays; };
+constexpr int kCamSlots = 8;
+// accumulator e of a view: 0-11 the (3, 4) pose matrix row-major, 12-13 focal, 14-15 center
+__device__ __forceinline__ float* cam_target(const CamGrads& cg, long long view, int e) {
+  if (e < 12) return cg.d_poses ? cg.d_poses + view * 12 + e : nullptr;
+  if (e < 14) return cg.d_focal ? cg.d_focal + view * 2 + (e - 12) : nullptr;
+  return cg.d_center ? cg.d_center + view * 2 + (e - 14) : nullptr;
+}
+template <bool CAM>
 __global__ void __launch_bounds__(256)
 gather_encode_bwd_kernel(pnr_scene sc, pnr_points q, const float* __restrict__ dlat, const float* __restrict__ dzf,
                          float* __restrict__ d_feat, float* __restrict__ d_xyz, float* __restrict__ d_z, int num_freqs,
-                         float freq_factor, long long n_rows) {
+                         float freq_factor, long long n_rows, CamGrads cg) {
+  extern __shared__ float s_cam[];                 // CAM: [kCamSlots][16] per-view sums of this block
   const int lane = threadIdx.x & 31;
   const long long warp = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const long long n_warps = ((long long)gridDim.x * blockDim.x) >> 5;
   const int NS = sc.NS, P = q.P, C = sc.C;
   const ZfLayout L = zf_layout(sc.flags, num_freqs);
-  const bool want_x = d_xyz || d_z;
-  for (long long row = warp; row < n_rows; row += n_warps) {
+  const bool want_x = CAM || d_xyz || d_z;
+  long long row_begin = warp, row_end = n_rows, row_step = n_warps;
+  long long v0 = 0;                                // first view of the block (CAM)
+  float acc[16], racc[6];                          // CAM: sums of the current view / ray (lane 0)
+  long long cur_view = -1, cur_ray = -1;
+  if constexpr (CAM) {
+    const long long rpw = (n_rows + n_warps - 1) / n_warps;
+    row_begin = warp * rpw;
+    row_end = row_begin + rpw < n_rows ? row_begin + rpw : n_rows;
+    row_step = 1;
+    v0 = ((long long)blockIdx.x * (blockDim.x >> 5) * rpw) / P;
+    for (int i = threadIdx.x; i < kCamSlots * 16; i += blockDim.x) s_cam[i] = 0.f;
+#pragma unroll
+    for (int e = 0; e < 16; ++e) acc[e] = 0.f;
+#pragma unroll
+    for (int e = 0; e < 6; ++e) racc[e] = 0.f;
+    __syncthreads();
+  }
+  auto flush_view = [&]() {
+    if (cur_view < 0) return;
+    const long long slot = cur_view - v0;
+#pragma unroll
+    for (int e = 0; e < 16; ++e) {
+      if (acc[e] != 0.f) {
+        if (slot >= 0 && slot < kCamSlots) atomicAdd(s_cam + slot * 16 + e, acc[e]);
+        else if (float* dst = cam_target(cg, cur_view, e)) atomicAdd(dst, acc[e]);
+      }
+      acc[e] = 0.f;
+    }
+  };
+  auto flush_ray = [&]() {
+    if (cur_ray < 0) return;
+#pragma unroll
+    for (int e = 0; e < 6; ++e) {
+      if (racc[e] != 0.f) atomicAdd(cg.d_rays + cur_ray * 8 + e, racc[e]);
+      racc[e] = 0.f;
+    }
+  };
+  for (long long row = row_begin; row < row_end; row += row_step) {
     const int view = (int)(row / P);
     const int p = (int)(row - (long long)view * P);
     const int s = view / NS;
@@ -613,11 +667,12 @@ gather_encode_bwd_kernel(pnr_scene sc, pnr_points q, const float* __restrict__ d
     }
     if (!want_x) continue;
     // z-feature: column j < n_code depends on encoder input i of u (zfeat_value).  Inputs i < n_xyz are coordinates of R x
-    // (R x + t with CAM_COORDS: same derivative), or -z alone with Z_ONLY; the view-direction values carry no gradient to
-    // the points.
-    float gx[3] = {0.f, 0.f, 0.f};
-    for (int j = lane; j < L.n_code; j += 32) {
+    // (R x + t with CAM_COORDS: same derivative), or -z alone with Z_ONLY; the view-direction values (inputs i >= n_xyz with
+    // CODE_VIEWDIRS, the raw columns from n_code on otherwise) carry gradient to the camera inputs only.
+    float gx[3] = {0.f, 0.f, 0.f}, gd[3] = {0.f, 0.f, 0.f};
+    for (int j = lane; j < (CAM ? L.width : L.n_code); j += 32) {
       const float gj = dzf[row * L.width + j];
+      if (CAM && j >= L.n_code) { gd[j - L.n_code] += gj; continue; }
       int i = j;
       float dv = gj;
       if (j >= L.n_raw) {
@@ -627,7 +682,10 @@ gather_encode_bwd_kernel(pnr_scene sc, pnr_points q, const float* __restrict__ d
         i = c.i;
         dv = gj * f * cosf(fmaf(zf_input(pr, L, i), f, ph));    // d/du sin(f u + ph)
       }
-      if (i >= L.n_xyz) continue;
+      if (i >= L.n_xyz) {
+        if (CAM) gd[i - L.n_xyz] += dv;
+        continue;
+      }
       if (L.n_xyz == 1) gx[2] -= dv;                             // u = -z
       else gx[i] += dv;
     }
@@ -638,20 +696,28 @@ gather_encode_bwd_kernel(pnr_scene sc, pnr_points q, const float* __restrict__ d
       gx[0] += __shfl_xor_sync(0xffffffffu, gx[0], d);
       gx[1] += __shfl_xor_sync(0xffffffffu, gx[1], d);
       gx[2] += __shfl_xor_sync(0xffffffffu, gx[2], d);
+      if constexpr (CAM) {
+        gd[0] += __shfl_xor_sync(0xffffffffu, gd[0], d);
+        gd[1] += __shfl_xor_sync(0xffffffffu, gd[1], d);
+        gd[2] += __shfl_xor_sync(0xffffffffu, gd[2], d);
+      }
     }
     if (lane == 0) {
       const float* M = sc.poses + (size_t)view * 12;
       const float xc = pr.xc, yc = pr.yc, zc = pr.zc;
       const float fxv = sc.focal[view * 2 + 0], fyv = sc.focal[view * 2 + 1];
       // ix = u * (lat_scale_x / image_w) * 0.5 * (Wl - 1),  u = -xc / zc * fx + cx
-      const float du = gix * (sc.lat_scale_x / sc.image_w) * 0.5f * (float)(sc.Wl - 1);
-      const float dv = giy * (sc.lat_scale_y / sc.image_h) * 0.5f * (float)(sc.Hl - 1);
+      float du = gix * (sc.lat_scale_x / sc.image_w) * 0.5f * (float)(sc.Wl - 1);
+      float dv = giy * (sc.lat_scale_y / sc.image_h) * 0.5f * (float)(sc.Hl - 1);
       const float inv_z = 1.0f / zc;
       float gc[3];
       gc[0] = -fxv * inv_z * du;
       gc[1] = -fyv * inv_z * dv;
       gc[2] = (xc * fxv * du + yc * fyv * dv) * inv_z * inv_z;
-      if (!isfinite(gc[0]) || !isfinite(gc[1]) || !isfinite(gc[2])) gc[0] = gc[1] = gc[2] = 0.f;   // point on the camera plane
+      if (!isfinite(gc[0]) || !isfinite(gc[1]) || !isfinite(gc[2])) {     // point on the camera plane, or a masked (NaN) row
+        gc[0] = gc[1] = gc[2] = 0.f;
+        du = dv = 0.f;
+      }
       const float r0 = gx[0] + gc[0], r1 = gx[1] + gc[1], r2 = gx[2] + gc[2];
       // x_rot = R x  =>  dx = R^T d(x_rot)
       const float wx = M[0] * r0 + M[4] * r1 + M[8] * r2;
@@ -659,8 +725,65 @@ gather_encode_bwd_kernel(pnr_scene sc, pnr_points q, const float* __restrict__ d
       const float wz = M[2] * r0 + M[6] * r1 + M[10] * r2;
       if (d_xyz) { atomicAdd(d_xyz + pidx * 3 + 0, wx); atomicAdd(d_xyz + pidx * 3 + 1, wy); atomicAdd(d_xyz + pidx * 3 + 2, wz); }
       if (d_z) atomicAdd(d_z + pidx, wx * vx + wy * vy + wz * vz);
+      if constexpr (CAM) {
+        if (view != cur_view) { flush_view(); cur_view = view; }
+        const float r[3] = {r0, r1, r2}, tx = L.cam ? 1.f : 0.f;
+#pragma unroll
+        for (int a = 0; a < 3; ++a) {
+          acc[a * 4 + 0] += r[a] * px + gd[a] * vx;
+          acc[a * 4 + 1] += r[a] * py + gd[a] * vy;
+          acc[a * 4 + 2] += r[a] * pz + gd[a] * vz;
+          acc[a * 4 + 3] += gc[a] + tx * gx[a];
+        }
+        acc[12] += du * (-xc * inv_z);
+        acc[13] += dv * (-yc * inv_z);
+        acc[14] += du;
+        acc[15] += dv;
+        // d_rot = R d  =>  d d = R^T d(d_rot)
+        const float ex = M[0] * gd[0] + M[4] * gd[1] + M[8] * gd[2];
+        const float ey = M[1] * gd[0] + M[5] * gd[1] + M[9] * gd[2];
+        const float ez = M[2] * gd[0] + M[6] * gd[1] + M[10] * gd[2];
+        if (cg.d_dirs) { atomicAdd(cg.d_dirs + pidx * 3 + 0, ex); atomicAdd(cg.d_dirs + pidx * 3 + 1, ey); atomicAdd(cg.d_dirs + pidx * 3 + 2, ez); }
+        if (cg.d_rays) {
+          const long long ray = pidx / q.K;
+          if (ray != cur_ray) { flush_ray(); cur_ray = ray; }
+          const float zz = q.z[pidx];
+          racc[0] += wx; racc[1] += wy; racc[2] += wz;
+          racc[3] += zz * wx + ex; racc[4] += zz * wy + ey; racc[5] += zz * wz + ez;
+        }
+      }
     }
   }
+  if constexpr (CAM) {
+    if (lane == 0) { flush_view(); if (cg.d_rays) flush_ray(); }
+    __syncthreads();
+    const long long n_views = (long long)sc.SB * NS;
+    for (int i = threadIdx.x; i < kCamSlots * 16; i += blockDim.x) {
+      const long long view = v0 + i / 16;
+      if (s_cam[i] == 0.f || view >= n_views) continue;
+      if (float* dst = cam_target(cg, view, i % 16)) atomicAdd(dst, s_cam[i]);
+    }
+  }
+}
+
+static bool wants_cams(const pnr_camera_grads* cams) {
+  return cams && (cams->d_poses || cams->d_focal || cams->d_center || cams->d_dirs || cams->d_rays);
+}
+// the last kernel of both backward chains: dlat / dzf -> feature maps, points, camera inputs
+static int gather_bwd(const pnr_scene* sc, const pnr_points* q, const float* dlat, const float* dzf, float* d_feat, float* d_xyz,
+                      float* d_z, const pnr_camera_grads* cams, int num_freqs, float freq_factor, long long rows, cudaStream_t st) {
+  long long blocks = (rows + 7) / 8;
+  if (blocks > 148LL * 64) blocks = 148LL * 64;
+  if (wants_cams(cams)) {
+    const CamGrads cg = {cams->d_poses, cams->d_focal, cams->d_center, cams->d_dirs, cams->d_rays};
+    gather_encode_bwd_kernel<true><<<(unsigned)blocks, 256, kCamSlots * 16 * sizeof(float), st>>>(*sc, *q, dlat, dzf, d_feat, d_xyz, d_z,
+                                                                                                  num_freqs, freq_factor, rows, cg);
+  } else {
+    gather_encode_bwd_kernel<false><<<(unsigned)blocks, 256, 0, st>>>(*sc, *q, dlat, dzf, d_feat, d_xyz, d_z, num_freqs, freq_factor, rows,
+                                                                      CamGrads{});
+  }
+  PNR_CHECK_LAUNCH("bwd::gather_encode_bwd_kernel");
+  return PNR_OK;
 }
 
 // fp32 (rows, H) -> bf16 slice of a wider channels-last map
@@ -867,14 +990,15 @@ static BwdWsB carve_bwd_b(uint8_t* base, long long rows, long long pts, int C, i
 }
 
 static int backward_bf16(const pnr_scene* sc, const pnr_points* q, const pnr_mlp_params* mp, const void* tape, const float* out,
-                         const float* d_out, const pnr_mlp_grads* gr, float* d_feat, float* d_xyz, float* d_z, void* workspace,
-                         int num_freqs, float freq_factor, cudaStream_t st) {
+                         const float* d_out, const pnr_mlp_grads* gr, float* d_feat, float* d_xyz, float* d_z,
+                         const pnr_camera_grads* cams, void* workspace, int num_freqs, float freq_factor, cudaStream_t st) {
   const long long rows = (long long)sc->SB * sc->NS * q->P, pts = (long long)sc->SB * q->P;
   const int H = mp->d_hidden, C = sc->C, d_in = mp->d_in, nb = mp->n_blocks, CL = mp->combine_layer, NS = sc->NS;
   const TapeB t = carve_tape_b(align1k(const_cast<void*>(tape)), rows, pts, C, H, nb, CL, pool_max(sc, mp));
   const BwdWsB ws = carve_bwd_b(align1k(workspace), rows, pts, C, d_in, H, nb, CL);
   const WPack w = wpack_layout(C, 64, H, nb, CL, true);
   int launches = 0, rc;
+  const bool want_in = d_feat || d_xyz || d_z || wants_cams(cams);
   if ((rc = pack_all(mp, C, true, ws.wpack, w, st, &launches))) return rc;
   const int raw = (sc->flags & PNR_SCENE_RAW_OUTPUT) ? 1 : 0;
   {
@@ -918,7 +1042,7 @@ static int backward_bf16(const pnr_scene* sc, const pnr_points* q, const pnr_mlp
   for (int b = CL - 1; b >= 0; --b) {
     if ((rc = block_bwd(t.RX[b], t.RN[b], b, ws.dx, rows))) return rc;                           // dx is now g_b, the gradient at x_b + lin_z[b](z)
     STEP(tg::wgrad(ws.dx16, H, t.lat, C, gr->linz_w[b], C, rows, H, C, st));                     // x += lin_z[b](z): resnetfc.py:176-182
-    if (d_feat || d_xyz || d_z) {
+    if (want_in) {
       tg::RowGemmArgs g = {};                                                                    // dlat (+)= g_b Wz_b
       g.M = rows; g.n_valid = C; g.out_f32 = ws.dlat; g.ld_f32 = C;
       if (b != CL - 1) { g.res_in = ws.dlat; g.ld_res = C; }
@@ -927,14 +1051,11 @@ static int backward_bf16(const pnr_scene* sc, const pnr_points* q, const pnr_mlp
   }
   STEP(tg::wgrad(ws.dx16, H, t.zf, 64, gr->lin_in_w, d_in, rows, H, d_in, st));
 #undef STEP
-  if (d_feat || d_xyz || d_z) {
+  if (want_in) {
     tg::RowGemmArgs g = {};                                                                      // dzf = dx W_in
     g.M = rows; g.n_valid = d_in; g.out_f32 = ws.dzf; g.ld_f32 = d_in;
     if ((rc = rg(ws.dx16, H, H, ws.wpack + w.lin_in, nullptr, 0, 0, nullptr, g, st, &launches))) return rc;
-    long long blocks = (rows + 7) / 8;
-    if (blocks > 148LL * 64) blocks = 148LL * 64;
-    gather_encode_bwd_kernel<<<(unsigned)blocks, 256, 0, st>>>(*sc, *q, ws.dlat, ws.dzf, d_feat, d_xyz, d_z, num_freqs, freq_factor, rows);
-    PNR_CHECK_LAUNCH("bwd::gather_encode_bwd_kernel");
+    if ((rc = gather_bwd(sc, q, ws.dlat, ws.dzf, d_feat, d_xyz, d_z, cams, num_freqs, freq_factor, rows, st))) return rc;
     ++launches;
   }
   reset_launch_count();
@@ -1010,18 +1131,31 @@ extern "C" int pnr_field_backward(const pnr_scene* sc, const pnr_points* q, cons
                                   const float* out, const float* d_out, const pnr_mlp_grads* gr, float* d_feat,
                                   float* d_xyz, float* d_z, void* workspace, size_t workspace_bytes, int num_freqs,
                                   float freq_factor, void* stream) {
+  return pnr_field_backward_cameras(sc, q, mp, tape, out, d_out, gr, d_feat, d_xyz, d_z, nullptr, workspace, workspace_bytes,
+                                    num_freqs, freq_factor, stream);
+}
+
+extern "C" int pnr_field_backward_cameras(const pnr_scene* sc, const pnr_points* q, const pnr_mlp_params* mp, const void* tape,
+                                          const float* out, const float* d_out, const pnr_mlp_grads* gr, float* d_feat,
+                                          float* d_xyz, float* d_z, const pnr_camera_grads* cams, void* workspace,
+                                          size_t workspace_bytes, int num_freqs, float freq_factor, void* stream) {
   reset_launch_count();
-  int rc = check_train(sc, q, mp, num_freqs, "pnr_field_backward");
+  const char* who = cams ? "pnr_field_backward_cameras" : "pnr_field_backward";
+  int rc = check_train(sc, q, mp, num_freqs, who);
   if (rc) return rc;
-  PNR_REQUIRE(tape && out && d_out && gr, PNR_ERR_ARG, "pnr_field_backward: null pointer");
+  PNR_REQUIRE(tape && out && d_out && gr, PNR_ERR_ARG, "%s: null pointer", who);
   PNR_REQUIRE(workspace && workspace_bytes >= pnr_field_backward_workspace_bytes(sc, q, mp), PNR_ERR_ARG,
-              "pnr_field_backward: workspace too small");
+              "%s: workspace too small", who);
   PNR_REQUIRE(!(d_xyz && q->mode != 0) && !(d_z && q->mode != 1), PNR_ERR_ARG,
-              "pnr_field_backward: d_xyz goes with explicit points (mode 0), d_z with rays x depths (mode 1)");
+              "%s: d_xyz goes with explicit points (mode 0), d_z with rays x depths (mode 1)", who);
+  PNR_REQUIRE(!cams || !cams->d_dirs || (q->mode == 0 && q->dirs), PNR_ERR_ARG,
+              "%s: d_dirs goes with explicit points and view directions (mode 0)", who);
+  PNR_REQUIRE(!cams || !cams->d_rays || q->mode == 1, PNR_ERR_ARG, "%s: d_rays goes with rays x depths (mode 1)", who);
   const long long rows = (long long)sc->SB * sc->NS * q->P, pts = (long long)sc->SB * q->P;
   if (pts == 0) return PNR_OK;
   if (sc->flags & PNR_SCENE_TRAIN_BF16)
-    return backward_bf16(sc, q, mp, tape, out, d_out, gr, d_feat, d_xyz, d_z, workspace, num_freqs, freq_factor, (cudaStream_t)stream);
+    return backward_bf16(sc, q, mp, tape, out, d_out, gr, d_feat, d_xyz, d_z, cams, workspace, num_freqs, freq_factor,
+                         (cudaStream_t)stream);
   const int H = mp->d_hidden, C = sc->C, d_in = mp->d_in, nb = mp->n_blocks, CL = mp->combine_layer, NS = sc->NS;
   cudaStream_t st = (cudaStream_t)stream;
   const Tape t = carve_tape((float*)const_cast<void*>(tape), rows, pts, C, d_in, H, nb, CL, pool_max(sc, mp));
@@ -1029,6 +1163,7 @@ extern "C" int pnr_field_backward(const pnr_scene* sc, const pnr_points* q, cons
   float* dB = dA + rows * H;                // dnet / scratch
   float* dlat = dB + rows * H;
   float* dzf = dlat + rows * C;
+  const bool want_in = d_feat || d_xyz || d_z || wants_cams(cams);
   int launches = 0;
   {
     const int rpw = 4;
@@ -1072,11 +1207,8 @@ extern "C" int pnr_field_backward(const pnr_scene* sc, const pnr_points* q, cons
   STEP(colsum(dA, gr->lin_in_b, rows, H, st));
   STEP(linear_bwd_input(dA, mp->lin_in_w, nullptr, dzf, rows, H, d_in, false, st));
 #undef STEP
-  if (d_feat || d_xyz || d_z) {
-    long long blocks = (rows + 7) / 8;
-    if (blocks > 148LL * 64) blocks = 148LL * 64;
-    gather_encode_bwd_kernel<<<(unsigned)blocks, 256, 0, st>>>(*sc, *q, dlat, dzf, d_feat, d_xyz, d_z, num_freqs, freq_factor, rows);
-    PNR_CHECK_LAUNCH("bwd::gather_encode_bwd_kernel");
+  if (want_in) {
+    if ((rc = gather_bwd(sc, q, dlat, dzf, d_feat, d_xyz, d_z, cams, num_freqs, freq_factor, rows, st))) return rc;
     ++launches;
   }
   reset_launch_count();

@@ -221,10 +221,14 @@ composite_resample_kernel(const float4* __restrict__ rgb_sigma, const float* __r
 //                    dsigma_i = dalpha_i delta_i (1 - alpha_i) [sigma_i > 0],   ddelta_i = dalpha_i relu(sigma_i) (1 - alpha_i)
 //                    dz_i = w_i d_depth + ddelta_{i-1} - ddelta_i          (delta_i = z_{i+1} - z_i, last: far - z_K)
 // alpha and T are recomputed exactly as composite_kernel does; the suffix sum runs in double.
+// RAYS: also d far (the last interval is far - z_K) added into column 7 of d_rays; the instantiation without it is the kernel
+// every training step runs.
+template <bool RAYS>
 __global__ void __launch_bounds__(kWarpsPerBlock * 32)
 composite_bwd_kernel(const float4* __restrict__ rgb_sigma, const float* __restrict__ z, const float* __restrict__ rays,
                      const float* __restrict__ d_rgb, const float* __restrict__ d_depth, const float* __restrict__ d_weights,
-                     float4* __restrict__ d_rgb_sigma, float* __restrict__ d_z, int B, int K, int white_bkgd) {
+                     float4* __restrict__ d_rgb_sigma, float* __restrict__ d_z, float* __restrict__ d_rays, int B, int K,
+                     int white_bkgd) {
   extern __shared__ float smem[];
   const int lane = threadIdx.x & 31;
   const int wid = threadIdx.x >> 5;
@@ -300,6 +304,7 @@ composite_bwd_kernel(const float4* __restrict__ rgb_sigma, const float* __restri
       d_z[(size_t)b * K + i] = w * gd + (i > 0 ? sD[i - 1] : 0.f) - sD[i];
     }
   }
+  if (RAYS && lane == ((K - 1) & 31)) d_rays[b * 8 + 7] += sD[K - 1];
 }
 
 // Backward of sample_fine_depth + cat + sort (nerf.py:156-167, 296-301) with respect to the coarse depth: the Kfd depth
@@ -330,6 +335,77 @@ __global__ void sample_depth_bwd_kernel(const float* __restrict__ z_sorted, cons
   if (lane == 0) d_depth[b] = acc;
 }
 
+// near / far gradients of the sample depths, one warp per ray.  Every sample is a function of the ray's bounds:
+//   coarse (nerf.py:117-121) and importance (nerf.py:147-153) samples z = lerp_depth(near, far, s), with s = steps_k + noise / Kc
+//   or s = (ind + jitter) / Kc (the bin is piecewise constant; the sampler reads detached weights, nerf.py:136,293);
+//   depth samples (nerf.py:163-166) z = clamp(depth + gauss std, near, far) send their gradient to the bound they clamp at.
+// z_sorted == nullptr: the coarse samples with their gradient d_z_coarse (B, Kc).  Otherwise the fine pass's merged row z_sorted
+// (B, Kc + Kf + Kfd) and its gradient: each sample of the concatenation (coarse, importance, depth; nerf.py:300-301) is found at
+// the position of its value, equal values taking consecutive positions in concatenation order; the coarse samples' share goes
+// to d_z_coarse_out (B, Kc; overwritten, may be null), the unclamped depth samples' share to the depth
+// (pnr_sample_fine_depth_backward).  d near / d far are added into columns 6 and 7 of d_rays (B, 8).
+__global__ void __launch_bounds__(kWarpsPerBlock * 32)
+sample_bounds_bwd_kernel(const float* __restrict__ rays, const float* __restrict__ steps, const float* __restrict__ noise,
+                         const float* __restrict__ d_z_coarse, const float* __restrict__ z_coarse, const float* __restrict__ z_sorted,
+                         const float* __restrict__ d_z_sorted, const int32_t* __restrict__ inds, const float* __restrict__ jitter,
+                         const float* __restrict__ depth, const float* __restrict__ gauss, float* __restrict__ d_rays,
+                         float* __restrict__ d_z_coarse_out, int B, int Kc, int Kf, int Kfd, float step, float depth_std, int lindisp) {
+  const int lane = threadIdx.x & 31;
+  const int b = blockIdx.x * kWarpsPerBlock + (threadIdx.x >> 5);
+  if (b >= B) return;
+  const float near = rays[b * 8 + 6], far = rays[b * 8 + 7];
+  float dn = 0.f, df = 0.f;
+  // z = near (1 - s) + far s, or 1 / ((1 - s) / near + s / far) with lindisp: dz/dnear = z^2 (1 - s) / near^2, dz/dfar = z^2 s / far^2
+  auto bounds = [&](float s, float g) {
+    if (!lindisp) { dn += g * (1.0f - s); df += g * s; return; }
+    const float z = lerp_depth(near, far, s, 1);
+    dn += g * z * z * (1.0f - s) / (near * near);
+    df += g * z * z * s / (far * far);
+  };
+  if (!z_sorted) {
+    for (int k = lane; k < Kc; k += 32) {
+      const size_t i = (size_t)b * Kc + k;
+      bounds(__fadd_rn(steps[k], __fmul_rn(noise[i], step)), d_z_coarse[i]);
+    }
+  } else {
+    const int K = Kc + Kf + Kfd;
+    const float* zs = z_sorted + (size_t)b * K;
+    const float* dzs = d_z_sorted + (size_t)b * K;
+    const float d = Kfd > 0 ? depth[b] : 0.f;
+    auto fine_s = [&](int j) { return __fdiv_rn(__fadd_rn((float)inds[(size_t)b * Kf + j], jitter[(size_t)b * Kf + j]), (float)Kc); };
+    auto depth_raw = [&](int j) { return __fadd_rn(d, __fmul_rn(gauss[(size_t)b * Kfd + j], depth_std)); };
+    auto cat_value = [&](int c) {            // sample c of the concatenation, exactly as pnr_sample_fine computes it
+      if (c < Kc) return z_coarse[(size_t)b * Kc + c];
+      if (c < Kc + Kf) return lerp_depth(near, far, fine_s(c - Kc), lindisp);
+      return fmaxf(fminf(depth_raw(c - Kc - Kf), far), near);
+    };
+    auto grad_at = [&](float v, int c) {     // gradient at the sorted position of sample c (value v)
+      int lo = 0, hi = K;
+      while (lo < hi) { const int mid = (lo + hi) >> 1; if (zs[mid] < v) lo = mid + 1; else hi = mid; }
+      if (lo + 1 < K && zs[lo + 1] == v)
+        for (int cc = 0; cc < c; ++cc) lo += cat_value(cc) == v;
+      return (lo < K && zs[lo] == v) ? dzs[lo] : 0.f;
+    };
+    for (int k = lane; k < Kc; k += 32) {
+      const float g = grad_at(z_coarse[(size_t)b * Kc + k], k);
+      if (d_z_coarse_out) d_z_coarse_out[(size_t)b * Kc + k] = g;
+    }
+    for (int j = lane; j < Kf; j += 32) {
+      const float s = fine_s(j);
+      bounds(s, grad_at(lerp_depth(near, far, s, lindisp), Kc + j));
+    }
+    for (int j = lane; j < Kfd; j += 32) {
+      const float raw = depth_raw(j);
+      if (raw > near && raw < far) continue;                    // unclamped: the gradient goes to the depth
+      const float g = grad_at(fmaxf(fminf(raw, far), near), Kc + Kf + j);
+      if (raw <= near) dn += g;
+      else if (raw >= far) df += g;
+    }
+  }
+  dn = warp_sum(dn);
+  df = warp_sum(df);
+  if (lane == 0) { d_rays[b * 8 + 6] += dn; d_rays[b * 8 + 7] += df; }
+}
 
 // YoloRenderer.forward's per-ray reduction (src/render/yolo.py:96-114): raw field values (B, K, A*7) -> (B, A, 7) =
 // [max_k p, sum_k(v * p) / (sum_k p + 1e-5)] with p = sigmoid(value 0 of the anchor).  One warp per (ray, anchor).
@@ -498,14 +574,47 @@ extern "C" int pnr_composite_resample(const float* rgb_sigma, const float* rays,
 extern "C" int pnr_composite_backward(const float* rgb_sigma, const float* z, const float* rays, const float* d_rgb,
                                       const float* d_depth, const float* d_weights, float* d_rgb_sigma, float* d_z,
                                       int B, int K, int white_bkgd, void* stream) {
+  return pnr_composite_backward_rays(rgb_sigma, z, rays, d_rgb, d_depth, d_weights, d_rgb_sigma, d_z, nullptr, B, K, white_bkgd,
+                                     stream);
+}
+
+extern "C" int pnr_composite_backward_rays(const float* rgb_sigma, const float* z, const float* rays, const float* d_rgb,
+                                           const float* d_depth, const float* d_weights, float* d_rgb_sigma, float* d_z,
+                                           float* d_rays, int B, int K, int white_bkgd, void* stream) {
   reset_launch_count();
   PNR_REQUIRE(rgb_sigma && z && rays && d_rgb && d_rgb_sigma, PNR_ERR_ARG, "pnr_composite_backward: null pointer");
   PNR_REQUIRE(B >= 0 && K > 0 && K <= 1024, PNR_ERR_ARG, "pnr_composite_backward: bad shape B=%d K=%d", B, K);
   if (B == 0) return PNR_OK;
   const size_t smem = (size_t)kWarpsPerBlock * 3 * K * sizeof(float);
-  composite_bwd_kernel<<<(B + kWarpsPerBlock - 1) / kWarpsPerBlock, kWarpsPerBlock * 32, smem, (cudaStream_t)stream>>>(
-      (const float4*)rgb_sigma, z, rays, d_rgb, d_depth, d_weights, (float4*)d_rgb_sigma, d_z, B, K, white_bkgd);
+  const unsigned grid = (B + kWarpsPerBlock - 1) / kWarpsPerBlock;
+  if (d_rays)
+    composite_bwd_kernel<true><<<grid, kWarpsPerBlock * 32, smem, (cudaStream_t)stream>>>(
+        (const float4*)rgb_sigma, z, rays, d_rgb, d_depth, d_weights, (float4*)d_rgb_sigma, d_z, d_rays, B, K, white_bkgd);
+  else
+    composite_bwd_kernel<false><<<grid, kWarpsPerBlock * 32, smem, (cudaStream_t)stream>>>(
+        (const float4*)rgb_sigma, z, rays, d_rgb, d_depth, d_weights, (float4*)d_rgb_sigma, d_z, nullptr, B, K, white_bkgd);
   PNR_CHECK_LAUNCH("composite_bwd_kernel");
+  return PNR_OK;
+}
+
+extern "C" int pnr_sample_bounds_backward(const float* rays, const float* steps, const float* noise_coarse, const float* d_z_coarse,
+                                          const float* z_coarse, const float* z_sorted, const float* d_z_sorted, const int32_t* inds,
+                                          const float* jitter, const float* depth, const float* gauss, float* d_rays,
+                                          float* d_z_coarse_out, int B, int Kc, int Kf, int Kfd, float depth_std, int lindisp,
+                                          void* stream) {
+  reset_launch_count();
+  PNR_REQUIRE(rays && d_rays, PNR_ERR_ARG, "pnr_sample_bounds_backward: null pointer");
+  PNR_REQUIRE(B >= 0 && Kc > 0 && Kf >= 0 && Kfd >= 0, PNR_ERR_ARG, "pnr_sample_bounds_backward: bad shape");
+  if (!z_sorted)
+    PNR_REQUIRE(steps && noise_coarse && d_z_coarse, PNR_ERR_ARG, "pnr_sample_bounds_backward: coarse inputs missing");
+  else
+    PNR_REQUIRE(z_coarse && d_z_sorted && (Kf == 0 || (inds && jitter)) && (Kfd == 0 || (depth && gauss)), PNR_ERR_ARG,
+                "pnr_sample_bounds_backward: fine-pass inputs missing");
+  if (B == 0) return PNR_OK;
+  sample_bounds_bwd_kernel<<<(B + kWarpsPerBlock - 1) / kWarpsPerBlock, kWarpsPerBlock * 32, 0, (cudaStream_t)stream>>>(
+      rays, steps, noise_coarse, d_z_coarse, z_coarse, z_sorted, d_z_sorted, inds, jitter, depth, gauss, d_rays, d_z_coarse_out, B, Kc,
+      z_sorted ? Kf : 0, z_sorted ? Kfd : 0, (float)(1.0 / (double)Kc), depth_std, lindisp);
+  PNR_CHECK_LAUNCH("sample_bounds_bwd_kernel");
   return PNR_OK;
 }
 

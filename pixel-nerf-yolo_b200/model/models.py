@@ -19,13 +19,15 @@ from .model_util import make_encoder, make_mlp
 class _FieldTrainFn(torch.autograd.Function):
     """PixelNeRFNet.forward with a backward pass (BASELINE config 3): ``pnr_field_forward_train`` keeps the
     activations on a tape, ``pnr_field_backward`` produces what autograd produces for the reference --
-    gradients of the ResnetFC parameters, of the feature maps and of the sample depths / query points."""
+    gradients of the ResnetFC parameters, of the feature maps and of the sample depths / query points.  When a camera input
+    requires grad (the per-view poses / focal / center tensors of ``_camera_tensors``, the view directions in point mode, the
+    rays in ray mode), ``pnr_field_backward_cameras`` adds those gradients in the same pass."""
 
     @staticmethod
-    def forward(ctx, net, mlp, mode, sb, feat, a, b, *params):
+    def forward(ctx, net, mlp, mode, sb, feat, a, b, cam_poses, cam_focal, cam_center, *params):
         lib = _lib.load()
         dev = feat.device
-        sc, keep = net._scene_for(feat, fp32_maps=True)
+        sc, keep = net._scene_for(feat, fp32_maps=True, cams=(cam_poses, cam_focal, cam_center) + net._camera_tensors()[3:])
         # mode "rays": a = rays (SB*B, 8), b = z (SB*B, K); mode "xyz": a = xyz (SB, P, 3), b = viewdirs (SB, P, 3)
         pts = _lib.points_rays(a, b, sb) if mode == "rays" else _lib.points_xyz(a, b)
         P = pts.P
@@ -60,16 +62,28 @@ class _FieldTrainFn(torch.autograd.Function):
         d_feat = torch.zeros_like(feat) if need_feat else None
         d_xyz = torch.zeros_like(a) if (mode == "xyz" and need_a) else None
         d_z = torch.zeros_like(b) if (mode == "rays" and need_b) else None
+        # camera inputs: per-view poses / focal / center, view directions (point mode), rays (ray mode)
+        zeros_if = lambda need, t: torch.zeros(t.shape, device=dev, dtype=torch.float32) if need else None
+        d_poses, d_focal, d_center = (zeros_if(ctx.needs_input_grad[7 + i], t) for i, t in enumerate(ctx.keep[:3]))
+        d_dirs = zeros_if(mode == "xyz" and need_b, b)
+        d_rays = zeros_if(mode == "rays" and need_a, a)
         ws = torch.empty(lib.pnr_field_backward_workspace_bytes(sc, pts, cp), dtype=torch.uint8, device=dev)
         d_out = d_out.contiguous().float()
+        args = (sc, pts, cp, tape.data_ptr(), out.data_ptr(), d_out.data_ptr(), mlp.c_grads(grads), _lib.ptr(d_feat),
+                _lib.ptr(d_xyz), _lib.ptr(d_z))
+        tail = (ws.data_ptr(), ws.numel(), *net.code_args(), _lib.stream_ptr(dev))
+        cam_grads = (d_poses, d_focal, d_center, d_dirs, d_rays)
         with torch.cuda.device(dev):
-            rc = lib.pnr_field_backward(sc, pts, cp, tape.data_ptr(), out.data_ptr(), d_out.data_ptr(),
-                                        mlp.c_grads(grads), _lib.ptr(d_feat), _lib.ptr(d_xyz), _lib.ptr(d_z),
-                                        ws.data_ptr(), ws.numel(), *net.code_args(),
-                                        _lib.stream_ptr(dev))
+            if any(t is not None for t in cam_grads):
+                cg = _lib.CameraGrads(*(_lib.ptr(t) for t in cam_grads))
+                rc = lib.pnr_field_backward_cameras(*args, cg, *tail)
+            else:
+                rc = lib.pnr_field_backward(*args, *tail)
         _lib.check(rc, "pnr_field_backward")
         net.last_bwd_launches = getattr(net, "last_bwd_launches", 0) + lib.pnr_last_launch_count()
-        return (None, None, None, None, d_feat, d_xyz, d_z, *grads)
+        d_a = d_xyz if mode == "xyz" else d_rays
+        d_b = d_dirs if mode == "xyz" else d_z
+        return (None, None, None, None, d_feat, d_a, d_b, d_poses, d_focal, d_center, *grads)
 
 
 class PixelNeRFNet(torch.nn.Module):
@@ -210,15 +224,20 @@ class PixelNeRFNet(torch.nn.Module):
         """pnr_scene view of the encoded state (+ the tensors that must stay alive during the call)."""
         return self._scene_for(self.encoder.packed_latent(fp32=fp32_maps), fp32_maps)
 
-    def _scene_for(self, feat, fp32_maps: bool, cams=None):
-        """pnr_scene over an explicit channels-last feature tensor (the training path passes the autograd-tracked
-        fp32 copy); ``cams`` re-uses the camera tensors captured at forward time."""
-        n_views = self.poses.shape[0]
-        NS = self.num_views_per_obj
-        self._check_views()
-        SB = n_views // NS
-        dev = self.poses.device
-        if self._cam_cache is None:
+    def _camera_tensors(self):
+        """(poses (SB*NS, 3, 4), focal (SB*NS, 2), center (SB*NS, 2), image w, image h, latent scaling x, y): the per-view
+        camera values the kernels read, computed from ``set_cameras``'s state once per encode.  They stay in torch's graph, so
+        gradients of the per-view tensors reach the caller's camera-to-world poses and intrinsics as in the reference; a cache
+        built without that graph (under no_grad) is rebuilt when a camera input requires grad."""
+        cache = self._cam_cache
+        stale = cache is not None and torch.is_grad_enabled() and any(
+            src.requires_grad and not t.requires_grad for src, t in zip((self.poses, self.focal, self.c), cache[:3]))
+        if cache is None or stale:
+            n_views = self.poses.shape[0]
+            NS = self.num_views_per_obj
+            SB = n_views // NS
+            dev = self.poses.device
+
             def per_view(t):     # (1|SB, 2) -> (SB*NS, 2): repeat_interleave over views (models.py:225-230)
                 t = t.to(dev).float()
                 if t.shape[0] == 1:
@@ -233,7 +252,16 @@ class PixelNeRFNet(torch.nn.Module):
             self._cam_cache = (self.poses.contiguous(), per_view(focal_k), per_view(self.c),
                                float(self.image_shape[0]), float(self.image_shape[1]),
                                float(self.encoder.latent_scaling[0]), float(self.encoder.latent_scaling[1]))
-        poses, focal, center, iw, ih, lsx, lsy = cams if cams is not None else self._cam_cache
+        return self._cam_cache
+
+    def _scene_for(self, feat, fp32_maps: bool, cams=None):
+        """pnr_scene over an explicit channels-last feature tensor (the training path passes the autograd-tracked
+        fp32 copy); ``cams`` re-uses the camera tensors captured at forward time."""
+        n_views = self.poses.shape[0]
+        NS = self.num_views_per_obj
+        self._check_views()
+        SB = n_views // NS
+        poses, focal, center, iw, ih, lsx, lsy = cams if cams is not None else self._camera_tensors()
         assert feat.shape[0] == n_views, "encoder.latent and poses disagree on the number of views"
         sc = _lib.Scene()
         sc.feat, sc.poses, sc.focal, sc.center = feat.data_ptr(), poses.data_ptr(), focal.data_ptr(), center.data_ptr()
@@ -335,13 +363,14 @@ class PixelNeRFNet(torch.nn.Module):
             assert viewdirs is not None
         _lib.require_cuda(xyz, "xyz")
         if viewdirs is not None:
-            viewdirs = viewdirs.detach().reshape(SB, B, 3).contiguous().float()
-        if self._wants_grad(coarse, xyz):
+            viewdirs = viewdirs.reshape(SB, B, 3).contiguous().float()
+        if self._wants_grad(coarse, xyz, viewdirs):
             assert SB * self.num_views_per_obj == self.poses.shape[0], "call encode() first"
             mlp = self._mlp(coarse)
             return _FieldTrainFn.apply(self, mlp, "xyz", SB, self._train_feat(), xyz.contiguous().float(), viewdirs,
-                                       *mlp.ordered_params())
+                                       *self._camera_tensors()[:3], *mlp.ordered_params())
         xyz = xyz.detach().contiguous().float()
+        viewdirs = None if viewdirs is None else viewdirs.detach()
         assert SB * self.num_views_per_obj == self.poses.shape[0], "call encode() first"
         outs = []
         step = B if self.precision == "bf16" else max(1, self.fp32_chunk_points // max(SB * self.num_views_per_obj, 1))
@@ -355,11 +384,12 @@ class PixelNeRFNet(torch.nn.Module):
     def _wants_grad(self, coarse, *tensors):
         """True when this call must record a backward pass.  The reference simply runs under autograd, whatever the module's
         train/eval mode: so does this -- gradient mode on and anything on the path requiring grad (query points / depths,
-        the network's parameters, the encoder's maps unless ``stop_encoder_grad``).  Inference callers wrap the call in
+        the network's parameters, the encoder's maps unless ``stop_encoder_grad``, the cameras of ``encode``: poses, focal, c;
+        the caller passes its own camera inputs, view directions or rays).  Inference callers wrap the call in
         ``torch.no_grad()`` as the reference's eval scripts do (eval/eval.py:262, trainer.py vis/eval steps)."""
         if not torch.is_grad_enabled():
             return False
-        want = any(t is not None and t.requires_grad for t in tensors)
+        want = any(t is not None and t.requires_grad for t in tensors + (self.poses, self.focal, self.c))
         want = want or any(p.requires_grad for p in self._mlp(coarse).parameters())
         if not want and not self.stop_encoder_grad:
             lat = self.encoder._latent
@@ -387,9 +417,9 @@ class PixelNeRFNet(torch.nn.Module):
         Bp = Bt // sb
         rays = rays.contiguous().float()
         z = z.contiguous().float()
-        if self._wants_grad(coarse, z):
+        if self._wants_grad(coarse, z, rays):
             mlp = self._mlp(coarse)
-            return _FieldTrainFn.apply(self, mlp, "rays", sb, self._train_feat(), rays.detach(), z,
+            return _FieldTrainFn.apply(self, mlp, "rays", sb, self._train_feat(), rays, z, *self._camera_tensors()[:3],
                                        *mlp.ordered_params()).reshape(Bt, K, self.d_out)
         if self.precision == "bf16":
             pts = _lib.points_rays(rays, z, sb)

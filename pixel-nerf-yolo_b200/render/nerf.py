@@ -13,6 +13,41 @@ from .. import _lib
 from ..conf import DotMap
 
 
+class _CoarseFn(torch.autograd.Function):
+    """sample_coarse (nerf.py:104-124, yolo.py:15-27) with the gradient autograd derives for the reference's near and far
+    (``pnr_sample_bounds_backward``).  Used when the rays require grad; otherwise the depths are drawn without a graph."""
+
+    @staticmethod
+    def forward(ctx, rays, noise, steps, lindisp):
+        lib = _lib.load()
+        B, Kc = noise.shape
+        dev = rays.device
+        noise = noise.contiguous()
+        z = torch.empty(B, Kc, device=dev, dtype=torch.float32)
+        with torch.cuda.device(dev):
+            rc = lib.pnr_sample_coarse(rays.data_ptr(), steps.data_ptr(), noise.data_ptr(), z.data_ptr(), B, Kc, int(lindisp),
+                                       _lib.stream_ptr(dev))
+        _lib.check(rc, "pnr_sample_coarse")
+        ctx.lindisp = int(lindisp)
+        ctx.save_for_backward(rays, noise, steps)
+        return z
+
+    @staticmethod
+    def backward(ctx, d_z):
+        lib = _lib.load()
+        rays, noise, steps = ctx.saved_tensors
+        B, Kc = noise.shape
+        dev = rays.device
+        d_rays = torch.zeros_like(rays)
+        d_z = d_z.contiguous().float()
+        with torch.cuda.device(dev):
+            rc = lib.pnr_sample_bounds_backward(rays.data_ptr(), steps.data_ptr(), noise.data_ptr(), d_z.data_ptr(), None, None,
+                                                None, None, None, None, None, d_rays.data_ptr(), None, B, Kc, 0, 0, 0.0,
+                                                ctx.lindisp, _lib.stream_ptr(dev))
+        _lib.check(rc, "pnr_sample_bounds_backward")
+        return d_rays, None, None, None
+
+
 class _CompositeFn(torch.autograd.Function):
     """composite (nerf.py:184-188, 229-255) with the backward pass autograd derives for the reference."""
 
@@ -45,17 +80,20 @@ class _CompositeFn(torch.autograd.Function):
             d_rgb = torch.zeros(B, 3, device=dev)
         d_out = torch.empty_like(out)
         d_z = torch.empty_like(z) if ctx.needs_input_grad[1] else None
+        d_rays = torch.zeros_like(rays) if ctx.needs_input_grad[2] else None      # far: the last interval is far - z_K
         with torch.cuda.device(dev):
-            rc = lib.pnr_composite_backward(out.data_ptr(), z.data_ptr(), rays.data_ptr(), d_rgb.data_ptr(),
-                                            _lib.ptr(d_depth), _lib.ptr(d_w), d_out.data_ptr(), _lib.ptr(d_z), B, K,
-                                            ctx.white, _lib.stream_ptr(dev))
+            rc = lib.pnr_composite_backward_rays(out.data_ptr(), z.data_ptr(), rays.data_ptr(), d_rgb.data_ptr(),
+                                                 _lib.ptr(d_depth), _lib.ptr(d_w), d_out.data_ptr(), _lib.ptr(d_z),
+                                                 _lib.ptr(d_rays), B, K, ctx.white, _lib.stream_ptr(dev))
         _lib.check(rc, "pnr_composite_backward")
-        return d_out, d_z, None, None
+        return d_out, d_z, d_rays, None
 
 
 class _ResampleFn(torch.autograd.Function):
-    """sample_fine + sample_fine_depth + cat + sort (nerf.py:126-167, 290-301).  Only the coarse depth carries a
-    gradient: the importance sampler is fed detached weights (nerf.py:136, 293)."""
+    """sample_fine + sample_fine_depth + cat + sort (nerf.py:126-167, 290-301).  The coarse depth carries a gradient to the
+    depth samples; when the rays require grad, the merged row also sends gradient to the coarse depths it contains and, from the
+    importance samples and the clamped depth samples, to near / far (the importance sampler is fed detached weights,
+    nerf.py:136, 293)."""
 
     @staticmethod
     def forward(ctx, depth, weights, rays, z_coarse, u, jitter, gauss, kf, kfd, depth_std, lindisp):
@@ -65,30 +103,45 @@ class _ResampleFn(torch.autograd.Function):
         z_out = torch.empty(B, Kc + kf + kfd, device=dev, dtype=torch.float32)
         c = lambda t: None if t is None else t.contiguous().data_ptr()
         depth = depth.contiguous()
+        bounds = ctx.needs_input_grad[2] or ctx.needs_input_grad[3]
+        inds = torch.empty(B, kf, device=dev, dtype=torch.int32) if bounds and kf > 0 else None
         with torch.cuda.device(dev):
             rc = lib.pnr_sample_fine(c(weights), depth.data_ptr(), rays.data_ptr(), z_coarse.data_ptr(), c(u), c(jitter),
-                                     c(gauss), z_out.data_ptr(), None, None, None, B, Kc, kf, kfd, float(depth_std),
+                                     c(gauss), z_out.data_ptr(), _lib.ptr(inds), None, None, B, Kc, kf, kfd, float(depth_std),
                                      int(lindisp), _lib.stream_ptr(dev))
         _lib.check(rc, "pnr_sample_fine")
-        ctx.kfd, ctx.depth_std = kfd, float(depth_std)
-        ctx.save_for_backward(z_out, depth, gauss.contiguous() if gauss is not None else None, rays)
+        ctx.kf, ctx.kfd, ctx.depth_std, ctx.lindisp = kf, kfd, float(depth_std), int(lindisp)
+        cont = lambda t: None if t is None else t.contiguous()
+        ctx.save_for_backward(z_out, depth, cont(gauss), rays, *((z_coarse, inds, cont(jitter)) if bounds else ()))
         return z_out
 
     @staticmethod
     def backward(ctx, d_z):
-        z_out, depth, gauss, rays = ctx.saved_tensors
-        d_depth = None
-        if ctx.kfd > 0 and ctx.needs_input_grad[0]:
-            lib = _lib.load()
-            B, K = z_out.shape
-            d_depth = torch.empty_like(depth)
-            d_z = d_z.contiguous().float()
-            with torch.cuda.device(rays.device):
+        lib = _lib.load()
+        z_out, depth, gauss, rays, *bounds = ctx.saved_tensors
+        B, K = z_out.shape
+        dev = rays.device
+        d_z = d_z.contiguous().float()
+        d_depth = d_rays = d_zc = None
+        with torch.cuda.device(dev):
+            if ctx.kfd > 0 and ctx.needs_input_grad[0]:
+                d_depth = torch.empty_like(depth)
                 rc = lib.pnr_sample_fine_depth_backward(z_out.data_ptr(), d_z.data_ptr(), depth.data_ptr(), gauss.data_ptr(),
                                                         rays.data_ptr(), d_depth.data_ptr(), B, K, ctx.kfd, ctx.depth_std,
-                                                        _lib.stream_ptr(rays.device))
-            _lib.check(rc, "pnr_sample_fine_depth_backward")
-        return (d_depth,) + (None,) * 10
+                                                        _lib.stream_ptr(dev))
+                _lib.check(rc, "pnr_sample_fine_depth_backward")
+            if bounds:
+                z_coarse, inds, jitter = bounds
+                Kc = z_coarse.shape[1]
+                d_rays = torch.zeros_like(rays)
+                d_zc = torch.empty_like(z_coarse)
+                rc = lib.pnr_sample_bounds_backward(rays.data_ptr(), None, None, None, z_coarse.data_ptr(), z_out.data_ptr(),
+                                                    d_z.data_ptr(), _lib.ptr(inds), _lib.ptr(jitter), depth.data_ptr(),
+                                                    _lib.ptr(gauss), d_rays.data_ptr(), d_zc.data_ptr(), B, Kc, ctx.kf, ctx.kfd,
+                                                    ctx.depth_std, ctx.lindisp, _lib.stream_ptr(dev))
+                _lib.check(rc, "pnr_sample_bounds_backward")
+        needs = ctx.needs_input_grad
+        return (d_depth, None, d_rays if needs[2] else None, d_zc if needs[3] else None) + (None,) * 7
 
 
 class _RenderWrapper(torch.nn.Module):
@@ -237,8 +290,8 @@ class NeRFRenderer(torch.nn.Module):
         rays = rays.reshape(-1, 8).contiguous().float()
         nz = self.noise_override or {}
         if torch.is_grad_enabled() and hasattr(model, "_wants_grad") and (
-                model._wants_grad(True) or (self.using_fine and model._wants_grad(False))):
-            return self._forward_train(model, rays.detach(), sb, want_weights, nz)
+                model._wants_grad(True, rays) or (self.using_fine and model._wants_grad(False))):
+            return self._forward_train(model, rays, sb, want_weights, nz)
         if getattr(model, "fused_render_ready", lambda: False)() and rays.shape[0] > 0:
             return self._forward_single_call(model, rays, sb, want_weights, nz)
         with torch.no_grad():
@@ -345,11 +398,19 @@ class NeRFRenderer(torch.nn.Module):
 
     def _forward_train(self, model, rays, sb, want_weights, nz):
         """The same sequence recorded for backward (PixelNerfTrainer.calc_losses -> loss.backward(), config 3):
-        every stage is an autograd.Function over the C-ABI forward/backward kernels."""
+        every stage is an autograd.Function over the C-ABI forward/backward kernels.  Rays that require grad get what autograd
+        gives the reference's: origin and direction from the field, near and far from the samplers and the last interval."""
         dev = rays.device
         B = rays.shape[0]
-        with torch.no_grad():
-            z_coarse = self.sample_coarse(rays, nz.get("coarse"))
+        if rays.requires_grad:
+            noise = nz.get("coarse")
+            if noise is None:
+                noise = torch.rand(B, self.n_coarse, device=dev, dtype=torch.float32)
+            z_coarse = _CoarseFn.apply(rays, noise, self._steps(dev), self.lindisp)
+            self.last_launches += _lib.last_launch_count()
+        else:
+            with torch.no_grad():
+                z_coarse = self.sample_coarse(rays, nz.get("coarse"))
         out_c = self._field(model, rays, z_coarse, True, sb)
         w_c, rgb_c, depth_c = _CompositeFn.apply(out_c, z_coarse, rays, self.white_bkgd)
         outputs = DotMap(coarse=self._format_outputs((w_c, rgb_c, depth_c), sb, want_weights))

@@ -92,11 +92,20 @@ class YoloRenderer(torch.nn.Module):
         res = torch.empty(B, A, 7, device=dev, dtype=torch.float32)
         if B == 0:
             return res
-        if torch.is_grad_enabled() and self.net._wants_grad(True):
+        if torch.is_grad_enabled() and self.net._wants_grad(True, rays):
             # training (YoloTrainer.calc_losses -> loss.backward(), train/trainlib/YoloTrainer.py:140-190): the field records its
-            # backward pass (pnr_field_forward_train / pnr_field_backward), the reduction has its own
-            with torch.no_grad():
-                z = self.sample_coarse(rays, self.noise_override)
+            # backward pass (pnr_field_forward_train / pnr_field_backward), the reduction has its own; rays that require grad
+            # also get their near / far gradient through the coarse sampler
+            if rays.requires_grad:
+                from .nerf import _CoarseFn
+                noise = self.noise_override
+                if noise is None:
+                    noise = torch.rand(B, self.n_coarse, device=dev, dtype=torch.float32)
+                steps = torch.linspace(0, 1 - 1.0 / self.n_coarse, self.n_coarse).to(dev)
+                z = _CoarseFn.apply(rays, noise, steps, False)
+            else:
+                with torch.no_grad():
+                    z = self.sample_coarse(rays, self.noise_override)
             out = self.net.field_from_rays(rays, z, coarse=True, sb=1)              # (B, K, A*7) raw, autograd-tracked
             assert out.shape[-1] == A * 7, f"model d_out {out.shape[-1]} != {A} anchors x 7"
             return _YoloReduceFn.apply(out, B, self.n_coarse, A)
